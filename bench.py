@@ -2,6 +2,7 @@
 """Benchmark of the SPART forward hot path (BASELINE.json metric: simulations / second).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2|3|4|5] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic parameter sets.  The headline line is
 BASELINE.json configs[1] (`--config 2`, the default): 1M-sample PROSPECT-5D + SAILH look-up table,
@@ -28,8 +29,14 @@ Keys of the JSON line:
                      148 SM x 64 DFMA/clk x 2 x the SM clock; `step_frac` is the share-weighted whole step.
                      roofline_hbm gives the same kernel against the measured HBM copy bandwidth,
                      roofline_fp32 the FP32 mode against the measured FFMA peak.
-  cpu_baseline       the UNMODIFIED reference (baseline/_ref, SPART(...).run() per sample, one fresh object
+  cpu_baseline       the UNMODIFIED reference (oracle/_ref, SPART(...).run() per sample, one fresh object
                      each, all host cores) on a bounded sample; the NumPy oracle port's rate is kept beside it.
+
+--dump-outputs DIR writes, after the timed steps of the headline config, the [rows, nb, 3] FP64 band results
+(R_TOC, R_TOA, L_TOA) its last step left in each sensor's output buffer as DIR/bands_<sensor>.npy (rank 0; for
+the chunked configs 4 / 5 the buffer holds the last chunk).  The parameters are generated from fixed seeds, so
+the same arguments give the same inputs on every run and two builds can be compared output for output.  The
+JSON line's `dump_outputs` key records the files, their shapes and which samples they hold.
 """
 import argparse
 import json
@@ -61,6 +68,7 @@ CONFIGS = {
                      "per 1Mi-sample chunk, gathered on rank 0"),
 }
 KERNELS = ("lidf_kernel", "geometry_kernel", "band_kernel")
+DUMP_BYTES = 48 << 20      # --dump-outputs: larger outputs are reduced to a fixed, seeded sample of rows
 
 
 def kernel_source_sha():
@@ -208,7 +216,7 @@ def time_oracle(total, cores, config=2, sensor="Sentinel2A-MSI", chunk=512, pool
     return len(tasks) * chunk / dt, len(tasks) * chunk
 
 
-REF_DIR = ROOT / "baseline" / "_ref"
+REF_DIR = ROOT / "oracle" / "_ref"        # installed by build() (tools/install_reference.py)
 
 
 def reference_available():
@@ -279,7 +287,7 @@ def run_reference(args):
         step = lambda i: time_reference(per_core, cores, args.config, sensor, pool=pool, seed0=9000 + 1000 * i)
         kind, per_step = "reference", per_core * cores
         sample = (f"{per_step} samples/step ({per_core} per core) of the same synthetic distribution through the "
-                  f"unmodified reference (baseline/_ref: fresh LeafBiology / SoilParameters / CanopyStructure / Angles / "
+                  f"unmodified reference (oracle/_ref: fresh LeafBiology / SoilParameters / CanopyStructure / Angles / "
                   f"AtmosphericProperties / SPART object per sample, run()), {cores} processes")
     else:
         per_step = 512 * cores * 2
@@ -287,7 +295,7 @@ def run_reference(args):
         step = lambda i: time_oracle(per_step, cores, args.config, sensor, pool=pool)
         kind = "port"
         sample = (f"{per_step} samples/step, NumPy oracle port (oracle/spart_oracle.py) in {cores} processes; "
-                  "baseline/_ref is missing (run tools/install_reference.py where /root/reference exists)")
+                  "oracle/_ref is missing (build() installs it where the reference checkout of BASELINE.json is readable)")
     for i in range(args.warmup):
         step(-1 - i)
     t0 = time.perf_counter()
@@ -481,6 +489,31 @@ def measure_resident(cx, config, steps, warmup, sampler=None, precision="fp64", 
            "kernel_ms": kern, "gpu_launches": launches, "bands": sum(nbs), "scaling": cfg["scaling"],
            "workload": cfg["workload"]}
     return res, params, outs, (prof_sensor, nbs)
+
+
+def dump_outputs(directory, names, outs, n, chunk):
+    """--dump-outputs: the rows of each sensor's output buffer that the last step wrote (the last chunk starts at
+    sample (n - 1) // chunk * chunk) as float64 <directory>/bands_<sensor>.npy; beyond DUMP_BYTES in all, a
+    sorted row sample drawn with a fixed seed, so that every run with the same arguments keeps the same rows.
+    Returns what was written, for the JSON line."""
+    import numpy as np
+    import torch
+    directory = Path(directory)
+    directory.mkdir(parents=True, exist_ok=True)
+    rows = n - (n - 1) // chunk * chunk
+    files, sampled = {}, False
+    for name, o in zip(names, outs):
+        o = o[:rows]
+        keep = DUMP_BYTES // len(outs) // (o[0].numel() * o.element_size())
+        if keep < rows:
+            sampled = True
+            idx = np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+            o = o[torch.from_numpy(idx).to(o.device)]
+        np.save(directory / f"bands_{name}.npy", o.cpu().numpy())
+        files[f"bands_{name}.npy"] = list(o.shape)
+    return {"dir": str(directory), "files": files, "rank": 0, "first_sample": n - rows, "samples": rows,
+            "rows": "sorted sample numpy.random.default_rng(0).choice(samples, rows, replace=False)" if sampled
+                    else "all"}
 
 
 def measure_e2e(cx, config, params_dev, n, variant, steps=5, precision="fp64"):
@@ -677,6 +710,8 @@ def run_ours(args):
     res, params, outs, (sensor0, nbs) = measure_resident(cx, config, args.steps, args.warmup, sampler, n=args.n)
     n = res["samples_per_gpu_per_step"]
     nb = res["bands"]
+    dump = dump_outputs(args.dump_outputs, cfg["sensors"], outs, n, res["chunk"]) if (args.dump_outputs and
+                                                                                    rank == 0) else None
     # keep the same loop busy for another 0.3 s so that the NVML sampler sees the clocks under this load
     t0 = time.perf_counter()
     while time.perf_counter() - t0 < 0.3:
@@ -803,13 +838,13 @@ def run_ours(args):
             rate, ran = time_reference(48, cores, config, sensor_name)       # ~22 s of reference work per core
             cpu = {"value": rate, "unit": "simulations/s", "cores": cores, "kind": "reference",
                    "sample": f"{ran} samples of the same synthetic distribution through the unmodified reference "
-                             f"(baseline/_ref, one fresh SPART object per sample, run()), {cores} processes",
+                             f"(oracle/_ref, one fresh SPART object per sample, run()), {cores} processes",
                    "port_value": port_rate,
                    "port_sample": f"{port_ran} samples, NumPy oracle port (oracle/spart_oracle.py), {cores} processes"}
         else:
             cpu = {"value": port_rate, "unit": "simulations/s", "cores": cores, "kind": "port",
                    "sample": f"{port_ran} samples of the same synthetic distribution, NumPy oracle port "
-                             f"(oracle/spart_oracle.py), {cores} processes; baseline/_ref is missing"}
+                             f"(oracle/spart_oracle.py), {cores} processes; oracle/_ref is missing"}
 
     line = {
         "metric": METRIC, "value": res["value"], "unit": "simulations/s",
@@ -829,6 +864,7 @@ def run_ours(args):
         "value_with_gather": gather["full"]["value_with_gather"] if gather else None,
         "configs": extras,
         "lut_retrieval": retrieval,
+        "dump_outputs": dump,
     }
     print(json.dumps(line), flush=True)
     if world > 1:
@@ -845,7 +881,13 @@ def main():
     ap.add_argument("--n", type=int, default=None, help="samples per GPU per step (default: the config's)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs 3/4/5 riding on the default line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the band results of the last timed step of the headline config to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -26,6 +26,13 @@ def load_golden(name):
         return {k: z[k] for k in z.files}
 
 
+def golden_columns(a, g):
+    """The wavelength columns of spectra `a` (last axis 2001 or 2162) that golden file `g` stores: its sorted
+    `wl_idx` (tools/make_golden.py::thin_spectra), cut to the width of `a`."""
+    idx = g["wl_idx"]
+    return a[..., idx[idx < a.shape[-1]]]
+
+
 def relerr(a, b):
     """max |a-b| / |b| with NaN == NaN treated as equal."""
     a = np.asarray(a, dtype=np.float64)

@@ -1,5 +1,6 @@
 """CPU-only checks of the host side: C-ABI symbols, loud failure without a GPU, host table
 folding against the oracle, parameter packing, world_size-2 gloo sharding."""
+import json
 import os
 import re
 import socket
@@ -69,6 +70,34 @@ def test_host_tables_match_oracle(optical):
         ak2 = (1 - c["wo"]) * (3 - c["wo"] * 3 * c["gc"])
         assert np.array_equal(st.smac[T.SMAC_ROWS.index("ak2")], ak2[0].astype(np.float64))
         assert ak2.dtype == c["wo"].dtype
+
+
+def test_reference_install(tmp_path, monkeypatch):
+    """tools/install_reference.py (run by build()): copies src/SPART of a reference checkout unchanged plus the
+    nvtx stand-in; a missing checkout, or one below a directory this user may not read, installs nothing."""
+    import importlib.util
+    import pathlib
+    spec = importlib.util.spec_from_file_location("install_reference", ROOT / "tools" / "install_reference.py")
+    inst = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(inst)
+    pkg = tmp_path / "checkout" / "src" / "SPART"
+    (pkg / "model_parameters").mkdir(parents=True)
+    (pkg / "SPART.py").write_text("class SPART:\n    pass\n")
+    (pkg / "model_parameters" / "optical_params.pkl").write_bytes(bytes(range(256)))
+    dest = tmp_path / "_ref"
+    target = inst.install(str(tmp_path / "checkout"), dest)
+    assert target == dest / "SPART" and (dest / "nvtx.py").is_file()
+    assert (target / "SPART.py").read_bytes() == (pkg / "SPART.py").read_bytes()
+    assert (target / "model_parameters" / "optical_params.pkl").read_bytes() == bytes(range(256))
+    assert inst.install(str(tmp_path / "missing"), tmp_path / "none") is None
+    assert not (tmp_path / "none").exists()
+
+    def unreadable(self):
+        raise PermissionError(13, "Permission denied", str(self))
+    monkeypatch.setattr(pathlib.Path, "is_dir", unreadable)
+    assert inst.install(str(tmp_path / "checkout"), tmp_path / "none") is None
+    assert not (tmp_path / "none").exists()
+    assert inst.default_source() == json.loads((ROOT / "BASELINE.json").read_text())["reference_path"]
 
 
 def test_unknown_sensor_raises_filenotfound():

@@ -178,6 +178,17 @@ def conftest_defaults():
     return p
 
 
+def thin_spectra(arrays, step):
+    """Keeps a fixture file under 1 MB: every array of `arrays` whose last axis holds a spectrum (2001 or 2162
+    wavelengths) is cut to every `step`-th wavelength plus 400-415 nm (where the README case is NaN) and the
+    edges of the 2001-sample range; all rows are kept.  The kept indices are stored as `wl_idx` (the tests
+    select the same columns with conftest.golden_columns)."""
+    idx = np.unique(np.r_[np.arange(0, 2162, step), np.arange(16), 1999, 2000, 2001, 2161])
+    out = {k: a[..., idx[idx < a.shape[-1]]] if a.ndim and a.shape[-1] in (2001, 2162) else a for k, a in arrays.items()}
+    out["wl_idx"] = idx
+    return out
+
+
 def readme_quickstart():
     """README.md:23-31 (note the positional slip: Cdm=10, Cs=0.01, Cca=0)."""
     p = conftest_defaults()
@@ -300,7 +311,7 @@ def main():
     P = np.concatenate([so.synthetic_params(3, 2, seed=31), so.synthetic_params(3, 3, seed=32),
                         conftest_defaults()[None, :], readme_quickstart()[None, :]])
     r = run_batch(P, "Sentinel2A-MSI", spectra=True)
-    np.savez_compressed(GOLD / "spectra.npz", params=P, **r)
+    np.savez_compressed(GOLD / "spectra.npz", params=P, **thin_spectra(r, 3))
     print("spectra done", flush=True)
 
     # 4. config 4: synthetic 2001-band sensor
@@ -321,7 +332,7 @@ def main():
     leaf7 = np.array([grid[i] for i in pick], dtype=np.float64)
     o1 = np.stack(pool.map(run_prospect, [(l, False) for l in leaf7]))
     o2 = np.stack(pool.map(run_prospect, [(l, True) for l in leaf7]))
-    np.savez_compressed(GOLD / "prospect_grid.npz", leaf7=leaf7, O1=o1, O2=o2)
+    np.savez_compressed(GOLD / "prospect_grid.npz", leaf7=leaf7, **thin_spectra(dict(O1=o1, O2=o2), 2))
     print("prospect grid done", flush=True)
 
     grid = list(itertools.product(np.arange(1, 8, 3), np.arange(-1, 1, 0.4), np.arange(-1, 1, 0.4),
@@ -335,7 +346,7 @@ def main():
     rho, tau, rs = spec["leaf_refl"], spec["leaf_tran"], spec["soil_refl"]
     res = pool.map(run_sailh, [(c, rho, tau, rs) for c in c7])
     np.savez_compressed(GOLD / "sailh_grid.npz", canopy_angles7=c7, leaf_refl=rho, leaf_tran=tau, soil_refl=rs,
-                        O1=np.stack([x[0] for x in res]), lidf=np.stack([x[1] for x in res]))
+                        lidf=np.stack([x[1] for x in res]), **thin_spectra(dict(O1=np.stack([x[0] for x in res])), 2))
     print("sailh grid done", flush=True)
     pool.close()
 
