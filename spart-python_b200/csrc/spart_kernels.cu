@@ -5,7 +5,7 @@
 //
 //   params [27][n]  --lidf_kernel------>  ws rows F_1..F_12 [12][n]   (block = 128 samples x 12 angles: the
 //        reference's truncated leaf-angle iteration, step for step, run as groups of 32 tasks sorted by
-//        predicted step count; lidf_kernel_v1 is the round-1 warp-queue version, kept behind SPART_LIDF_V2=0)
+//        predicted step count)
 //   params + F      --geometry_kernel-> rec [R_COUNT][n]   (one thread per sample: 13-class volume
 //        scattering, hot-spot integrals, soil vector weights, SMAC geometry/pressure scalars, ET scale)
 //   params + rec    --band_kernel---->  out [n][nb][3]      (one thread per sample, looping over a
@@ -37,23 +37,14 @@
 
 using namespace spart;
 
-// tuning knobs: build alternatives with -D... and time them with SPART_B200_LIB=<so> python tools/kbench.py
+// tuning knobs (numeric; build alternatives with tools/build_alt.sh -D... and time them with
+// SPART_B200_LIB=<so> python tools/kbench.py): SPART_BAND_CHUNK, SPART_BAND_THREADS, the *_MINBLOCKS values,
+// SPART_LIDF_DEG, SPART_LIDF2_R / RA / RB / SUB, and SPART_TAU_SPLIT / SPART_LOG_SPLIT in spart_device.cuh
 #ifndef SPART_BAND_CHUNK
 #define SPART_BAND_CHUNK 16
 #endif
-#ifndef SPART_BAND_SMEM_STATE
-#define SPART_BAND_SMEM_STATE 1
-#endif
-// SPART_BAND_PAIR = 1: the two interpolation knots of a band with a fractional centre wavelength are evaluated side
-// by side (see plate_tau_nb).  Bit-identical; measured: TerraAqua-MODIS (20 bands x 2 knots) 1.558 -> 1.529 ms at
-// 128 registers / 4 blocks per SM (1.559 at 96 registers), Sentinel-3 OLCI 1.283 -> 1.395 ms, and 3 % SLOWER on the
-// one-knot sensors of the benchmark (Sentinel-2A 0.602 -> 0.620 ms): the FP64 pipe gains nothing from a second chain
-// per warp when the operands come from registers (tools/micro/fp64_horner.cu).  Kept as a build knob, off.
-#ifndef SPART_BAND_PAIR
-#define SPART_BAND_PAIR 0
-#endif
 #ifndef SPART_BAND_MINBLOCKS_U
-#define SPART_BAND_MINBLOCKS_U (SPART_BAND_PAIR ? 4 : 5)
+#define SPART_BAND_MINBLOCKS_U 5
 #endif
 #ifndef SPART_SRF_MINBLOCKS
 #define SPART_SRF_MINBLOCKS 5
@@ -200,11 +191,10 @@ struct SpartCtx {
   // staging buffers that are only allocated when the caller's memory is pageable)
   std::mutex mu;
   static const int kSlots = 4;
-  cudaStream_t streams[kSlots] = {};
   cudaEvent_t slot_done[kSlots] = {};      // the slot's device->host copy has finished
   cudaEvent_t slot_k[kSlots] = {};         // the slot's kernels have finished
   cudaStream_t h2d_stream = nullptr, d2h_stream = nullptr;   // one stream per copy direction (see the host path)
-  cudaStream_t join_stream = nullptr;
+  cudaStream_t compute_stream = nullptr, join_stream = nullptr;
   static const int kInSlots = 3;           // device buffers for the parameter spans of the host path
   void* in_params[kInSlots] = {};
   cudaEvent_t in_done[kInSlots] = {};      // the span's host->device copies have finished
@@ -244,48 +234,10 @@ constexpr int kFlagLidfDirect = 1 << 29;
 constexpr uint32_t kLidfRows = (1u << P_LIDFA) | (1u << P_LIDFB);
 constexpr uint32_t kGeometryRows = (1u << P_SZA) | (1u << P_VZA) | (1u << P_RAA);
 
-// Leaf inclination distribution for the 32 samples of a warp (sailh.py:351-398).
-// The 32 x 12 (sample, angle) fixed-point iterations need between 1 and ~120 steps each, so
-// they are treated as a queue of 384 tasks: a lane that converges stores its F value and
-// takes the next task, which keeps all lanes busy until the queue drains.
-// column = thread index in the block.
 __constant__ double c_theta2[12];   // 2 * (pi/180) * theta for theta = 10..80 step 10, 82..88 step 2
 
-#ifndef SPART_LIDF_SPW
-#define SPART_LIDF_SPW 64       // samples per warp in the leaf-angle task queue
-#endif
-#ifndef SPART_LIDF_BATCH
-#define SPART_LIDF_BATCH 6      // idle lanes that trigger a (divergent) task hand-out
-#endif
-constexpr int kLidfSpw = SPART_LIDF_SPW;
-
-// Leaf inclination distribution for the kLidfSpw samples of a warp (sailh.py:351-398).
-//
-// The reference's dcum is the fixed-point iteration x <- x + (y(x) - x + theta2)/2,
-// y = a sin x + b/2 sin 2x, stopped at |dx| <= 1e-8; its result depends on the number of steps
-// taken (1 ... ~120), so the sequence of iterates has to be reproduced, not just its limit.
-// The iterates are reproduced in two stages:
-//   A  exact steps (one sincos each) until the remaining distance to the fixed point is below
-//      ~SPART_LIDF_TAU: |dx| <= TAU (1 - y'(x))/2;
-//   B  from that iterate x_s on, y is replaced by its degree-SPART_LIDF_DEG Taylor polynomial
-//      around x_s.  |x - x_s| <= ~TAU for all later iterates, so the truncation error is below
-//      (|a| + 2^DEG |b|) TAU^(DEG+1) / (DEG+1)! (3e-15 for DEG = 6, TAU = 1.6e-2; measured 5e-15 on
-//      F) and the map
-//      u <- g(u) = (u + y~(u) + theta2 - x_s)/2 is one Horner evaluation per step instead of a
-//      sincos.  Stage B continues the SAME
-//      sequence with the same stopping rule; against the step-by-step iteration the final
-//      F values agree to 1e-15 over the whole |a| + |b| <= 1 domain (tools/check_lidf_taylor.py).
-// Both stages run as a warp-wide task queue over the 12 * kLidfSpw (sample, angle) pairs: a
-// lane that finishes a task goes idle and as soon as SPART_LIDF_BATCH lanes are idle they are
-// all handed new tasks (handing out per finished lane would execute the divergent hand-out
-// code on almost every step).  sA/sB: the warp's LIDFa/LIDFb; sX: per-task hand-over value
-// (x_s, or 2 y + theta2 for a task that already converged in stage A, flagged in sDone).
-// Results F(theta) go to global memory at out[ang * stride_ang + smp * stride_smp].
 #ifndef SPART_LIDF_DEG
-#define SPART_LIDF_DEG 6         // degree of the Taylor model of y around the hand-over iterate
-#endif
-#ifndef SPART_LIDF_TAU
-#define SPART_LIDF_TAU 1.6e-2    // hand-over distance; truncation error ~ 2^DEG TAU^(DEG+1) / (DEG+1)!
+#define SPART_LIDF_DEG 6         // degree of the Taylor model of y in stage B of lidf_kernel
 #endif
 constexpr int kLidfDeg = SPART_LIDF_DEG;
 
@@ -297,343 +249,18 @@ __device__ __forceinline__ double lidf_poly(const double (&g)[kLidfDeg + 1], dou
   return r;
 }
 
-// coefficients of g(u) = (u + y~(u) + k0) / 2, y~ = sum_k y^(k)(xs) u^k / k!, from sin/cos of xs:
-// y^(k) = a sin^(k) x + b 2^(k-1) sin^(k) 2x and sin^(k) cycles through (s, c, -s, -c)
-__device__ __forceinline__ void lidf_poly_setup(double a, double b, double s, double c, double k0,
-                                                double (&g)[kLidfDeg + 1]) {
-  const double s2 = 2.0 * s * c, c2 = fma(2.0 * c, c, -1.0);
-  double fact = 1.0, pow2 = 0.5;        // k!, 2^(k-1)
-#pragma unroll
-  for (int k = 0; k <= kLidfDeg; ++k) {
-    if (k > 0) {
-      fact *= (double)k;
-      pow2 *= 2.0;
-    }
-    const double t1 = (k & 1) ? c : s, t2 = (k & 1) ? c2 : s2;
-    const double sign = (k & 2) ? -1.0 : 1.0;
-    g[k] = (sign * 0.5 / fact) * fma(a, t1, (b * pow2) * t2);
-  }
-  g[0] += 0.5 * k0;
-  g[1] += 0.5;
-}
-
-#ifndef SPART_LIDF_ASTEPS
-#define SPART_LIDF_ASTEPS 2      // exact steps per bookkeeping round
-#endif
-#ifndef SPART_LIDF_A2
-#define SPART_LIDF_A2 0          // 1: stage A steps two tasks per lane side by side (ILP 2); measured 7 % SLOWER
-#endif                           // (0.620 vs 0.580 ms per 1M samples, same 62 registers), kept as a build knob
-#ifndef SPART_LIDF_BSTEPS
-#define SPART_LIDF_BSTEPS 20     // polynomial steps per bookkeeping round (best of 12..24)
-#endif
-#ifndef SPART_LIDF_BLOOP
-#define SPART_LIDF_BLOOP 0
-#endif
-#ifndef SPART_LIDF_BATCH_B
-#define SPART_LIDF_BATCH_B 8     // idle lanes that trigger a stage-B hand-out (its set-up costs a sincos)
-#endif
-constexpr int kLidfTasks = 12 * kLidfSpw;
-
-__device__ __forceinline__ void warp_lidf(const double* sA, const double* sB, double* sX, unsigned char* sDone,
-                                          double* __restrict__ out, int64_t stride_ang, int64_t stride_smp,
-                                          int nvalid) {
-  const unsigned full = 0xffffffffu;
-  const int lane = threadIdx.x & 31;
-  const unsigned lt_mask = (1u << lane) - 1u;
-
-  // ---- stage A: exact steps ------------------------------------------------------------
-#if SPART_LIDF_A2
-  // Experiment (VERDICT r1, item 4): two tasks per lane, stepped branch-free side by side, so that the second
-  // task's dependent chain fills the first one's latency slots.  Same results bit for bit, same 62 registers,
-  // but 7 % slower on the B200 (the selects that keep finished slots frozen and the doubled hand-out
-  // bookkeeping cost more issue slots than the extra ILP recovers), so it is off by default.
-  {
-    int next = 64;                 // warp-uniform: first unassigned task; task t -> angle t / SPW, sample t % SPW
-    int task[2] = {lane, lane + 32};
-    double a[2], b[2], theta2[2], x[2], y[2];
-    bool running[2], conv[2];
-#pragma unroll
-    for (int j = 0; j < 2; ++j) {
-      const int ang = task[j] / kLidfSpw, smp = task[j] % kLidfSpw;
-      a[j] = sA[smp];
-      b[j] = sB[smp];
-      theta2[j] = c_theta2[ang];
-      x[j] = theta2[j];
-      y[j] = 0.0;
-      running[j] = true;
-      conv[j] = false;
-      if (a[j] > 1.0) {            // sailh.py:371-372: closed form F = 1 - cos(theta), no iteration
-        y[j] = 0.5 * (SPART_PI * (1.0 - cos(0.5 * theta2[j])) - theta2[j]);
-        running[j] = false;
-        conv[j] = true;
-      }
-    }
-    int iters = 0;                 // warp-uniform runaway guard (non-convergent garbage input)
-    while (true) {
-#pragma unroll
-      for (int rep = 0; rep < SPART_LIDF_ASTEPS; ++rep) {
-        double s[2], c[2];
-#pragma unroll
-        for (int j = 0; j < 2; ++j) sincos_small(x[j], s[j], c[j]);
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-          const double yn = s[j] * fma(b[j], c[j], a[j]);                    // a sin x + b/2 sin 2x
-          const double dx = fma(0.5, yn, 0.5 * (theta2[j] - x[j]));          // (y - x + theta2) / 2
-          const double adx = fabs(dx);
-          const double yp = fma(a[j], c[j], b[j] * fma(2.0 * c[j], c[j], -1.0));   // y'(x) = a cos x + b cos 2x
-          const bool cv = !(adx > 1e-8);                                      // the reference's stop (NaN stops too)
-          const bool go = !(cv || adx <= (0.5 * SPART_LIDF_TAU) * (1.0 - yp));
-          // a lane whose task is finished keeps its values (selects, no branch: both chains stay interleaved)
-          y[j] = running[j] ? yn : y[j];
-          x[j] = running[j] ? x[j] + dx : x[j];
-          conv[j] = running[j] ? cv : conv[j];
-          running[j] = running[j] && go;
-        }
-      }
-      const unsigned idle0 = __ballot_sync(full, !running[0]);
-      const unsigned idle1 = __ballot_sync(full, !running[1]);
-      const int n0 = __popc(idle0), nidle = n0 + __popc(idle1);
-      if (next < kLidfTasks) {
-        if (nidle >= 2 * SPART_LIDF_BATCH) {
-#pragma unroll
-          for (int j = 0; j < 2; ++j) {
-            if (!running[j]) {
-              if (task[j] >= 0) {
-                sX[task[j]] = conv[j] ? 2.0 * y[j] + theta2[j] : x[j];
-                sDone[task[j]] = conv[j] ? 1 : 0;
-              }
-              task[j] = next + (j == 0 ? __popc(idle0 & lt_mask) : n0 + __popc(idle1 & lt_mask));
-              if (task[j] < kLidfTasks) {
-                const int ang = task[j] / kLidfSpw, smp = task[j] % kLidfSpw;
-                a[j] = sA[smp];
-                b[j] = sB[smp];
-                theta2[j] = c_theta2[ang];
-                x[j] = theta2[j];
-                running[j] = true;
-                conv[j] = false;
-                if (a[j] > 1.0) {
-                  y[j] = 0.5 * (SPART_PI * (1.0 - cos(0.5 * theta2[j])) - theta2[j]);
-                  running[j] = false;
-                  conv[j] = true;
-                }
-              } else {
-                task[j] = -1;      // nothing left for this slot
-                conv[j] = true;
-              }
-            }
-          }
-          next += nidle;
-        }
-      } else if (nidle == 64) {
-        break;
-      }
-      if (++iters > (1 << 22)) break;
-    }
-#pragma unroll
-    for (int j = 0; j < 2; ++j)
-      if (task[j] >= 0) {          // every slot ends idle with its last task's hand-over value in registers
-        sX[task[j]] = conv[j] ? 2.0 * y[j] + theta2[j] : x[j];
-        sDone[task[j]] = conv[j] ? 1 : 0;
-      }
-  }
-#else
-  {
-    int next = 32;                 // warp-uniform: first unassigned task; task t -> angle t / SPW, sample t % SPW
-    int task = lane;
-    double a = sA[lane], b = sB[lane];
-    double theta2 = c_theta2[0];
-    double x = theta2, y = 0.0;
-    bool running = true, conv = false;
-    if (a > 1.0) {                 // sailh.py:371-372: closed form F = 1 - cos(theta), no iteration
-      y = 0.5 * (SPART_PI * (1.0 - cos(0.5 * theta2)) - theta2);
-      running = false;
-      conv = true;
-    }
-    int iters = 0;                 // warp-uniform runaway guard (non-convergent garbage input)
-    while (true) {
-#pragma unroll
-      for (int rep = 0; rep < SPART_LIDF_ASTEPS; ++rep) {
-        if (running) {
-          double s, c;
-          sincos_small(x, s, c);
-          y = s * fma(b, c, a);                                  // a sin x + b/2 sin 2x
-          const double dx = fma(0.5, y, 0.5 * (theta2 - x));     // (y - x + theta2) / 2
-          x += dx;
-          const double adx = fabs(dx);
-          const double yp = fma(a, c, b * fma(2.0 * c, c, -1.0));   // y'(x) = a cos x + b cos 2x
-          conv = !(adx > 1e-8);                                  // the reference's stop (NaN stops too)
-          running = !(conv || adx <= (0.5 * SPART_LIDF_TAU) * (1.0 - yp));
-        }
-      }
-      const unsigned idle = __ballot_sync(full, !running);
-      const int nidle = __popc(idle);
-      if (next < kLidfTasks) {
-        if (nidle >= SPART_LIDF_BATCH) {
-          if (!running) {
-            sX[task] = conv ? 2.0 * y + theta2 : x;
-            sDone[task] = conv ? 1 : 0;
-            task = next + __popc(idle & lt_mask);
-            if (task < kLidfTasks) {
-              const int ang = task / kLidfSpw, smp = task % kLidfSpw;
-              a = sA[smp];
-              b = sB[smp];
-              theta2 = c_theta2[ang];
-              x = theta2;
-              running = true;
-              conv = false;
-              if (a > 1.0) {
-                y = 0.5 * (SPART_PI * (1.0 - cos(0.5 * theta2)) - theta2);
-                running = false;
-                conv = true;
-              }
-            } else {
-              task = -1;           // nothing left for this lane
-            }
-          }
-          next += nidle;
-        }
-      } else if (nidle == 32) {
-        break;
-      }
-      if (++iters > (1 << 22)) break;
-    }
-    if (task >= 0) {               // every lane ends idle with its last task's hand-over value in registers
-      sX[task] = conv ? 2.0 * y + theta2 : x;
-      sDone[task] = conv ? 1 : 0;
-    }
-  }
-#endif
-  __syncwarp();
-
-  // ---- stage B: Taylor-model steps -------------------------------------------------------
-  {
-    int next = 0;
-    int ang = 0, smp = kLidfSpw;   // no task yet
-    double g[kLidfDeg + 1] = {0.0};
-    double u = 0.0, uf = 0.0, k0 = 0.0, theta2 = 0.0;
-    double num = 0.0;              // 2 y + theta2 of a task that converged in stage A
-    bool direct = false;
-    bool running = false;
-    int iters = 0;
-    while (true) {
-#if SPART_LIDF_BLOOP
-      // up to SPART_LIDF_BSTEPS polynomial steps per bookkeeping round; converged lanes drop out of
-      // the loop (hardware divergence), so a step costs the 7 FMA, the difference and the test only
-      for (int rep = 0; rep < SPART_LIDF_BSTEPS && running; ++rep) {
-        const double un = lidf_poly(g, u);
-        if (!(fabs(un - u) > 1e-8)) {
-          uf = u;
-          running = false;
-        }
-        u = un;
-      }
-#else
-      // SPART_LIDF_BSTEPS polynomial steps per bookkeeping round, branch-free: a lane that
-      // converges inside the round freezes (u, u_new) of its last step with selects
-#pragma unroll
-      for (int rep = 0; rep < SPART_LIDF_BSTEPS; ++rep) {
-        const double un = lidf_poly(g, u);
-        // first step with |du| <= 1e-8: remember the iterate it started from; u itself may keep
-        // iterating (a finished lane is never looked at again), which saves the selects on u
-        if (running && !(fabs(un - u) > 1e-8)) {
-          uf = u;
-          running = false;
-        }
-        u = un;
-      }
-#endif
-      const unsigned idle = __ballot_sync(full, !running);
-      const int nidle = __popc(idle);
-      if (next < kLidfTasks) {
-        if (nidle >= SPART_LIDF_BATCH_B || next == 0) {
-          if (!running) {
-            // y~(u) = 2 g(u) - u - k0, so 2 y + theta2 = 4 g(u) - 2 u - 2 k0 + theta2 at the last iterate
-            if (smp < nvalid) {
-              const double unf = lidf_poly(g, uf);
-              out[ang * stride_ang + smp * stride_smp] =
-                  (direct ? num : 2.0 * (2.0 * unf - uf - k0) + theta2) * (1.0 / SPART_PI);
-            }
-            const int task = next + __popc(idle & lt_mask);
-            if (task < kLidfTasks) {
-              ang = task / kLidfSpw;
-              smp = task % kLidfSpw;
-              theta2 = c_theta2[ang];
-              const double xs = sX[task];
-              direct = sDone[task] != 0;
-              if (direct) {
-                num = xs;          // converged in stage A: xs already is 2 y + theta2
-              } else {
-                const double a = sA[smp], b = sB[smp];
-                double s, c;
-                sincos_small(xs, s, c);
-                k0 = theta2 - xs;
-                lidf_poly_setup(a, b, s, c, k0, g);
-                u = 0.0;
-                running = true;
-              }
-            } else {
-              smp = kLidfSpw;      // nothing left to write for this lane
-            }
-          }
-          next += nidle;
-        }
-      } else if (nidle == 32) {
-        break;
-      }
-      if (++iters > (1 << 22)) break;
-    }
-    if (smp < nvalid) {
-      const double unf = lidf_poly(g, uf);
-      out[ang * stride_ang + smp * stride_smp] =
-          (direct ? num : 2.0 * (2.0 * unf - uf - k0) + theta2) * (1.0 / SPART_PI);
-    }
-  }
-}
-
 // workspace rows: the per-sample record followed by the 12 cumulative leaf-angle values
 constexpr int kRowF = R_COUNT;
 constexpr int kWsRows = R_COUNT + 13;     // (the 13th row is used by a caller-supplied distribution only)
 
-#ifndef SPART_LIDF_THREADS
-#define SPART_LIDF_THREADS 128
-#endif
-#ifndef SPART_LIDF_MINBLOCKS
-#define SPART_LIDF_MINBLOCKS (1024 / SPART_LIDF_THREADS)
-#endif
-constexpr int kLidfThreads = SPART_LIDF_THREADS;
-
-// Kernel 1: leaf inclination distribution (CanopyStructure.__init__, sailh.py:340-398).
-// A kernel of its own so that it runs at ~54 registers / 36 warps per SM: the iteration is
-// one long dependent FP64 chain per lane and needs the occupancy to fill the FP64 pipe.
-// ab0/ab1: the LIDFa / LIDFb rows with element strides st0/st1 (1, or 0 for a broadcast row);
-// F(theta_i) of sample s is written to out[i * stride_ang + s * stride_smp].
-__global__ void __launch_bounds__(kLidfThreads, SPART_LIDF_MINBLOCKS)
-lidf_kernel_v1(const double* __restrict__ ab0, const double* __restrict__ ab1, int64_t st0, int64_t st1, int64_t n,
-            double* __restrict__ out, int64_t stride_ang, int64_t stride_smp) {
-  constexpr int kWarps = kLidfThreads / 32;
-  __shared__ double sA[kWarps][kLidfSpw], sB[kWarps][kLidfSpw];
-  __shared__ double sX[kWarps][kLidfTasks];
-  __shared__ unsigned char sDone[kWarps][kLidfTasks];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int64_t base = ((int64_t)blockIdx.x * kWarps + warp) * kLidfSpw;   // first sample of this warp
-  if (base >= n) return;
-  for (int j = lane; j < kLidfSpw; j += 32) {
-    const int64_t s = (base + j < n) ? base + j : n - 1;     // tail entries shadow the last sample
-    sA[warp][j] = ab0[s * st0];      // st = 0: the row is constant over the batch (broadcast row)
-    sB[warp][j] = ab1[s * st1];
-  }
-  __syncwarp();
-  const int nvalid = (int)((n - base < kLidfSpw) ? (n - base) : kLidfSpw);
-  warp_lidf(sA[warp], sB[warp], sX[warp], sDone[warp], out + base * stride_smp, stride_ang, stride_smp, nvalid);
-}
-
-// ---- leaf-angle kernel, version 2: the same iterations, scheduled as length-sorted groups ----------------
-// lidf_kernel_v1 above treats a warp's (sample, angle) tasks as a queue; with task lengths of 1..26 exact and
-// 3..84 polynomial steps (mean 4.3 / 19.9 on the benchmark distribution) its lanes spend ~45 % of the issued
-// instructions in rounds they have already finished or in divergent hand-out code (tools/lidf_queue_sim.py).
-// Version 2 runs the same iterations per task (with SPART_LIDF2_CENTRED = 0 the very same arithmetic: results
-// are bit-identical; with the centred Taylor model of the default build F agrees to 1e-15, see lidf2_hand) but
-// orders the work by *predicted* length first:
+// ---- Kernel 1: leaf inclination distribution (CanopyStructure.__init__, sailh.py:340-398) ----------------------
+// The reference's dcum is the fixed-point iteration x <- x + (y(x) - x + theta2)/2, y = a sin x + b/2 sin 2x,
+// stopped at |dx| <= 1e-8; its result depends on the number of steps taken, so the sequence of iterates has to be
+// reproduced, not just its limit.  Exact steps (one sincos each) run until the iterate is close to the fixed point;
+// from there on y is replaced by a degree-SPART_LIDF_DEG Taylor model around a point near the fixed point, one
+// Horner evaluation per step (see lidf2_hand).  A block takes 128 samples, i.e. 12 x 128 (sample, angle) tasks,
+// whose step counts vary widely; so that the 32 lanes of a warp run tasks of about the same length, the work is
+// ordered by *predicted* length first:
 //   A1  the first exact step of all 12 x 128 tasks of a block, without a sincos (x0 = theta2 is one of twelve
 //       constants, whose sine / cosine sit in a table filled by the same sincos_small); from its |dx| and
 //       y'(x0) the linear-convergence model predicts the remaining exact steps (or, for a task that hands
@@ -644,29 +271,17 @@ lidf_kernel_v1(const double* __restrict__ ab0, const double* __restrict__ ab1, i
 //   sort by predicted polynomial steps; B: the same with the Taylor-model steps (a vote every
 //       SPART_LIDF2_RB steps); results are staged in shared memory and written as 12 coalesced rows.
 // The predictions only decide the grouping, never a result: every task runs until its own stop criterion.
-#ifndef SPART_LIDF_V2
-#define SPART_LIDF_V2 1
-#endif
+// The iteration is one long dependent FP64 chain per lane, so the kernel is kept apart from the others and
+// needs the occupancy of SPART_LIDF2_MINBLOCKS blocks per SM to fill the FP64 pipe.
+// (The round-1 version, a per-warp task queue, is in git history at 64fd57e.)
 #ifndef SPART_LIDF2_RB
 #define SPART_LIDF2_RB 4
 #endif
 #ifndef SPART_LIDF2_RA
 #define SPART_LIDF2_RA 1
 #endif
-#ifndef SPART_LIDF2_CENTRED
-#define SPART_LIDF2_CENTRED 1    // 0: hand over at TAU and expand around the hand-over iterate (bit-identical to lidf_kernel_v1)
-#endif
 #ifndef SPART_LIDF2_R
 #define SPART_LIDF2_R 0.15       // hand-over radius of the centred Taylor model
-#endif
-#ifndef SPART_LIDF2_AB_SMEM
-#define SPART_LIDF2_AB_SMEM 1    // 0: stages A2 / B re-read LIDFa / LIDFb from global memory (2 KB less shared memory)
-#endif
-#ifndef SPART_LIDF2_BILP
-#define SPART_LIDF2_BILP 1       // groups a warp steps side by side in stage B
-#endif
-#ifndef SPART_LIDF2_SKIP
-#define SPART_LIDF2_SKIP 0       // timing experiments only: 1 = stop after A1 + sort, 2 = stop after A2 + sort
 #endif
 #ifndef SPART_LIDF2_MINBLOCKS
 #define SPART_LIDF2_MINBLOCKS 8
@@ -685,15 +300,11 @@ constexpr int kL2MaxVotes = 1 << 15;
 
 struct Lidf2Smem {
   double x[kL2Tasks];            // x_1 -> hand-over iterate x_s (or 2 y + theta2 of a task that converged in stage A) -> F
-#if SPART_LIDF2_AB_SMEM
   double a[kL2Samples], b[kL2Samples];
-#endif
   double theta2[12], sin0[12], cos0[12];
   unsigned short perm[kL2Tasks];
   unsigned short rank[kL2Tasks];
-#if SPART_LIDF2_CENTRED
   signed char dq[kL2Tasks];      // (expansion centre - hand-over iterate) * 2^8
-#endif
   // per task: 0 = converged in stage A ("direct"), 1..63 = predicted polynomial steps of a handed-over task,
   // 128 + k = k more exact steps predicted
   unsigned char key[kL2Tasks];
@@ -712,41 +323,31 @@ __device__ __forceinline__ float lidf2_lg2(float x) {
   return r;
 }
 
-// Hand-over test of an exact step at x with step dx and slope yp = y'(x).
-// SPART_LIDF2_CENTRED = 0: the Newton estimate 2 |dx| / (1 - y') of the distance to the fixed point is below TAU
-//   (the rule of lidf_kernel_v1; stage B expands around the next iterate).
-// SPART_LIDF2_CENTRED = 1: stage B expands around the Newton estimate xc = x + 2 dx / (1 - y') of the fixed point
-//   itself.  The truncation error c |x_n - xc|^7 of the degree-6 model is then largest for the first
-//   polynomial iterates, where it matters least: the iteration contracts an error made at distance d from the
-//   fixed point by ~1e-8 / d before the stop.  That admits a ten times larger hand-over radius,
-//   |2 dx / (1 - y')| <= R (1 - lam)^(1/3) with R = 0.15 (the cube root keeps slowly converging tasks, whose Newton
-//   estimate is poor and whose errors contract slowly, on exact steps for longer): 2.0 exact steps per task
-//   instead of 4.3 on the benchmark distribution (the first one is free) for 2.2 more polynomial steps, F within
-//   9e-16 of the step-by-step iteration over the whole |a| + |b| <= 1 domain, its boundary included
-//   (tools/check_lidf_centred.py: NumPy prototype with the kernel's arithmetic; GPU: tools/lidf_parity_scale.py).  The test is
-//   written without a division: 8 |dx|^3 <= R^3 (1 - y')^3 (1 - y') / 2.
+// Hand-over test of an exact step at x with step dx and slope yp = y'(x).  Stage B expands around the Newton
+// estimate xc = x + 2 dx / (1 - y') of the fixed point itself.  The truncation error c |x_n - xc|^7 of the
+// degree-6 model is then largest for the first polynomial iterates, where it matters least: the iteration
+// contracts an error made at distance d from the fixed point by ~1e-8 / d before the stop.  That admits a ten
+// times larger hand-over radius than an expansion around the hand-over iterate,
+// |2 dx / (1 - y')| <= R (1 - lam)^(1/3) with R = 0.15 (the cube root keeps slowly converging tasks, whose Newton
+// estimate is poor and whose errors contract slowly, on exact steps for longer): 2.0 exact steps per task
+// instead of 4.3 on the benchmark distribution (the first one is free) for 2.2 more polynomial steps, F within
+// 9e-16 of the step-by-step iteration over the whole |a| + |b| <= 1 domain, its boundary included
+// (tools/check_lidf_centred.py: NumPy prototype with the kernel's arithmetic; GPU: tools/lidf_parity_scale.py).
+// The test is written without a division: 8 |dx|^3 <= R^3 (1 - y')^3 (1 - y') / 2.
 __device__ __forceinline__ bool lidf2_hand(double adx, double yp) {
-#if SPART_LIDF2_CENTRED
   const double w = 1.0 - yp, w2 = w * w;
   return adx * adx * adx <= (SPART_LIDF2_R * SPART_LIDF2_R * SPART_LIDF2_R / 16.0) * (w2 * w2);
-#else
-  return adx <= (0.5 * SPART_LIDF_TAU) * (1.0 - yp);
-#endif
 }
 
 // Sort key of a task that leaves an exact step unconverged, from the linear-convergence model in single
 // precision (three MUFU.LG2 / RCP pairs; it only decides the grouping): lam = g'(x) = (1 + y') / 2,
 //   hand-over:  polynomial steps until |du| = |dx| lam^(n+1) <= 1e-8            -> key 1 .. 63
 //   otherwise:  exact steps until the distance |dx| lam^n 2 / (1 - y') <= radius  -> key 128 + (1 .. 31)
-// and, for the centred model, dq = (centre - next iterate) 2^8 with centre - next iterate =
+// and dq = (centre - next iterate) 2^8 with centre - next iterate =
 // (x + 2 dx / (1 - y')) - (x + dx) = dx (1 + y') / (1 - y'): any point within ~1e-2 of the fixed point serves as
 // expansion centre (the Newton estimate itself is no better), and xc = x_next + dq 2^-8 is exact in FP64.
 __device__ __forceinline__ unsigned char lidf2_leave(double dx, double yp, bool hand, signed char& dq) {
-#if SPART_LIDF2_CENTRED
   const float inv_radius = (float)(2.0 / SPART_LIDF2_R);
-#else
-  const float inv_radius = (float)(2.0 / SPART_LIDF_TAU);
-#endif
   const float ypf = (float)yp, dxf = (float)dx;
   const float rw = lidf2_rcp(1.0f - ypf);
   const float lam = fminf(fmaxf(fmaf(0.5f, ypf, 0.5f), 1e-3f), 0.9995f);
@@ -757,8 +358,9 @@ __device__ __forceinline__ unsigned char lidf2_leave(double dx, double yp, bool 
   return hand ? (unsigned char)min(k + 1, 63) : (unsigned char)(128 + min(max(k, 1), 31));
 }
 
-// lidf_poly_setup with the products a sin, a cos, b sin 2x, b cos 2x formed once: g_k = C_k (A_k + 2^(k-1) B_k),
-// C_k = +-1 / (2 k!) -- 23 FP64 operations instead of 33 (the coefficients differ from lidf_poly_setup's by an ulp)
+// coefficients of the map g(u) = (u + y~(u) + k0) / 2 of stage B, y~ = sum_k y^(k)(xc) u^k / k!, from sin / cos of
+// the expansion centre xc: y^(k) = a sin^(k) x + b 2^(k-1) sin^(k) 2x and sin^(k) cycles through (s, c, -s, -c).
+// The products a sin, a cos, b sin 2x, b cos 2x are formed once: g_k = C_k (A_k + 2^(k-1) B_k), C_k = +-1 / (2 k!).
 __device__ __forceinline__ void lidf2_poly_setup(double a, double b, double s, double c, double k0,
                                                  double (&g)[kLidfDeg + 1]) {
   const double s2 = 2.0 * s * c, c2 = fma(2.0 * c, c, -1.0);
@@ -833,22 +435,15 @@ lidf_kernel(const double* __restrict__ ab0, const double* __restrict__ ab1, int6
   if (tid < 12) {
     const double th = c_theta2[tid];
     double s, c;
-    sincos_small(th, s, c);          // the values the first exact step of lidf_kernel_v1 computes
+    sincos_small(th, s, c);          // sine / cosine of the first exact step, which starts at x0 = theta2
     S.theta2[tid] = th;
     S.sin0[tid] = s;
     S.cos0[tid] = c;
   }
   const int64_t smp_g = (base + tid < n) ? base + tid : n - 1;     // tail entries shadow the last sample
   const double a = ab0[smp_g * st0], b = ab1[smp_g * st1];         // st = 0: broadcast row
-#if SPART_LIDF2_AB_SMEM
   S.a[tid] = a;
   S.b[tid] = b;
-#define LIDF2_A(smp) S.a[smp]
-#define LIDF2_B(smp) S.b[smp]
-#else
-#define LIDF2_A(smp) ab0[((base + (smp) < n) ? base + (smp) : n - 1) * st0]
-#define LIDF2_B(smp) ab1[((base + (smp) < n) ? base + (smp) : n - 1) * st1]
-#endif
   __syncthreads();
 
   // ---- A1: first exact step of every task (thread = sample, loop over the angles) ------------------------
@@ -869,9 +464,7 @@ lidf_kernel(const double* __restrict__ ab0, const double* __restrict__ ab1, int6
       const bool conv = !(adx > 1e-8);
       signed char dq;
       const unsigned char key = lidf2_leave(dx, yp, lidf2_hand(adx, yp), dq);
-#if SPART_LIDF2_CENTRED
       S.dq[t] = dq;
-#endif
       S.x[t] = conv ? 2.0 * y + theta2 : theta2 + dx;
       S.key[t] = conv ? (unsigned char)0 : key;
     }
@@ -880,7 +473,7 @@ lidf_kernel(const double* __restrict__ ab0, const double* __restrict__ ab1, int6
   lidf2_sort(S, [](unsigned char v) { return v >= 128 ? 159 - (int)v : 32; }, 32);   // 31 .. 1 more steps -> bins 0 .. 30
 
   // ---- A2: remaining exact steps, groups of 32 tasks of similar predicted length -------------------------
-  if (SPART_LIDF2_SKIP != 1) {
+  {
     const int nwork = S.nwork;
     while (true) {
       int g = 0;
@@ -891,7 +484,7 @@ lidf_kernel(const double* __restrict__ ab0, const double* __restrict__ ab1, int6
       const bool has = pos < nwork;
       const int t = S.perm[has ? pos : 0];
       const int ang = t / kL2Samples, smp = t % kL2Samples;
-      const double ta = LIDF2_A(smp), tb = LIDF2_B(smp), theta2 = S.theta2[ang];
+      const double ta = S.a[smp], tb = S.b[smp], theta2 = S.theta2[ang];
       double x = S.x[t], y = 0.0, dx = 1.0, yp = 0.0;
       bool running = has, conv = false;
       int iters = 0;
@@ -916,19 +509,18 @@ lidf_kernel(const double* __restrict__ ab0, const double* __restrict__ ab1, int6
         signed char dq;
         const unsigned char key = lidf2_leave(dx, yp, true, dq);
         S.key[t] = conv ? (unsigned char)0 : key;
-#if SPART_LIDF2_CENTRED
         S.dq[t] = dq;
-#endif
       }
     }
   }
   lidf2_sort(S, [](unsigned char v) { return 63 - (int)(v & 63); }, 63);   // 63 .. 1 polynomial steps -> bins 0 .. 62
 
-  // ---- B: Taylor-model steps ---------------------------------------------------------------------------
-  // A warp takes SPART_LIDF2_BILP consecutive groups (neighbours in the sorted order, so of about the same length)
-  // and steps them side by side: the Horner chains of the groups interleave and fill each other's latency slots.
-  if (SPART_LIDF2_SKIP == 0) {
-    constexpr int NG = SPART_LIDF2_BILP;
+  // ---- B: Taylor-model steps, groups of 32 tasks of similar predicted length ----------------------------
+  // One group per warp (NG = 1): two neighbouring groups stepped side by side, their Horner chains interleaved,
+  // gained nothing (DESIGN.md).  The loops over the one group stay: the same steps written with scalars compile to
+  // a different register allocation than the build the measurements under profiles/ were taken on.
+  {
+    constexpr int NG = 1;
     const int nwork = S.nwork;
     while (true) {
       int g = 0;
@@ -946,21 +538,12 @@ lidf_kernel(const double* __restrict__ ab0, const double* __restrict__ ab1, int6
         const int ang = t[j] / kL2Samples, smp = t[j] % kL2Samples;
         theta2[j] = S.theta2[ang];
         const double xs = S.x[t[j]];
-#if SPART_LIDF2_CENTRED
         const double xc = xs + (double)S.dq[t[j]] * (1.0 / 256.0);   // expansion centre: near the fixed point
         u[j] = xs - xc;                                               // (exact)
-#else
-        const double xc = xs;
-        u[j] = 0.0;
-#endif
         double s, c;
         sincos_small(xc, s, c);
         k0[j] = theta2[j] - xc;
-#if SPART_LIDF2_CENTRED
-        lidf2_poly_setup(LIDF2_A(smp), LIDF2_B(smp), s, c, k0[j], gk[j]);
-#else
-        lidf_poly_setup(LIDF2_A(smp), LIDF2_B(smp), s, c, k0[j], gk[j]);      // bit-identical to lidf_kernel_v1
-#endif
+        lidf2_poly_setup(S.a[smp], S.b[smp], s, c, k0[j], gk[j]);
       }
       bool running = false;
       int iters = 0;
@@ -969,21 +552,13 @@ lidf_kernel(const double* __restrict__ ab0, const double* __restrict__ ab1, int6
         // repeats that step, so no separate "finished" state is carried through the steps
 #pragma unroll
         for (int rep = 0; rep < SPART_LIDF2_RB; ++rep) {
-          // the Horner chains of the NG groups advance together, term by term: independent FP64 instructions
-          // issued back to back by one warp keep the pipe's 2-cycle cadence, whereas FP64 instructions of
-          // different warps follow each other every 3 cycles (tools/micro/fp64_latency.cu)
           double un[NG];
 #pragma unroll
           for (int j = 0; j < NG; ++j) un[j] = gk[j][kLidfDeg];
 #pragma unroll
           for (int k = kLidfDeg - 1; k >= 0; --k)
 #pragma unroll
-            for (int j = 0; j < NG; ++j) {
-              if (NG > 1)     // volatile: keeps the term-by-term order through the compiler's own scheduling
-                asm volatile("fma.rn.f64 %0, %1, %2, %3;" : "=d"(un[j]) : "d"(un[j]), "d"(u[j]), "d"(gk[j][k]));
-              else
-                un[j] = fma(un[j], u[j], gk[j][k]);
-            }
+            for (int j = 0; j < NG; ++j) un[j] = fma(un[j], u[j], gk[j][k]);
           running = false;
 #pragma unroll
           for (int j = 0; j < NG; ++j) {
@@ -1285,6 +860,55 @@ __device__ __forceinline__ SoilPar load_soil(const Params& P,
 constexpr int kBandThreads = SPART_BAND_THREADS;
 constexpr int kBandChunk = SPART_BAND_CHUNK;   // bands handled by one block (per-sample state is loaded once per chunk)
 
+__device__ __forceinline__ AtmSample load_atm(const Params& P, const double* __restrict__ rec, int64_t n, int64_t s) {
+  AtmSample A;
+  A.us = rec[R_US * n + s];
+  A.uv = rec[R_UV * n + s];
+  A.m = rec[R_M * n + s];
+  A.Peq = rec[R_PEQ * n + s];
+  A.lo3 = rec[R_LO3 * n + s];
+  A.lh2o = rec[R_LH2O * n + s];
+  A.lm = rec[R_LM * n + s];
+  A.lpeq = rec[R_LPEQ * n + s];
+  A.cksi = rec[R_CKSI * n + s];
+  A.ksiD = rec[R_KSID * n + s];
+  A.ray_phase = rec[R_RAYPH * n + s];
+  A.taup550 = P.at(P_AOT, s);
+  A.inv_us = rec[R_INVUS * n + s];
+  A.inv_uv = rec[R_INVUV * n + s];
+  A.inv_1pus = rec[R_INV1PUS * n + s];
+  A.inv_1puv = rec[R_INV1PUV * n + s];
+  A.aa3 = rec[R_AA3 * n + s];
+  return A;
+}
+
+// The band kernels park the soil and canopy state in shared memory (one column per thread, no synchronisation
+// needed) and re-read it per wavelength right before use: soil before bsm_point, canopy before sailh_point.  That
+// keeps 34 registers less live across the leaf model; the re-reads are volatile so that the compiler keeps them
+// where they are instead of hoisting them back into registers.
+constexpr int kStateRows = 17;
+__device__ __forceinline__ void park_state(double (*st)[kBandThreads], const SoilPar& S, const CanopyGeo& G) {
+  const double v[kStateRows] = {S.f1, S.f2, S.f3, S.mu, S.emu, S.film, G.LAI, G.k, G.K, G.bf, G.sob, G.sof,
+                                G.tau_ss, G.tau_oo, G.sumpso, G.pso2w, G.Z};
+#pragma unroll
+  for (int i = 0; i < kStateRows; ++i) st[i][threadIdx.x] = v[i];
+}
+
+__device__ __forceinline__ SoilPar reload_soil(volatile double (*st)[kBandThreads]) {
+  const int t = threadIdx.x;
+  SoilPar S;
+  S.f1 = st[0][t]; S.f2 = st[1][t]; S.f3 = st[2][t]; S.mu = st[3][t]; S.emu = st[4][t]; S.film = st[5][t];
+  return S;
+}
+
+__device__ __forceinline__ CanopyGeo reload_geo(volatile double (*st)[kBandThreads]) {
+  const int t = threadIdx.x;
+  CanopyGeo G;
+  G.LAI = st[6][t]; G.k = st[7][t]; G.K = st[8][t]; G.bf = st[9][t]; G.sob = st[10][t]; G.sof = st[11][t];
+  G.tau_ss = st[12][t]; G.tau_oo = st[13][t]; G.sumpso = st[14][t]; G.pso2w = st[15][t]; G.Z = st[16][t];
+  return G;
+}
+
 // One thread per sample, looping over a chunk of up to kBandChunk bands; blockIdx.x = band
 // chunk, blockIdx.y = sample tile.  The per-sample state (leaf, soil, canopy geometry, SMAC
 // scalars: 44 doubles) is read from HBM once per chunk and kept in registers; the per-band
@@ -1329,22 +953,8 @@ band_kernel(const Params P, int64_t n, const double* __restrict__ rec,
   if (s >= n) return;
 
   const LeafPar L = load_leaf(P, s);
-#if SPART_BAND_SMEM_STATE
-  // soil and canopy state parked in shared memory (one column per thread, no synchronisation needed)
-  // and re-read per band right before use: 34 registers less live across the leaf model
-  __shared__ double s_st[17][kBandThreads];
-  SoilPar S = load_soil(P, rec, n, s);
-  CanopyGeo G = load_geo(P, rec, n, s);
-  {
-    const double v[17] = {S.f1, S.f2, S.f3, S.mu, S.emu, S.film, G.LAI, G.k, G.K, G.bf, G.sob, G.sof,
-                          G.tau_ss, G.tau_oo, G.sumpso, G.pso2w, G.Z};
-#pragma unroll
-    for (int i = 0; i < 17; ++i) s_st[i][threadIdx.x] = v[i];
-  }
-#else
-  const SoilPar S = load_soil(P, rec, n, s);
-  const CanopyGeo G = load_geo(P, rec, n, s);
-#endif
+  __shared__ double s_st[kStateRows][kBandThreads];
+  park_state(s_st, load_soil(P, rec, n, s), load_geo(P, rec, n, s));
   AtmSample A;
   AtmColumn C;
   if (kUniform) {
@@ -1354,23 +964,7 @@ band_kernel(const Params P, int64_t n, const double* __restrict__ rec,
     C.lpeq = rec[R_LPEQ * n + s];
     C.taup550 = P.at(P_AOT, s);
   } else {
-    A.us = rec[R_US * n + s];
-    A.uv = rec[R_UV * n + s];
-    A.m = rec[R_M * n + s];
-    A.Peq = rec[R_PEQ * n + s];
-    A.lo3 = rec[R_LO3 * n + s];
-    A.lh2o = rec[R_LH2O * n + s];
-    A.lm = rec[R_LM * n + s];
-    A.lpeq = rec[R_LPEQ * n + s];
-    A.cksi = rec[R_CKSI * n + s];
-    A.ksiD = rec[R_KSID * n + s];
-    A.ray_phase = rec[R_RAYPH * n + s];
-    A.taup550 = P.at(P_AOT, s);
-    A.inv_us = rec[R_INVUS * n + s];
-    A.inv_uv = rec[R_INVUV * n + s];
-    A.inv_1pus = rec[R_INV1PUS * n + s];
-    A.inv_1puv = rec[R_INV1PUV * n + s];
-    A.aa3 = rec[R_AA3 * n + s];
+    A = load_atm(P, rec, n, s);
   }
   const double etscale = rec[R_ETSCALE * n + s];
   // full output: [n][nb][3]; compact output (SPART_FLAG_COMPACT_OUT): [n][nb][2] followed by etscale[n]
@@ -1384,48 +978,13 @@ band_kernel(const Params P, int64_t n, const double* __restrict__ rec,
     // PROSPECT + BSM + SAILH at the one or two wavelengths np.interp touches (SPART.py:220-223)
     double rso = 0.0, rdo = 0.0, rsd = 0.0, rdd = 0.0;
     const int npts = (__double2hiint(bt[BT_NPTS]) >= 0x40000000) ? 2 : 1;   // 2.0 or 1.0, integer-pipe test
-#if SPART_BAND_PAIR && SPART_BAND_SMEM_STATE
-    if (npts == 2) {
-      const double* lc0 = &bt[BT_LC0];
-      const double* lc1 = &bt[BT_LC1];
-      double refl0, tran0, refl1, tran1, rwet0, rwet1;
-      prospect_point_nb(L, lc0, &s_tau, refl0, tran0);
-      prospect_point_nb(L, lc1, &s_tau, refl1, tran1);
-      volatile double(*st)[kBandThreads] = s_st;
-      const int t = threadIdx.x;
-      S.f1 = st[0][t]; S.f2 = st[1][t]; S.f3 = st[2][t]; S.mu = st[3][t]; S.emu = st[4][t]; S.film = st[5][t];
-      bsm_pair(S, lc0, lc1, rwet0, rwet1);
-      G.LAI = st[6][t]; G.k = st[7][t]; G.K = st[8][t]; G.bf = st[9][t]; G.sob = st[10][t]; G.sof = st[11][t];
-      G.tau_ss = st[12][t]; G.tau_oo = st[13][t]; G.sumpso = st[14][t]; G.pso2w = st[15][t]; G.Z = st[16][t];
-      double b0, b1, b2, b3;
-      sailh_point<true>(G, refl0, tran0, rwet0, rso, rdo, rsd, rdd);
-      sailh_point<true>(G, refl1, tran1, rwet1, b0, b1, b2, b3);
-      const double fr = bt[BT_FRAC];
-      rso = (b0 - rso) * fr + rso;
-      rdo = (b1 - rdo) * fr + rdo;
-      rsd = (b2 - rsd) * fr + rsd;
-      rdd = (b3 - rdd) * fr + rdd;
-    } else
-#endif
 #pragma unroll 1
     for (int pt = 0; pt < npts; ++pt) {
       const double* lc = &bt[BT_LC0 + pt * LC_COUNT];
       double refl, tran, kchl, rwet, rdry, a0, a1, a2, a3;
       prospect_point<false>(L, lc, &s_tau, refl, tran, kchl);
-#if SPART_BAND_SMEM_STATE
-      {
-        volatile double(*st)[kBandThreads] = s_st;
-        const int t = threadIdx.x;
-        S.f1 = st[0][t]; S.f2 = st[1][t]; S.f3 = st[2][t]; S.mu = st[3][t]; S.emu = st[4][t]; S.film = st[5][t];
-        bsm_point(S, lc, rwet, rdry);
-        G.LAI = st[6][t]; G.k = st[7][t]; G.K = st[8][t]; G.bf = st[9][t]; G.sob = st[10][t]; G.sof = st[11][t];
-        G.tau_ss = st[12][t]; G.tau_oo = st[13][t]; G.sumpso = st[14][t]; G.pso2w = st[15][t]; G.Z = st[16][t];
-        sailh_point(G, refl, tran, rwet, a0, a1, a2, a3);
-      }
-#else
-      bsm_point(S, lc, rwet, rdry);
-      sailh_point(G, refl, tran, rwet, a0, a1, a2, a3);
-#endif
+      bsm_point(reload_soil(s_st), lc, rwet, rdry);
+      sailh_point(reload_geo(s_st), refl, tran, rwet, a0, a1, a2, a3);
       if (pt == 0) {
         rso = a0; rdo = a1; rsd = a2; rdd = a3;
       } else {
@@ -1490,16 +1049,8 @@ band_kernel_srf(const Params P, int64_t n, const double* __restrict__ rec,
   const bool valid = s_raw < n;
   const int64_t s = valid ? s_raw : n - 1;
   const LeafPar L = load_leaf(P, s);
-  // soil and canopy state parked in a per-thread shared-memory column, as in band_kernel
-  __shared__ double s_st[17][kBandThreads];
-  SoilPar S = load_soil(P, rec, n, s);
-  CanopyGeo G = load_geo(P, rec, n, s);
-  {
-    const double v[17] = {S.f1, S.f2, S.f3, S.mu, S.emu, S.film, G.LAI, G.k, G.K, G.bf, G.sob, G.sof,
-                          G.tau_ss, G.tau_oo, G.sumpso, G.pso2w, G.Z};
-#pragma unroll
-    for (int i = 0; i < 17; ++i) s_st[i][t] = v[i];
-  }
+  __shared__ double s_st[kStateRows][kBandThreads];
+  park_state(s_st, load_soil(P, rec, n, s), load_geo(P, rec, n, s));
   const double etscale = rec[R_ETSCALE * n + s];
   const int nout = compact ? 2 : SPART_NOUT;
   if (compact && valid) out[(size_t)n * nb * 2 + s] = etscale;
@@ -1518,14 +1069,8 @@ band_kernel_srf(const Params P, int64_t n, const double* __restrict__ rec,
     for (int j = 0; j < m; ++j) {
       double refl, tran, kchl, rwet, rdry, a0, a1, a2, a3;
       prospect_point<false>(L, s_lc[j], &s_tau, refl, tran, kchl);
-      {
-        volatile double(*st)[kBandThreads] = s_st;
-        S.f1 = st[0][t]; S.f2 = st[1][t]; S.f3 = st[2][t]; S.mu = st[3][t]; S.emu = st[4][t]; S.film = st[5][t];
-        bsm_point(S, s_lc[j], rwet, rdry);
-        G.LAI = st[6][t]; G.k = st[7][t]; G.K = st[8][t]; G.bf = st[9][t]; G.sob = st[10][t]; G.sof = st[11][t];
-        G.tau_ss = st[12][t]; G.tau_oo = st[13][t]; G.sumpso = st[14][t]; G.pso2w = st[15][t]; G.Z = st[16][t];
-        sailh_point(G, refl, tran, rwet, a0, a1, a2, a3);
-      }
+      bsm_point(reload_soil(s_st), s_lc[j], rwet, rdry);
+      sailh_point(reload_geo(s_st), refl, tran, rwet, a0, a1, a2, a3);
       // add into every band that contains this wavelength (own column of the slot: no synchronisation)
 #pragma unroll 1
       for (int p = s_poff[j]; p < s_poff[j + 1]; ++p) {
@@ -1544,14 +1089,7 @@ band_kernel_srf(const Params P, int64_t n, const double* __restrict__ rec,
         const double rso = acc[0 * kBandThreads], rdo = acc[1 * kBandThreads], rsd = acc[2 * kBandThreads],
                      rdd = acc[3 * kBandThreads];
         acc[0 * kBandThreads] = acc[1 * kBandThreads] = acc[2 * kBandThreads] = acc[3 * kBandThreads] = 0.0;
-        AtmSample A;
-        A.us = rec[R_US * n + s]; A.uv = rec[R_UV * n + s]; A.m = rec[R_M * n + s]; A.Peq = rec[R_PEQ * n + s];
-        A.lo3 = rec[R_LO3 * n + s]; A.lh2o = rec[R_LH2O * n + s]; A.lm = rec[R_LM * n + s];
-        A.lpeq = rec[R_LPEQ * n + s];
-        A.cksi = rec[R_CKSI * n + s]; A.ksiD = rec[R_KSID * n + s]; A.ray_phase = rec[R_RAYPH * n + s];
-        A.taup550 = P.at(P_AOT, s);
-        A.inv_us = rec[R_INVUS * n + s]; A.inv_uv = rec[R_INVUV * n + s];
-        A.inv_1pus = rec[R_INV1PUS * n + s]; A.inv_1puv = rec[R_INV1PUV * n + s]; A.aa3 = rec[R_AA3 * n + s];
+        const AtmSample A = load_atm(P, rec, n, s);
         const double* bt = band_table + (size_t)b * BT_COUNT;
         double R_TOC, R_TOA, L_TOA;
         smac_toa_band(A, bt + BT_SMAC, __ldg(bt + BT_CONVEA), etscale, rso, rdo, rdd, rsd, R_TOC, R_TOA, L_TOA);
@@ -1578,14 +1116,7 @@ smac_kernel(const Params P, int64_t n, const double* __restrict__ rec,
   __syncthreads();
   const int64_t s = (int64_t)blockIdx.y * kBandThreads + threadIdx.x;
   if (s >= n) return;
-  AtmSample A;
-  A.us = rec[R_US * n + s]; A.uv = rec[R_UV * n + s]; A.m = rec[R_M * n + s]; A.Peq = rec[R_PEQ * n + s];
-  A.lo3 = rec[R_LO3 * n + s]; A.lh2o = rec[R_LH2O * n + s]; A.lm = rec[R_LM * n + s]; A.lpeq = rec[R_LPEQ * n + s];
-  A.cksi = rec[R_CKSI * n + s]; A.ksiD = rec[R_KSID * n + s]; A.ray_phase = rec[R_RAYPH * n + s];
-  A.taup550 = P.at(P_AOT, s);
-  A.inv_us = rec[R_INVUS * n + s]; A.inv_uv = rec[R_INVUV * n + s];
-  A.inv_1pus = rec[R_INV1PUS * n + s]; A.inv_1puv = rec[R_INV1PUV * n + s]; A.aa3 = rec[R_AA3 * n + s];
-  const AtmOptics O = smac_band(A, s_c);
+  const AtmOptics O = smac_band(load_atm(P, rec, n, s), s_c);
   double* o = out + (size_t)s * 9 * nb + b;
   o[0 * nb] = O.Ta_s;
   o[1 * nb] = O.Ta_o;
@@ -1623,8 +1154,8 @@ sailh_spectra_kernel(const Params P, int64_t n, const double* __restrict__ rec,
 // ---- FP32 mode (SPART_FP32) -----------------------------------------------------------------
 // Two kernels: per-sample geometry (leaf angles by safeguarded Newton, volume scattering,
 // hot-spot integrals, soil / atmosphere scalars) and the band kernel.  The per-sample record
-// is kept as float [R_COUNT][n] in the same workspace; parameters are read as double and
-// results are written as double.
+// is kept as float [R_COUNT][n] in the same workspace; parameters are read and results are
+// written as TIO: double, or float with SPART_FLAG_F32_IO.
 __constant__ float c_sin_ttli_f[13];
 __constant__ float c_cos_ttli_f[13];
 __constant__ float c_theta2_f[12];
@@ -2070,15 +1601,14 @@ int spart_device_count(void) {
 int spart_destroy(SpartCtx* ctx) {
   if (!ctx) return SPART_OK;
   DeviceGuard guard(ctx->device);
+  if (ctx->compute_stream) cudaStreamSynchronize(ctx->compute_stream);
   for (int i = 0; i < SpartCtx::kSlots; ++i) {
-    if (ctx->streams[i]) cudaStreamSynchronize(ctx->streams[i]);
     if (ctx->slot_rec[i]) cudaFree(ctx->slot_rec[i]);
     if (ctx->slot_out[i]) cudaFree(ctx->slot_out[i]);
     if (ctx->stage_in[i]) cudaFreeHost(ctx->stage_in[i]);
     if (ctx->stage_out[i]) cudaFreeHost(ctx->stage_out[i]);
     if (ctx->slot_done[i]) cudaEventDestroy(ctx->slot_done[i]);
     if (ctx->slot_k[i]) cudaEventDestroy(ctx->slot_k[i]);
-    if (ctx->streams[i]) cudaStreamDestroy(ctx->streams[i]);
   }
   for (int i = 0; i < SpartCtx::kInSlots; ++i) {
     if (ctx->in_params[i]) cudaFree(ctx->in_params[i]);
@@ -2090,6 +1620,7 @@ int spart_destroy(SpartCtx* ctx) {
   if (ctx->bc_stage) cudaFreeHost(ctx->bc_stage);
   if (ctx->h2d_stream) cudaStreamDestroy(ctx->h2d_stream);
   if (ctx->d2h_stream) cudaStreamDestroy(ctx->d2h_stream);
+  if (ctx->compute_stream) cudaStreamDestroy(ctx->compute_stream);
   if (ctx->join_stream) cudaStreamDestroy(ctx->join_stream);
   delete ctx->pool;
   for (auto& pe : ctx->prof_pending) for (int i = 0; i < 4; ++i) cudaEventDestroy(pe.e[i]);
@@ -2286,18 +1817,10 @@ static int launch_lidf(const Params& P, int64_t n_batch, double* ws, cudaStream_
   // LIDFa and LIDFb both broadcast rows (a look-up table with one leaf-angle distribution): the twelve
   // iterations run once, geometry_kernel reads element 0 of the F rows (kFlagLidfBcast)
   const int64_t n = ((P.bc & kLidfRows) == kLidfRows) ? 1 : n_batch;
-#if SPART_LIDF_V2
   const unsigned blocks = (unsigned)((n + kL2Samples - 1) / kL2Samples);
   lidf_kernel<<<blocks, kL2Threads, 0, st>>>(P.ptr(P_LIDFA, 0), P.ptr(P_LIDFB, 0),
                                                 ((P.bc >> P_LIDFA) & 1u) ? 0 : 1, ((P.bc >> P_LIDFB) & 1u) ? 0 : 1, n,
                                                 ws + (size_t)kRowF * n_batch, n_batch, 1);
-#else
-  const int64_t per_block = (int64_t)(kLidfThreads / 32) * kLidfSpw;
-  const unsigned blocks = (unsigned)((n + per_block - 1) / per_block);
-  lidf_kernel_v1<<<blocks, kLidfThreads, 0, st>>>(P.ptr(P_LIDFA, 0), P.ptr(P_LIDFB, 0),
-                                                 ((P.bc >> P_LIDFA) & 1u) ? 0 : 1, ((P.bc >> P_LIDFB) & 1u) ? 0 : 1, n,
-                                                 ws + (size_t)kRowF * n_batch, n_batch, 1);
-#endif
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   return SPART_OK;
@@ -2713,14 +2236,8 @@ int spart_leafangles(const double* ab_dev, int64_t n, int64_t ld, double* out_de
     if (rc) return rc;
   }
   NvtxRange r("spart::leaf_angles");
-#if SPART_LIDF_V2
   lidf_kernel<<<(unsigned)((n + kL2Samples - 1) / kL2Samples), kL2Threads, 0, (cudaStream_t)stream>>>(
       ab_dev, ab_dev + ld, 1, 1, n, out_dev, 1, 13);
-#else
-  const int64_t per_block = (int64_t)(kLidfThreads / 32) * kLidfSpw;
-  const unsigned blocks = (unsigned)((n + per_block - 1) / per_block);
-  lidf_kernel_v1<<<blocks, kLidfThreads, 0, (cudaStream_t)stream>>>(ab_dev, ab_dev + ld, 1, 1, n, out_dev, 1, 13);
-#endif
   ++g_launches;
   CUDA_TRY(cudaGetLastError());
   lidf_diff_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(out_dev, n);
@@ -2743,16 +2260,14 @@ static bool is_pinned_host(const void* p) {
 // output slots of `chunk` samples, pinned staging buffers for pageable caller memory
 static int ensure_slots(SpartCtx* ctx, int64_t span, int64_t chunk, size_t out_bytes, bool stage_in, bool stage_out) {
   const size_t in_bytes = sizeof(double) * P_COUNT * (size_t)span;
-  cudaStream_t* extra[3] = {&ctx->h2d_stream, &ctx->d2h_stream, &ctx->join_stream};
-  for (cudaStream_t* e : extra) {
+  cudaStream_t* streams[4] = {&ctx->h2d_stream, &ctx->d2h_stream, &ctx->compute_stream, &ctx->join_stream};
+  for (cudaStream_t* e : streams) {
     if (!*e) CUDA_TRY(cudaStreamCreateWithFlags(e, cudaStreamNonBlocking));
     CUDA_TRY(cudaStreamSynchronize(*e));
   }
   for (int i = 0; i < SpartCtx::kSlots; ++i) {
-    if (!ctx->streams[i]) CUDA_TRY(cudaStreamCreateWithFlags(&ctx->streams[i], cudaStreamNonBlocking));
     if (!ctx->slot_done[i]) CUDA_TRY(cudaEventCreateWithFlags(&ctx->slot_done[i], cudaEventDisableTiming));
     if (!ctx->slot_k[i]) CUDA_TRY(cudaEventCreateWithFlags(&ctx->slot_k[i], cudaEventDisableTiming));
-    CUDA_TRY(cudaStreamSynchronize(ctx->streams[i]));
     if (ctx->slot_cap < chunk) {
       if (ctx->slot_rec[i]) cudaFree(ctx->slot_rec[i]);
       ctx->slot_rec[i] = nullptr;
@@ -2841,8 +2356,10 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
   //   evaluated in place (params = span + offset, broadcast rows from the span's first elements, see ParamsT),
   //   so results start to flow back after the first chunk, not after the first span.
   // Streams: ONE per copy direction (each slot's own stream first carried its copies too: the host->device copy of
-  // a later chunk then queued behind the device->host copy of an earlier one), one compute stream per output
-  // slot and a join stream, tied together by events:
+  // a later chunk then queued behind the device->host copy of an earlier one), ONE compute stream (with a stream per
+  // output slot the chunks of a span share the SMs and finish together, a span's worth of kernel time after its
+  // copy; on one stream they finish one after the other and results flow back sooner) and a join stream, tied
+  // together by events:
   //   H2D(span j)  waits until the kernels of every chunk of span j - kInSlots have finished (join stream)
   //   kernels(i)   wait for H2D(span of i) and for D2H(i - kSlots)   (the slot's output buffer is free)
   //   D2H(i)       waits for kernels(i)
@@ -2925,7 +2442,7 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
     return SPART_OK;
   };
   auto run = [&]() -> int {
-    cudaStream_t sin = ctx->h2d_stream, sout = ctx->d2h_stream, sjoin = ctx->join_stream;
+    cudaStream_t sin = ctx->h2d_stream, sout = ctx->d2h_stream, st = ctx->compute_stream, sjoin = ctx->join_stream;
     bool in_used[SpartCtx::kInSlots] = {}, used[SpartCtx::kSlots] = {};
     int slot = 0;
     std::vector<int> fifo;       // pageable output: slots whose chunks are still to be copied out, oldest first
@@ -2952,7 +2469,6 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
     }
     // compact result in pinned memory: the etscale values travel once per span instead of once per chunk
     const bool ets_per_span = compact && !stage_out;
-    const bool single_compute = getenv("SPART_HOST_MULTI_COMPUTE") == nullptr;
     for (size_t j = 0; j < spans.size(); ++j) {
       const int islot = (int)(j % SpartCtx::kInSlots);
       const int64_t sp0 = spans[j].s0, sm = spans[j].m;
@@ -3001,9 +2517,6 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
       int64_t off = 0;
       for (size_t ci = 0; ci < sizes.size(); off += sizes[ci], ++ci, slot = (slot + 1) % SpartCtx::kSlots) {
         const int64_t m = sizes[ci], s0 = sp0 + off;
-        // one compute stream: the chunks of a span finish one after the other (on four streams they share the
-        // SMs and finish together, a span's worth of kernel time after its copy), so results flow back sooner
-        cudaStream_t st = ctx->streams[single_compute ? 0 : slot];
         int rc2 = unstage(slot);      // pageable output: the slot's previous chunk leaves its staging buffer
         if (rc2) return rc2;
         trace_new(m, slot, false);
@@ -3065,10 +2578,7 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
   // write the caller's memory) when it returns
   char keep[sizeof(g_err)];
   memcpy(keep, g_err, sizeof(keep));
-  for (int i = 0; i < SpartCtx::kSlots + 3; ++i) {
-    cudaStream_t sy = i < SpartCtx::kSlots ? ctx->streams[i]
-                                           : (i == SpartCtx::kSlots ? ctx->h2d_stream
-                                                                    : (i == SpartCtx::kSlots + 1 ? ctx->d2h_stream : ctx->join_stream));
+  for (cudaStream_t sy : {ctx->compute_stream, ctx->h2d_stream, ctx->d2h_stream, ctx->join_stream}) {
     const cudaError_t e = cudaStreamSynchronize(sy);
     if (e != cudaSuccess && rc == SPART_OK) {
       snprintf(keep, sizeof(keep), "cudaStreamSynchronize failed: %s", cudaGetErrorString(e));
