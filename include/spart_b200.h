@@ -101,7 +101,16 @@ enum {
    * distribution (spart_set_lidf on the same workspace and stream): LIDFa / LIDFb are ignored, the
    * leaf-angle kernel is skipped and the 13 values enter k, K, bf, sob, sof as they are -- what the
    * reference does with an assigned CanopyStructure.lidf (sailh.py:81-97 read canopy.lidf). */
-  SPART_FLAG_USER_LIDF = 64
+  SPART_FLAG_USER_LIDF = 64,
+  /* the context was created with a soil library (spart_create_with_soils): params row 9 (B) holds each
+   * sample's 0-based library index as a whole number in the row's element type, rows 10 and 11 (lat, lon)
+   * are ignored and rdry = library[index] -- a LUT whose entries each take one measured dry-soil spectrum,
+   * as the reference does with one SoilParametersFromFile per SPART object (bsm.py:42-43, 155-226).
+   * Row 9 may be a broadcast row.  An index that is not a whole number in [0, n_soils) (NaN included)
+   * gives NaN in every output that depends on the soil; nothing outside the library is read.  Excludes
+   * SPART_FLAG_SOIL_SPECTRUM; combines with every other flag.  Each sample's result equals bit for bit a
+   * run of that sample with SPART_FLAG_SOIL_SPECTRUM and the spectrum library[index]. */
+  SPART_FLAG_SOIL_LIBRARY = 128
 };
 
 /* elements of the result buffer of spart_forward_bands for n samples, nb bands and these flags */
@@ -154,6 +163,12 @@ int spart_device_count(void);
  * all sensors to `device` once.  *out must be released with spart_destroy. */
 int spart_create(const SpartTables* tables, const SpartSensor* sensors, int32_t n_sensors,
                  int32_t device, SpartCtx** out);
+/* spart_create plus a soil library for SPART_FLAG_SOIL_LIBRARY: soils is host memory, double
+ * [n_soils][SPART_NWL] (dry-soil reflectance on 400..2400 nm), uploaded once; 1 <= n_soils <= 2^24 (a float
+ * holds every whole number up to 2^24, so the index stays exact under SPART_FLAG_F32_IO).  The context
+ * serves runs without the flag exactly like one from spart_create. */
+int spart_create_with_soils(const SpartTables* tables, const SpartSensor* sensors, int32_t n_sensors,
+                            const double* soils, int32_t n_soils, int32_t device, SpartCtx** out);
 int spart_destroy(SpartCtx* ctx);
 
 /* Device scratch the caller must provide to the *_dev entry points for a batch of n samples. */
@@ -198,7 +213,8 @@ int spart_set_lidf(const double* lidf_dev, int64_t n, void* workspace_dev, void*
  *   (value at 2400 nm beyond)  5 rso  6 rdo  7 rsd  8 rdd.
  * rho_thermal / tau_thermal: leaf reflectance / transmittance beyond 2400 nm
  * (LeafBiology.rho_thermal / tau_thermal, prospect_5d.py:82-83, SPART.py:461-466; the reference's
- * default is 0.01 each).  flags: 0, SPART_FLAG_SOIL_SPECTRUM and / or SPART_FLAG_USER_LIDF. */
+ * default is 0.01 each).  flags: 0, SPART_FLAG_SOIL_SPECTRUM or SPART_FLAG_SOIL_LIBRARY (plane 4 is then the
+ * sample's library spectrum), and / or SPART_FLAG_USER_LIDF. */
 int spart_forward_spectrum(const SpartCtx* ctx, const double* params_dev, int64_t n, int64_t ld,
                            int32_t flags, double rho_thermal, double tau_thermal,
                            void* workspace_dev, double* out_dev, void* stream);

@@ -163,9 +163,8 @@ struct SoilParF {
   float f1, f2, f3, mu, emu, film;
 };
 
-// bsm.py:49-52, 99-124 at one wavelength
-__device__ __forceinline__ float bsm_point_f(const SoilParF& S, const float* lc) {
-  const float rdry = S.f1 * lc[LC_GSV0] + S.f2 * lc[LC_GSV1] + S.f3 * lc[LC_GSV2];
+// bsm.py:99-124 at one wavelength: wet soil from a given dry reflectance
+__device__ __forceinline__ float bsm_wet_f(const SoilParF& S, const float* lc, float rdry) {
   if (!(S.mu > 0.0f)) return rdry;
   const float rbac = 1.0f - (1.0f - rdry) * (rdry * lc[LC_SOILC1] + 1.0f - rdry);
   const float p = lc[LC_SOILP], Rw = lc[LC_SOILRW];
@@ -182,6 +181,11 @@ __device__ __forceinline__ float bsm_point_f(const SoilParF& S, const float* lc)
     acc += (Rw + g * x * rcp(1.0f - p * x)) * fk;
   }
   return acc;
+}
+
+// bsm.py:49-52, 99-124 at one wavelength
+__device__ __forceinline__ float bsm_point_f(const SoilParF& S, const float* lc) {
+  return bsm_wet_f(S, lc, S.f1 * lc[LC_GSV0] + S.f2 * lc[LC_GSV1] + S.f3 * lc[LC_GSV2]);
 }
 
 struct CanopyGeoF {

@@ -12,6 +12,8 @@
 //        chunk of <= 16 bands: PROSPECT + BSM + SAILH at the 1-2 wavelengths np.interp touches,
 //        SMAC, TOC->TOA; <true> = all samples share the sun / view geometry)
 //   params + rec    --spectrum_kernel-> spec [n][9][2162]   (leafopt/soilopt/canopyopt; thread = wavelength)
+//   (soillib_* = the band / spectrum kernels with each sample's dry soil read from a soil library,
+//    SPART_FLAG_SOIL_LIBRARY)
 //
 // In band_kernel / spectrum_kernel all lanes of a warp work on the same wavelength, so the
 // per-wavelength and per-band constants are warp-uniform shared-memory broadcasts and the
@@ -176,7 +178,11 @@ struct SpartCtx {
   int sm_count = 0;
   double* d_lc = nullptr;               // [LC_COUNT][SPART_NWL]
   std::vector<double*> d_band;          // per sensor [nb][BT_COUNT]
+  std::vector<int32_t*> d_knot;         // per sensor [nb][2]: wl_lo, wl_hi (read by the soil-library kernels)
   std::vector<int> n_bands;
+  // optional soil library (spart_create_with_soils): [n_soils + 1][SPART_NWL], the extra last row all NaN
+  double* d_soils = nullptr;
+  int n_soils = 0;
   // optional SRF tables per sensor (band_mode "srf"): per band the number of non-zero weights and
   // its offset into the concatenated (wavelength index, normalised weight) lists; nullptr when
   // the sensor was created without them
@@ -909,23 +915,74 @@ __device__ __forceinline__ CanopyGeo reload_geo(volatile double (*st)[kBandThrea
   return G;
 }
 
+// Dry-soil source of the band-path kernels (the `Soil` parameter of their bodies below).
+//   GsvSoil:     the record's soil-vector weights times the context's three GSV vectors -- the B / lat / lon
+//                model, or a user spectrum in GSV0 with weights (1, 0, 0) (SPART_FLAG_SOIL_SPECTRUM).
+//   LibrarySoil: row `index` of the context's soil library, index = params row 9 (SPART_FLAG_SOIL_LIBRARY).  The
+//                geometry kernels then run with SPART_FLAG_SOIL_SPECTRUM, so the record is that of a user spectrum
+//                and, since 1 * x + 0 * y + 0 * z == x, every sample equals bit for bit a run with
+//                soil_spectrum = its library row.  The index is read from params, not from the record, so
+//                SPART_FLAG_REUSE_RECORD works unchanged.
+// `wl` is the index into 400..2400 nm of the wavelength whose constants `lc` holds; GsvSoil does not need it.
+struct SoilLib {                // device view of a context's soil library
+  const double* rows;           // [k + 1][SPART_NWL]; row k is all NaN
+  int k;
+};
+
+struct GsvSoil {
+  static constexpr bool kLibrary = false;
+  template <typename T>
+  __device__ __forceinline__ static GsvSoil select(const ParamsT<T>&, int64_t, const SoilLib&) { return {}; }
+  __device__ __forceinline__ void point(const SoilPar& S, const double* lc, int, double& rwet, double& rdry) const {
+    bsm_point(S, lc, rwet, rdry);
+  }
+  __device__ __forceinline__ float point_f(const spart::f32::SoilParF& S, const float* lc, int) const {
+    return spart::f32::bsm_point_f(S, lc);
+  }
+};
+
+struct LibrarySoil {
+  static constexpr bool kLibrary = true;
+  const double* row;
+  // An index that is not a whole number in [0, k) (NaN included) selects the NaN row: the address stays inside the
+  // library and every soil-dependent output of the sample is NaN.  float -> double is exact, so F32_IO indices
+  // are judged the same way.
+  template <typename T>
+  __device__ __forceinline__ static LibrarySoil select(const ParamsT<T>& P, int64_t s, const SoilLib& lib) {
+    const double v = (double)P.at(P_B, s);
+    const bool ok = v >= 0.0 && v < (double)lib.k && v == trunc(v);
+    return {lib.rows + (size_t)(ok ? (int)v : lib.k) * SPART_NWL};
+  }
+  __device__ __forceinline__ void point(const SoilPar& S, const double* lc, int wl, double& rwet, double& rdry) const {
+    rdry = __ldg(row + wl);
+    bsm_wet(S, lc, rdry, rwet);
+  }
+  __device__ __forceinline__ float point_f(const spart::f32::SoilParF& S, const float* lc, int wl) const {
+    return spart::f32::bsm_wet_f(S, lc, (float)__ldg(row + wl));
+  }
+};
+
 // One thread per sample, looping over a chunk of up to kBandChunk bands; blockIdx.x = band
 // chunk, blockIdx.y = sample tile.  The per-sample state (leaf, soil, canopy geometry, SMAC
 // scalars: 44 doubles) is read from HBM once per chunk and kept in registers; the per-band
-// constants are warp-uniform shared-memory broadcasts.
-template <bool kUniform>
-__global__ void __launch_bounds__(kBandThreads, kUniform ? SPART_BAND_MINBLOCKS_U : SPART_BAND_MINBLOCKS)
-band_kernel(const Params P, int64_t n, const double* __restrict__ rec,
-            const double* __restrict__ band_table, int nb, double* __restrict__ out, int compact) {
+// constants are warp-uniform shared-memory broadcasts.  knots: [nb][2] wavelength indices of the
+// band's np.interp knots, read by LibrarySoil only.
+template <bool kUniform, class Soil>
+__device__ __forceinline__ void band_body(const Params& P, int64_t n, const double* __restrict__ rec,
+                                          const double* __restrict__ band_table, int nb, double* __restrict__ out,
+                                          int compact, const SoilLib& lib, const int32_t* __restrict__ knots) {
   __shared__ TauTable s_tau;
   __shared__ double s_bt[kBandChunk][BT_COUNT];
   __shared__ double s_ug[kUniform ? kBandChunk : 1][UG_COUNT];
+  __shared__ int s_knot[Soil::kLibrary ? kBandChunk : 1][2];
   const int b0 = blockIdx.x * kBandChunk;
   const int nbc = min(kBandChunk, nb - b0);
   load_tau_table(&s_tau);
   exp_table_load();
   for (int i = threadIdx.x; i < nbc * BT_COUNT; i += blockDim.x)
     (&s_bt[0][0])[i] = band_table[(size_t)b0 * BT_COUNT + i];
+  if (Soil::kLibrary)
+    for (int i = threadIdx.x; i < nbc * 2; i += blockDim.x) (&s_knot[0][0])[i] = knots[(size_t)b0 * 2 + i];
   __syncthreads();
   if (kUniform) {
     // all samples share the geometry: fold it into per-band constants, one thread per band,
@@ -953,6 +1010,7 @@ band_kernel(const Params P, int64_t n, const double* __restrict__ rec,
   if (s >= n) return;
 
   const LeafPar L = load_leaf(P, s);
+  const Soil soil = Soil::select(P, s, lib);
   __shared__ double s_st[kStateRows][kBandThreads];
   park_state(s_st, load_soil(P, rec, n, s), load_geo(P, rec, n, s));
   AtmSample A;
@@ -983,7 +1041,7 @@ band_kernel(const Params P, int64_t n, const double* __restrict__ rec,
       const double* lc = &bt[BT_LC0 + pt * LC_COUNT];
       double refl, tran, kchl, rwet, rdry, a0, a1, a2, a3;
       prospect_point<false>(L, lc, &s_tau, refl, tran, kchl);
-      bsm_point(reload_soil(s_st), lc, rwet, rdry);
+      soil.point(reload_soil(s_st), lc, Soil::kLibrary ? s_knot[bi][pt] : 0, rwet, rdry);
       sailh_point(reload_geo(s_st), refl, tran, rwet, a0, a1, a2, a3);
       if (pt == 0) {
         rso = a0; rdo = a1; rsd = a2; rdd = a3;
@@ -1005,6 +1063,21 @@ band_kernel(const Params P, int64_t n, const double* __restrict__ rec,
     o[bi * nout + 1] = R_TOA;
     if (!compact) o[bi * nout + 2] = L_TOA;
   }
+}
+
+template <bool kUniform>
+__global__ void __launch_bounds__(kBandThreads, kUniform ? SPART_BAND_MINBLOCKS_U : SPART_BAND_MINBLOCKS)
+band_kernel(const Params P, int64_t n, const double* __restrict__ rec,
+            const double* __restrict__ band_table, int nb, double* __restrict__ out, int compact) {
+  band_body<kUniform, GsvSoil>(P, n, rec, band_table, nb, out, compact, SoilLib{nullptr, 0}, nullptr);
+}
+
+// band_kernel with the dry soil of each sample taken from the soil library (SPART_FLAG_SOIL_LIBRARY)
+template <bool kUniform>
+__global__ void __launch_bounds__(kBandThreads, kUniform ? SPART_BAND_MINBLOCKS_U : SPART_BAND_MINBLOCKS)
+soillib_bands(const Params P, int64_t n, const double* __restrict__ rec, const double* __restrict__ band_table,
+              int nb, double* __restrict__ out, int compact, const SoilLib lib, const int32_t* __restrict__ knots) {
+  band_body<kUniform, LibrarySoil>(P, n, rec, band_table, nb, out, compact, lib, knots);
 }
 
 // Band kernel of the SRF mode (SPART_FLAG_SRF_BANDS): the four canopy reflectances of a band are
@@ -1033,10 +1106,11 @@ struct SrfPlan {               // device pointers, built by spart_create
   const int32_t* fin_slot;
 };
 
-__global__ void __launch_bounds__(kBandThreads, SPART_SRF_MINBLOCKS)
-band_kernel_srf(const Params P, int64_t n, const double* __restrict__ rec,
-                const double* __restrict__ band_table, const double* __restrict__ lc_table, const SrfPlan plan,
-                int nb, double* __restrict__ out, int compact) {
+template <class Soil>
+__device__ __forceinline__ void srf_body(const Params& P, int64_t n, const double* __restrict__ rec,
+                                         const double* __restrict__ band_table, const double* __restrict__ lc_table,
+                                         const SrfPlan& plan, int nb, double* __restrict__ out, int compact,
+                                         const SoilLib& lib) {
   extern __shared__ double s_acc[];            // [n_slots][4][kBandThreads]
   __shared__ TauTable s_tau;
   __shared__ double s_lc[kSrfChunk][LC_COUNT];
@@ -1049,6 +1123,7 @@ band_kernel_srf(const Params P, int64_t n, const double* __restrict__ rec,
   const bool valid = s_raw < n;
   const int64_t s = valid ? s_raw : n - 1;
   const LeafPar L = load_leaf(P, s);
+  const Soil soil = Soil::select(P, s, lib);
   __shared__ double s_st[kStateRows][kBandThreads];
   park_state(s_st, load_soil(P, rec, n, s), load_geo(P, rec, n, s));
   const double etscale = rec[R_ETSCALE * n + s];
@@ -1069,7 +1144,7 @@ band_kernel_srf(const Params P, int64_t n, const double* __restrict__ rec,
     for (int j = 0; j < m; ++j) {
       double refl, tran, kchl, rwet, rdry, a0, a1, a2, a3;
       prospect_point<false>(L, s_lc[j], &s_tau, refl, tran, kchl);
-      bsm_point(reload_soil(s_st), s_lc[j], rwet, rdry);
+      soil.point(reload_soil(s_st), s_lc[j], Soil::kLibrary ? __ldg(plan.wl_idx + c0 + j) : 0, rwet, rdry);
       sailh_point(reload_geo(s_st), refl, tran, rwet, a0, a1, a2, a3);
       // add into every band that contains this wavelength (own column of the slot: no synchronisation)
 #pragma unroll 1
@@ -1102,6 +1177,21 @@ band_kernel_srf(const Params P, int64_t n, const double* __restrict__ rec,
       }
     }
   }
+}
+
+__global__ void __launch_bounds__(kBandThreads, SPART_SRF_MINBLOCKS)
+band_kernel_srf(const Params P, int64_t n, const double* __restrict__ rec,
+                const double* __restrict__ band_table, const double* __restrict__ lc_table, const SrfPlan plan,
+                int nb, double* __restrict__ out, int compact) {
+  srf_body<GsvSoil>(P, n, rec, band_table, lc_table, plan, nb, out, compact, SoilLib{nullptr, 0});
+}
+
+// band_kernel_srf with the dry soil of each sample taken from the soil library (SPART_FLAG_SOIL_LIBRARY)
+__global__ void __launch_bounds__(kBandThreads, SPART_SRF_MINBLOCKS)
+soillib_srf(const Params P, int64_t n, const double* __restrict__ rec, const double* __restrict__ band_table,
+            const double* __restrict__ lc_table, const SrfPlan plan, int nb, double* __restrict__ out, int compact,
+            const SoilLib lib) {
+  srf_body<LibrarySoil>(P, n, rec, band_table, lc_table, plan, nb, out, compact, lib);
 }
 
 // SMAC alone (the reference's SMAC(angles, atm, coefs), smac.py:14-213): the nine
@@ -1301,24 +1391,28 @@ geometry_kernel_f32(const ParamsT<TIO> P, int64_t n, float* __restrict__ rec, in
   }
 }
 
-template <typename TIO>
-__global__ void __launch_bounds__(kBandThreads)
-band_kernel_f32(const ParamsT<TIO> P, int64_t n, const float* __restrict__ rec,
-                const double* __restrict__ band_table, int nb, TIO* __restrict__ out, int compact) {
+template <typename TIO, class Soil>
+__device__ __forceinline__ void band_body_f32(const ParamsT<TIO>& P, int64_t n, const float* __restrict__ rec,
+                                              const double* __restrict__ band_table, int nb, TIO* __restrict__ out,
+                                              int compact, const SoilLib& lib, const int32_t* __restrict__ knots) {
   using namespace spart::f32;
   __shared__ TauTableF s_tau;
   __shared__ float s_bt[kBandChunk][BT_COUNT];
+  __shared__ int s_knot[Soil::kLibrary ? kBandChunk : 1][2];
   const int b0 = blockIdx.x * kBandChunk;
   const int nbc = min(kBandChunk, nb - b0);
   load_tau_table_f(&s_tau);
   exp_table_load();       // the FP64 Stokes solve of near-conservative leaves uses the table-driven exp
   for (int i = threadIdx.x; i < nbc * BT_COUNT; i += blockDim.x)
     (&s_bt[0][0])[i] = (float)band_table[(size_t)b0 * BT_COUNT + i];
+  if (Soil::kLibrary)
+    for (int i = threadIdx.x; i < nbc * 2; i += blockDim.x) (&s_knot[0][0])[i] = knots[(size_t)b0 * 2 + i];
   __syncthreads();
   const int64_t s = (int64_t)blockIdx.y * kBandThreads + threadIdx.x;
   if (s >= n) return;
 
   const LeafParF L = load_leaf_f(P, s);
+  const Soil soil = Soil::select(P, s, lib);
   SoilParF S;
   S.f1 = rec[R_F1 * n + s]; S.f2 = rec[R_F2 * n + s]; S.f3 = rec[R_F3 * n + s];
   S.mu = rec[R_MU * n + s]; S.emu = rec[R_EMU * n + s]; S.film = (float)P.at(P_FILM, s);
@@ -1350,7 +1444,7 @@ band_kernel_f32(const ParamsT<TIO> P, int64_t n, const float* __restrict__ rec,
       const float* lc = &bt[BT_LC0 + pt * LC_COUNT];
       float refl, tran, absorb, a0, a1, a2, a3;
       prospect_point_f(L, lc, &s_tau, refl, tran, absorb);
-      const float rwet = bsm_point_f(S, lc);
+      const float rwet = soil.point_f(S, lc, Soil::kLibrary ? s_knot[bi][pt] : 0);
       sailh_point_f(G, refl, tran, absorb, rwet, a0, a1, a2, a3);
       if (pt == 0) {
         rso = a0; rdo = a1; rsd = a2; rdd = a3;
@@ -1370,16 +1464,31 @@ band_kernel_f32(const ParamsT<TIO> P, int64_t n, const float* __restrict__ rec,
   }
 }
 
+template <typename TIO>
+__global__ void __launch_bounds__(kBandThreads)
+band_kernel_f32(const ParamsT<TIO> P, int64_t n, const float* __restrict__ rec,
+                const double* __restrict__ band_table, int nb, TIO* __restrict__ out, int compact) {
+  band_body_f32<TIO, GsvSoil>(P, n, rec, band_table, nb, out, compact, SoilLib{nullptr, 0}, nullptr);
+}
+
+// band_kernel_f32 with the dry soil of each sample taken from the soil library (SPART_FLAG_SOIL_LIBRARY)
+template <typename TIO>
+__global__ void __launch_bounds__(kBandThreads)
+soillib_bands_f32(const ParamsT<TIO> P, int64_t n, const float* __restrict__ rec, const double* __restrict__ band_table,
+                  int nb, TIO* __restrict__ out, int compact, const SoilLib lib, const int32_t* __restrict__ knots) {
+  band_body_f32<TIO, LibrarySoil>(P, n, rec, band_table, nb, out, compact, lib, knots);
+}
+
 // Full-spectrum planes (leafopt / soilopt / canopyopt): thread = wavelength, blockIdx.y = sample.
 // Every load of the per-wavelength constants and every store of the nine output planes is then
 // coalesced along the wavelength axis (the output is 155 KB per sample, so this kernel lives on
 // its store pattern); the sample's parameters and record are warp-uniform broadcast loads.
 constexpr int kSpecThreads = 256;
 
-__global__ void __launch_bounds__(kSpecThreads)
-spectrum_kernel(const Params P, int64_t n, const double* __restrict__ rec,
-                const double* __restrict__ lc_table, int64_t s0, double rho_thermal, double tau_thermal,
-                double* __restrict__ out) {
+template <class Soil>
+__device__ __forceinline__ void spectrum_body(const Params& P, int64_t n, const double* __restrict__ rec,
+                                              const double* __restrict__ lc_table, int64_t s0, double rho_thermal,
+                                              double tau_thermal, double* __restrict__ out, const SoilLib& lib) {
   __shared__ TauTable s_tau;
   load_tau_table(&s_tau);
   exp_table_load();
@@ -1395,7 +1504,7 @@ spectrum_kernel(const Params P, int64_t n, const double* __restrict__ rec,
 #pragma unroll
   for (int r = 0; r < LC_COUNT; ++r) lc[r] = lc_table[(size_t)r * SPART_NWL + wc];
   double refl, tran, kchl, rwet, rdry, rso, rdo, rsd, rdd;
-  bsm_point(S, lc, rwet, rdry);
+  Soil::select(P, s, lib).point(S, lc, wc, rwet, rdry);
   if (w < SPART_NWL) {
     prospect_point<true>(L, lc, &s_tau, refl, tran, kchl);
   } else {  // thermal assumptions (SPART.py:461-466): LeafBiology.rho_thermal / tau_thermal
@@ -1414,6 +1523,20 @@ spectrum_kernel(const Params P, int64_t n, const double* __restrict__ rec,
   o[6 * SPART_NWL_S] = rdo;
   o[7 * SPART_NWL_S] = rsd;
   o[8 * SPART_NWL_S] = rdd;
+}
+
+__global__ void __launch_bounds__(kSpecThreads)
+spectrum_kernel(const Params P, int64_t n, const double* __restrict__ rec,
+                const double* __restrict__ lc_table, int64_t s0, double rho_thermal, double tau_thermal,
+                double* __restrict__ out) {
+  spectrum_body<GsvSoil>(P, n, rec, lc_table, s0, rho_thermal, tau_thermal, out, SoilLib{nullptr, 0});
+}
+
+// spectrum_kernel with the dry soil of each sample taken from the soil library (SPART_FLAG_SOIL_LIBRARY)
+__global__ void __launch_bounds__(kSpecThreads)
+soillib_spectrum(const Params P, int64_t n, const double* __restrict__ rec, const double* __restrict__ lc_table,
+                 int64_t s0, double rho_thermal, double tau_thermal, double* __restrict__ out, const SoilLib lib) {
+  spectrum_body<LibrarySoil>(P, n, rec, lc_table, s0, rho_thermal, tau_thermal, out, lib);
 }
 
 // ---- peak micro-benchmarks ---------------------------------------------------------------
@@ -1626,6 +1749,8 @@ int spart_destroy(SpartCtx* ctx) {
   for (auto& pe : ctx->prof_pending) for (int i = 0; i < 4; ++i) cudaEventDestroy(pe.e[i]);
   for (auto& pe : ctx->prof_free) for (int i = 0; i < 4; ++i) cudaEventDestroy(pe.e[i]);
   for (double* d : ctx->d_band) cudaFree(d);
+  for (int32_t* d : ctx->d_knot) cudaFree(d);
+  if (ctx->d_soils) cudaFree(ctx->d_soils);
   for (auto& v : ctx->srf) {
     cudaFree(v.wl_idx); cudaFree(v.pair_off); cudaFree(v.pair_slot); cudaFree(v.fin_off); cudaFree(v.fin_band);
     cudaFree(v.fin_slot); cudaFree(v.pair_w);
@@ -1738,13 +1863,23 @@ extern "C" {
 
 // body of spart_create; on any failure the caller releases the partially built context
 static int create_into(SpartCtx* ctx, const SpartTables* tables, const SpartSensor* sensors, int32_t n_sensors,
-                       int32_t device) {
+                       const double* soils, int32_t n_soils, int32_t device) {
   CUDA_TRY(cudaDeviceGetAttribute(&ctx->sm_count, cudaDevAttrMultiProcessorCount, device));
   int rc = init_device_constants(device);
   if (rc) return rc;
   const size_t lc_bytes = sizeof(double) * LC_COUNT * SPART_NWL;
   CUDA_TRY(cudaMalloc(&ctx->d_lc, lc_bytes));
   CUDA_TRY(cudaMemcpy(ctx->d_lc, tables->lc, lc_bytes, cudaMemcpyHostToDevice));
+  if (soils) {
+    // the library plus one row of NaN that invalid sample indices are pointed at
+    const size_t lib_bytes = sizeof(double) * (size_t)n_soils * SPART_NWL;
+    const std::vector<double> nan_row(SPART_NWL, __builtin_nan(""));
+    CUDA_TRY(cudaMalloc(&ctx->d_soils, lib_bytes + sizeof(double) * SPART_NWL));
+    CUDA_TRY(cudaMemcpy(ctx->d_soils, soils, lib_bytes, cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(ctx->d_soils + (size_t)n_soils * SPART_NWL, nan_row.data(), sizeof(double) * SPART_NWL,
+                        cudaMemcpyHostToDevice));
+    ctx->n_soils = n_soils;
+  }
 
   for (int i = 0; i < n_sensors; ++i) {
     const SpartSensor& S = sensors[i];
@@ -1762,10 +1897,18 @@ static int create_into(SpartCtx* ctx, const SpartTables* tables, const SpartSens
     }
     // every vector gets its slot first, so that spart_destroy releases whatever was allocated
     ctx->d_band.push_back(nullptr);
+    ctx->d_knot.push_back(nullptr);
     ctx->n_bands.push_back(S.n_bands);
     ctx->srf.emplace_back();
     CUDA_TRY(cudaMalloc(&ctx->d_band[i], bt.size() * sizeof(double)));
     CUDA_TRY(cudaMemcpy(ctx->d_band[i], bt.data(), bt.size() * sizeof(double), cudaMemcpyHostToDevice));
+    std::vector<int32_t> knots((size_t)S.n_bands * 2);
+    for (int b = 0; b < S.n_bands; ++b) {
+      knots[(size_t)b * 2] = S.wl_lo[b];
+      knots[(size_t)b * 2 + 1] = S.wl_hi[b];
+    }
+    rc = upload(knots, &ctx->d_knot[i]);
+    if (rc) return rc;
     if (S.srf_idx && S.srf_len && S.srf_w) {
       rc = build_srf_plan(S, ctx->srf[i]);
       if (rc) return rc;
@@ -1774,8 +1917,8 @@ static int create_into(SpartCtx* ctx, const SpartTables* tables, const SpartSens
   return SPART_OK;
 }
 
-int spart_create(const SpartTables* tables, const SpartSensor* sensors, int32_t n_sensors, int32_t device,
-                 SpartCtx** out) {
+static int create_ctx(const SpartTables* tables, const SpartSensor* sensors, int32_t n_sensors, const double* soils,
+                      int32_t n_soils, int32_t device, SpartCtx** out) {
   if (!tables || !tables->lc || !out || n_sensors < 0 || (n_sensors > 0 && !sensors))
     return fail(SPART_EINVAL, "spart_create: null argument%s");
   if (tables->n_wl != SPART_NWL) return fail(SPART_EINVAL, "spart_create: tables->n_wl must be 2001%s");
@@ -1795,7 +1938,7 @@ int spart_create(const SpartTables* tables, const SpartSensor* sensors, int32_t 
   if (!ctx) return fail(SPART_ENOMEM, "spart_create: out of host memory%s");
   ctx->device = device;
   ctx->n_sensors = n_sensors;
-  const int rc = create_into(ctx, tables, sensors, n_sensors, device);
+  const int rc = create_into(ctx, tables, sensors, n_sensors, soils, n_soils, device);
   if (rc) {
     char keep[sizeof(g_err)];
     memcpy(keep, g_err, sizeof(keep));      // spart_destroy must not disturb the error text
@@ -1805,6 +1948,19 @@ int spart_create(const SpartTables* tables, const SpartSensor* sensors, int32_t 
   }
   *out = ctx;
   return SPART_OK;
+}
+
+int spart_create(const SpartTables* tables, const SpartSensor* sensors, int32_t n_sensors, int32_t device,
+                 SpartCtx** out) {
+  return create_ctx(tables, sensors, n_sensors, nullptr, 0, device, out);
+}
+
+int spart_create_with_soils(const SpartTables* tables, const SpartSensor* sensors, int32_t n_sensors,
+                            const double* soils, int32_t n_soils, int32_t device, SpartCtx** out) {
+  if (!soils) return fail(SPART_EINVAL, "spart_create_with_soils: null soil library%s");
+  // F32_IO carries the index as a float, which holds every whole number only up to 2^24
+  if (n_soils < 1 || n_soils > (1 << 24)) return fail(SPART_EINVAL, "spart_create_with_soils: need 1 <= n_soils <= 2^24%s");
+  return create_ctx(tables, sensors, n_sensors, soils, n_soils, device, out);
 }
 
 size_t spart_workspace_bytes(const SpartCtx* ctx, int64_t n) {
@@ -1846,7 +2002,22 @@ static int check_batch(const SpartCtx* ctx, const void* params, int64_t n, int64
 }
 
 static const int kKnownFlags = SPART_FLAG_SOIL_SPECTRUM | SPART_FLAG_SRF_BANDS | SPART_FLAG_REUSE_RECORD |
-                               SPART_FLAG_F32_IO | SPART_FLAG_COMPACT_OUT | SPART_FLAG_USER_LIDF;
+                               SPART_FLAG_F32_IO | SPART_FLAG_COMPACT_OUT | SPART_FLAG_USER_LIDF |
+                               SPART_FLAG_SOIL_LIBRARY;
+
+// SPART_FLAG_SOIL_LIBRARY needs a context with a library and excludes SPART_FLAG_SOIL_SPECTRUM
+static int check_soil_library(const SpartCtx* ctx, int32_t flags, const char* who) {
+  if (!(flags & SPART_FLAG_SOIL_LIBRARY)) return SPART_OK;
+  if (flags & SPART_FLAG_SOIL_SPECTRUM)
+    return fail(SPART_EINVAL, "%s: SPART_FLAG_SOIL_LIBRARY and SPART_FLAG_SOIL_SPECTRUM exclude each other", who);
+  if (!ctx->d_soils) return fail(SPART_EINVAL, "%s: SPART_FLAG_SOIL_LIBRARY needs a context created with a soil library", who);
+  return SPART_OK;
+}
+
+// the geometry kernels see a library run as a user-spectrum run: soil weights (1, 0, 0)
+static int soil_kflags(int32_t flags) {
+  return (flags & (SPART_FLAG_SOIL_SPECTRUM | SPART_FLAG_SOIL_LIBRARY)) ? SPART_FLAG_SOIL_SPECTRUM : 0;
+}
 
 // flag / precision combinations shared by the device and the host entry point
 static int check_mode(const SpartCtx* ctx, int32_t sensor, int32_t precision, int32_t flags, const char* who) {
@@ -1864,14 +2035,15 @@ static int check_mode(const SpartCtx* ctx, int32_t sensor, int32_t precision, in
     if (precision != SPART_FP64) return fail(SPART_EINVAL, "%s: SRF band mode needs SPART_FP64", who);
     if (!ctx->srf[sensor].pair_w) return fail(SPART_EINVAL, "%s: this sensor was created without SRF tables", who);
   }
-  return SPART_OK;
+  return check_soil_library(ctx, flags, who);
 }
 
 }  // extern "C"
 
 template <typename TIO>
 static int launch_fp32(const SpartCtx* ctx, int sensor, const void* params_dev, const void* params_bc_dev, int64_t n,
-                       int64_t ld, uint32_t bc, int kflags, bool reuse, bool compact, float* rec, void* out_dev,
+                       int64_t ld, uint32_t bc, int kflags, bool reuse, bool compact, bool library, float* rec,
+                       void* out_dev,
                        dim3 grid, cudaStream_t st, bool prof, const SpartCtx::ProfEvents& pe) {
   const ParamsT<TIO> P{(const TIO*)params_dev, ld, bc, (const TIO*)params_bc_dev};
   if (prof) CUDA_TRY(cudaEventRecord(pe.e[1], st));
@@ -1884,8 +2056,13 @@ static int launch_fp32(const SpartCtx* ctx, int sensor, const void* params_dev, 
   }
   if (prof) CUDA_TRY(cudaEventRecord(pe.e[2], st));
   NvtxRange r("spart::bands_f32");
-  band_kernel_f32<TIO><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], ctx->n_bands[sensor],
-                                                      (TIO*)out_dev, compact ? 1 : 0);
+  if (library)
+    soillib_bands_f32<TIO><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], ctx->n_bands[sensor],
+                                                          (TIO*)out_dev, compact ? 1 : 0,
+                                                          SoilLib{ctx->d_soils, ctx->n_soils}, ctx->d_knot[sensor]);
+  else
+    band_kernel_f32<TIO><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], ctx->n_bands[sensor],
+                                                        (TIO*)out_dev, compact ? 1 : 0);
   return SPART_OK;
 }
 
@@ -1923,7 +2100,9 @@ static int forward_bands_impl(const SpartCtx* ctx, int32_t sensor, const void* p
   // one sun / observer geometry for the whole batch by construction: rows 19..21 are broadcast rows
   const bool uniform = (broadcast_rows & kGeometryRows) == kGeometryRows;
   const bool user_lidf = (flags & SPART_FLAG_USER_LIDF) != 0;   // the workspace holds the caller's distribution
-  const int kflags = (flags & SPART_FLAG_SOIL_SPECTRUM) | (uniform ? kFlagUniform : 0) | (user_lidf ? kFlagLidfDirect : 0);
+  const bool library = (flags & SPART_FLAG_SOIL_LIBRARY) != 0;    // per-sample dry soil from the context's library
+  const SoilLib lib{ctx->d_soils, ctx->n_soils};
+  const int kflags = soil_kflags(flags) | (uniform ? kFlagUniform : 0) | (user_lidf ? kFlagLidfDirect : 0);
   if (prof) CUDA_TRY(cudaEventRecord(pe.e[0], st));
   if (precision == SPART_FP64) {
     const Params P{(const double*)params_dev, ld, broadcast_rows, (const double*)params_bc_dev};
@@ -1946,10 +2125,25 @@ static int forward_bands_impl(const SpartCtx* ctx, int32_t sensor, const void* p
       const SrfPlan plan{v.n_wl, v.n_slots, v.wl_idx, v.pair_off, v.pair_slot, v.pair_w, v.fin_off, v.fin_band,
                          v.fin_slot};
       const size_t acc_bytes = sizeof(double) * v.n_slots * 4 * kBandThreads;
-      if (acc_bytes > 16 * 1024)
-        CUDA_TRY(cudaFuncSetAttribute(band_kernel_srf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)acc_bytes));
-      band_kernel_srf<<<(unsigned)((n + kBandThreads - 1) / kBandThreads), kBandThreads, acc_bytes, st>>>(
-          P, n, rec, ctx->d_band[sensor], ctx->d_lc, plan, nb, out, compact ? 1 : 0);
+      const unsigned blocks = (unsigned)((n + kBandThreads - 1) / kBandThreads);
+      if (library) {
+        if (acc_bytes > 16 * 1024)
+          CUDA_TRY(cudaFuncSetAttribute(soillib_srf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)acc_bytes));
+        soillib_srf<<<blocks, kBandThreads, acc_bytes, st>>>(P, n, rec, ctx->d_band[sensor], ctx->d_lc, plan, nb, out,
+                                                             compact ? 1 : 0, lib);
+      } else {
+        if (acc_bytes > 16 * 1024)
+          CUDA_TRY(cudaFuncSetAttribute(band_kernel_srf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)acc_bytes));
+        band_kernel_srf<<<blocks, kBandThreads, acc_bytes, st>>>(P, n, rec, ctx->d_band[sensor], ctx->d_lc, plan, nb,
+                                                                 out, compact ? 1 : 0);
+      }
+    } else if (library) {
+      if (uniform)
+        soillib_bands<true><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], nb, out, compact ? 1 : 0,
+                                                           lib, ctx->d_knot[sensor]);
+      else
+        soillib_bands<false><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], nb, out, compact ? 1 : 0,
+                                                            lib, ctx->d_knot[sensor]);
     } else if (uniform) {
       band_kernel<true><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], nb, out, compact ? 1 : 0);
     } else {
@@ -1957,10 +2151,10 @@ static int forward_bands_impl(const SpartCtx* ctx, int32_t sensor, const void* p
     }
   } else {   // SPART_FP32: the leaf angles are solved inside the geometry kernel
     if (flags & SPART_FLAG_F32_IO)
-      rc = launch_fp32<float>(ctx, sensor, params_dev, params_bc_dev, n, ld, broadcast_rows, kflags, reuse, compact, (float*)rec,
+      rc = launch_fp32<float>(ctx, sensor, params_dev, params_bc_dev, n, ld, broadcast_rows, kflags, reuse, compact, library, (float*)rec,
                               out_dev, grid, st, prof, pe);
     else
-      rc = launch_fp32<double>(ctx, sensor, params_dev, params_bc_dev, n, ld, broadcast_rows, kflags, reuse, compact, (float*)rec,
+      rc = launch_fp32<double>(ctx, sensor, params_dev, params_bc_dev, n, ld, broadcast_rows, kflags, reuse, compact, library, (float*)rec,
                                out_dev, grid, st, prof, pe);
     if (rc) return rc;
   }
@@ -2017,8 +2211,10 @@ int spart_forward_spectrum(const SpartCtx* ctx, const double* params_dev, int64_
                            void* stream) {
   int rc = check_batch(ctx, params_dev, n, ld, 0, workspace_dev, out_dev, "spart_forward_spectrum");
   if (rc) return rc;
-  if (flags & ~(SPART_FLAG_SOIL_SPECTRUM | SPART_FLAG_USER_LIDF))
+  if (flags & ~(SPART_FLAG_SOIL_SPECTRUM | SPART_FLAG_USER_LIDF | SPART_FLAG_SOIL_LIBRARY))
     return fail(SPART_EINVAL, "spart_forward_spectrum: unknown flag bit%s");
+  rc = check_soil_library(ctx, flags, "spart_forward_spectrum");
+  if (rc) return rc;
   if (n == 0) return SPART_OK;
   GUARD_DEVICE(ctx->device);
   NvtxRange r("spart::spectrum");
@@ -2030,12 +2226,16 @@ int spart_forward_spectrum(const SpartCtx* ctx, const double* params_dev, int64_
     rc = launch_lidf(P, n, rec, st);
     if (rc) return rc;
   }
-  rc = launch_geometry(P, n, rec, (flags & SPART_FLAG_SOIL_SPECTRUM) | (user_lidf ? kFlagLidfDirect : 0), st);
+  rc = launch_geometry(P, n, rec, soil_kflags(flags) | (user_lidf ? kFlagLidfDirect : 0), st);
   if (rc) return rc;
   for (int64_t s0 = 0; s0 < n; s0 += 65535) {
     const unsigned ny = (unsigned)((n - s0 < 65535) ? (n - s0) : 65535);
     dim3 grid((SPART_NWL_S + kSpecThreads - 1) / kSpecThreads, ny);
-    spectrum_kernel<<<grid, kSpecThreads, 0, st>>>(P, n, rec, ctx->d_lc, s0, rho_thermal, tau_thermal, out_dev);
+    if (flags & SPART_FLAG_SOIL_LIBRARY)
+      soillib_spectrum<<<grid, kSpecThreads, 0, st>>>(P, n, rec, ctx->d_lc, s0, rho_thermal, tau_thermal, out_dev,
+                                                      SoilLib{ctx->d_soils, ctx->n_soils});
+    else
+      spectrum_kernel<<<grid, kSpecThreads, 0, st>>>(P, n, rec, ctx->d_lc, s0, rho_thermal, tau_thermal, out_dev);
     ++g_launches;
     CUDA_TRY(cudaGetLastError());
   }

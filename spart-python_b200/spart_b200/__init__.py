@@ -10,13 +10,14 @@ from . import lut
 from .engine import CompactBands, Engine, default_engine
 from .model import SPART, SpectralBands, load_optical_parameters, load_sensor_info
 from .params import (Angles, AtmosphericProperties, CanopyStructure, LeafBiology, SoilParameters,
-                     SoilParametersFromFile, pack_params)
+                     SoilLibrary, SoilParametersFromFile, pack_params)
 from .stages import (BSM, PROSPECT_5D, SAILH, SMAC, bsm_batch, prospect_batch, sailh_batch, smac_batch,
                      set_leaf_refl_trans_assumptions, set_soil_refl_trans_assumptions)
 from .tables import SENSOR_NAMES, synthetic_fullspectrum_sensorinfo
 
 __all__ = [
-    "SPART", "SpectralBands", "LeafBiology", "SoilParameters", "SoilParametersFromFile", "CanopyStructure", "Angles",
+    "SPART", "SpectralBands", "LeafBiology", "SoilParameters", "SoilParametersFromFile", "SoilLibrary",
+    "CanopyStructure", "Angles",
     "AtmosphericProperties", "run_batch", "run_batch_params", "pack_batch", "pack_params",
     "row_as_dataframe", "lut", "Engine", "CompactBands", "default_engine", "SpartError", "SENSOR_NAMES",
     "load_optical_parameters", "load_sensor_info", "synthetic_fullspectrum_sensorinfo",

@@ -19,6 +19,7 @@ FLAG_REUSE_RECORD = 8
 FLAG_F32_IO = 16
 FLAG_COMPACT_OUT = 32
 FLAG_USER_LIDF = 64
+FLAG_SOIL_LIBRARY = 128
 NKERNELS = 3
 NPAR = 27
 # rows 19..21 (sun zenith, observer zenith, relative azimuth) as broadcast rows = one geometry for
@@ -29,7 +30,8 @@ FP64 = 64
 FP32 = 32
 
 EXPORTS = (
-    "spart_abi_version", "spart_last_error", "spart_device_count", "spart_create", "spart_destroy",
+    "spart_abi_version", "spart_last_error", "spart_device_count", "spart_create", "spart_create_with_soils",
+    "spart_destroy",
     "spart_workspace_bytes", "spart_forward_bands", "spart_forward_bands_host", "spart_forward_spectrum",
     "spart_smac", "spart_sailh", "spart_lut_workspace_bytes", "spart_lut_nearest", "spart_lut_nearest_tc", "spart_lut_unpack",
     "spart_leafangles", "spart_set_lidf", "spart_profile_enable", "spart_profile_read", "spart_measure_peaks", "spart_measure_fp64_chain", "spart_launch_count",
@@ -75,6 +77,8 @@ def load():
     lib.spart_last_error.restype = c_char_p
     lib.spart_device_count.restype = ctypes.c_int
     lib.spart_create.argtypes = [POINTER(SpartTables), POINTER(SpartSensor), c_int32, c_int32, POINTER(c_void_p)]
+    lib.spart_create_with_soils.argtypes = [POINTER(SpartTables), POINTER(SpartSensor), c_int32, POINTER(c_double),
+                                            c_int32, c_int32, POINTER(c_void_p)]
     lib.spart_destroy.argtypes = [c_void_p]
     lib.spart_workspace_bytes.argtypes = [c_void_p, c_int64]
     lib.spart_workspace_bytes.restype = c_size_t

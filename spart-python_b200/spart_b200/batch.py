@@ -88,7 +88,7 @@ def _pro_warning(params):
 
 def run_batch_params(params, sensor, precision="fp64", device=None, out=None, uniform_geometry=False,
                      soil_spectrum=None, band_mode="interp", broadcast_rows=0, compact=False, warn=False,
-                     lidf=None):
+                     lidf=None, soil_library=None):
     """params: [27, n] float64 (float32 with precision="fp32": float32 in, float32 out).  CUDA tensor
     in -> CUDA tensor [n, nb, 3] out (asynchronous on the current stream); NumPy array / CPU tensor
     in -> NumPy array out (copies pipelined in the C library).
@@ -99,6 +99,9 @@ def run_batch_params(params, sensor, precision="fp64", device=None, out=None, un
     result is the same to a few ulp, only faster.
     soil_spectrum: dry-soil reflectance [2001] shared by the batch (the reference's
     SoilParametersFromFile, bsm.py:155-226); the B / lat / lon rows are then ignored.
+    soil_library: a SoilLibrary of measured dry-soil spectra, one selected per sample: row 9 (B) holds the
+    sample's 0-based index into the library (a broadcast row 9 selects one spectrum for the batch), rows 10, 11
+    are ignored.  An index that is not a whole number in [0, k) gives NaN soil-dependent outputs.
     band_mode="srf" replaces the reference's np.interp band sampling of the canopy reflectances by
     the sensor's spectral-response-weighted band means (FP64 only).
     compact=True returns a CompactBands (R_TOC, R_TOA and the per-sample ET scale; L_TOA is rebuilt
@@ -109,7 +112,7 @@ def run_batch_params(params, sensor, precision="fp64", device=None, out=None, un
     if warn:
         _pro_warning(params)
     kw = dict(precision=precision, uniform_geometry=uniform_geometry, soil_spectrum=soil_spectrum,
-              band_mode=band_mode, broadcast_rows=broadcast_rows, compact=compact)
+              soil_library=soil_library, band_mode=band_mode, broadcast_rows=broadcast_rows, compact=compact)
     if isinstance(sensor, (list, tuple)):      # several sensors on one batch (e.g. Sentinel-2A + -2B)
         if not (isinstance(params, torch.Tensor) and params.is_cuda):
             eng = default_engine(device)
@@ -135,9 +138,13 @@ def run_batch_params(params, sensor, precision="fp64", device=None, out=None, un
 
 
 def run_batch(leaf, soil, canopy, angles, atm, doy, sensor, precision="fp64", device=None, out=None,
-              soil_spectrum=None, band_mode="interp", compact=False):
+              soil_spectrum=None, band_mode="interp", compact=False, soil_library=None, soil_index=None):
     """Batched SPART forward run -> [n, nb, 3] ordered (R_TOC, R_TOA, L_TOA).  Arguments given in
-    their short forms (angles [3], scalar doy, leaf [n, 7], soil [n, 4]) become broadcast rows."""
+    their short forms (angles [3], scalar doy, leaf [n, 7], soil [n, 4]) become broadcast rows.
+    soil_library (a SoilLibrary) with soil_index ([n] 0-based indices, or one index for the whole batch):
+    every sample takes its dry-soil spectrum from the library; soil's B / lat / lon columns are then ignored."""
+    if (soil_library is None) != (soil_index is None):
+        raise ValueError("soil_library and soil_index go together")
     ndim = lambda x: x.dim() if hasattr(x, "dim") else np.ndim(x)
     width = lambda x: x.shape[1] if ndim(x) == 2 else None
     rows = []
@@ -151,8 +158,16 @@ def run_batch(leaf, soil, canopy, angles, atm, doy, sensor, precision="fp64", de
         rows += [13, 14]               # SMC = 25, film = 0.015
         _warn_once("smc", "BSM soil model: SMC not supplied, set to default of 25 %")
         _warn_once("film", "BSM soil model: water film optical thickness not supplied, set to default of 0.0150 cm")
-    return run_batch_params(pack_batch(leaf, soil, canopy, angles, atm, doy, device), sensor, precision, device, out,
-                            soil_spectrum=soil_spectrum, band_mode=band_mode, broadcast_rows=rows, compact=compact,
+    params = pack_batch(leaf, soil, canopy, angles, atm, doy, device)
+    if soil_index is not None:
+        if ndim(soil_index) == 0:
+            rows += [9]
+        if isinstance(params, torch.Tensor):
+            params[9] = torch.as_tensor(soil_index, dtype=torch.float64, device=params.device)
+        else:
+            params[9] = np.asarray(soil_index, dtype=np.float64)
+    return run_batch_params(params, sensor, precision, device, out, soil_spectrum=soil_spectrum,
+                            soil_library=soil_library, band_mode=band_mode, broadcast_rows=rows, compact=compact,
                             warn=True)
 
 

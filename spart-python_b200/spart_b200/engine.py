@@ -13,13 +13,14 @@ import torch
 
 from . import _lib
 from . import tables as T
+from .params import SoilLibrary
 
 NPAR = 27
 NOUT = 3
 NSPEC = 9
 NWL_S = 2162
 MAX_SAMPLES_PER_CALL = 65535 * 128    # grid.y limit of band_kernel, see spart_forward_bands
-MAX_CONTEXTS = 32                     # cached (sensor, soil spectrum) contexts per engine
+MAX_CONTEXTS = 32                     # cached (sensor, soil spectrum or library) contexts per engine
 
 _PRECISION = {"fp64": _lib.FP64, 64: _lib.FP64, "fp32": _lib.FP32, 32: _lib.FP32}
 
@@ -113,20 +114,29 @@ class Engine:
         self._lock = threading.Lock()
 
     # ---- contexts ------------------------------------------------------------------
-    def sensor(self, sensor, soil_spectrum=None):
+    def sensor(self, sensor, soil_spectrum=None, soil_library=None):
         """(ctx, SensorTables) for a shipped sensor name or a reference-style sensorinfo dict.
         Custom dicts are keyed by the content of every array the hot path uses (so an edited dict
         is a new sensor).  soil_spectrum: optional user dry-soil reflectance [2001]
         (SoilParametersFromFile); such a context carries the spectrum as its first soil vector and
-        must be run with SPART_FLAG_SOIL_SPECTRUM.  At most MAX_CONTEXTS contexts are kept; the least
-        recently used one is destroyed (its device tables are freed) when a new one is needed."""
+        must be run with SPART_FLAG_SOIL_SPECTRUM.  soil_library: optional SoilLibrary, uploaded once
+        into the context (spart_create_with_soils) for runs with SPART_FLAG_SOIL_LIBRARY; keyed by its
+        content digest.  At most MAX_CONTEXTS contexts are kept; the least recently used one is
+        destroyed (its device tables are freed) when a new one is needed."""
         skey = sensor if isinstance(sensor, str) else ("custom", _sensor_digest(sensor))
         soil = None
+        if soil_spectrum is not None and soil_library is not None:
+            raise ValueError("soil_spectrum and soil_library exclude each other")
+        if soil_library is not None and not isinstance(soil_library, SoilLibrary):
+            raise TypeError("soil_library must be a SoilLibrary")
         if soil_spectrum is not None:
             soil = np.ascontiguousarray(np.asarray(soil_spectrum, dtype=np.float64).reshape(-1))
             if soil.shape[0] != T.NWL:
                 raise ValueError("soil_spectrum must have 2001 values (400..2400 nm)")
-        key = (skey, None if soil is None else hashlib.sha1(soil.tobytes()).hexdigest())
+        if soil_library is not None:
+            key = (skey, ("lib", soil_library.digest))
+        else:
+            key = (skey, None if soil is None else hashlib.sha1(soil.tobytes()).hexdigest())
         with self._lock:
             hit = self._ctx.get(key)
             if hit is not None:
@@ -146,8 +156,15 @@ class Engine:
                                   srf_len=_lib.as_int32_ptr(st.srf_len), srf_idx=_lib.as_int32_ptr(st.srf_idx),
                                   srf_w=_lib.as_double_ptr(st.srf_w))
             handle = _lib.c_void_p()
-            _lib.check(self.lib.spart_create(_lib.byref(tabs), _lib.byref(cs), 1, self.device.index,
-                                             _lib.byref(handle)), "spart_create")
+            if soil_library is None:
+                _lib.check(self.lib.spart_create(_lib.byref(tabs), _lib.byref(cs), 1, self.device.index,
+                                                 _lib.byref(handle)), "spart_create")
+            else:
+                lib_rows = soil_library.spectra
+                _lib.check(self.lib.spart_create_with_soils(_lib.byref(tabs), _lib.byref(cs), 1,
+                                                            _lib.as_double_ptr(lib_rows), lib_rows.shape[0],
+                                                            self.device.index, _lib.byref(handle)),
+                           "spart_create_with_soils")
             while len(self._ctx) >= MAX_CONTEXTS:
                 _, (old, _, _) = self._ctx.popitem(last=False)
                 self.lib.spart_destroy(old)
@@ -193,10 +210,11 @@ class Engine:
         return mask | _lib.GEOMETRY_ROWS
 
     @staticmethod
-    def _flags(soil_spectrum, band_mode, f32_io=False, compact=False, reuse=False):
+    def _flags(soil_spectrum, band_mode, f32_io=False, compact=False, reuse=False, soil_library=None):
         if band_mode not in ("interp", "srf"):
             raise ValueError("band_mode must be 'interp' or 'srf'")
         return ((_lib.FLAG_SOIL_SPECTRUM if soil_spectrum is not None else 0)
+                | (_lib.FLAG_SOIL_LIBRARY if soil_library is not None else 0)
                 | (_lib.FLAG_SRF_BANDS if band_mode == "srf" else 0)
                 | (_lib.FLAG_F32_IO if f32_io else 0) | (_lib.FLAG_COMPACT_OUT if compact else 0)
                 | (_lib.FLAG_REUSE_RECORD if reuse else 0))
@@ -218,14 +236,17 @@ class Engine:
 
     def forward_bands(self, params, sensor, out=None, precision="fp64", uniform_geometry=False,
                       soil_spectrum=None, band_mode="interp", broadcast_rows=0, compact=False,
-                      reuse_record=False, workspace=None, lidf=None):
+                      reuse_record=False, workspace=None, lidf=None, soil_library=None):
         """params: CUDA float64 [27, n] -> CUDA float64 [n, nb, 3] = (R_TOC, R_TOA, L_TOA).
         Asynchronous on the current torch stream.
 
         broadcast_rows: bit mask / iterable of rows that are constant over the batch (only their
         element 0 is read).  uniform_geometry=True: the three angle rows are verified to be constant
         and passed as broadcast rows (raises SpartError otherwise).  soil_spectrum: dry soil
-        reflectance [2001] used instead of the B/lat/lon soil vectors.  band_mode: "interp" (the
+        reflectance [2001] used instead of the B/lat/lon soil vectors.  soil_library: a SoilLibrary;
+        row 9 (B) then holds each sample's index into it (a broadcast row 9 gives the whole batch one
+        spectrum) and rows 10, 11 are ignored; an index that is not a whole number in [0, k) gives NaN
+        soil-dependent outputs.  Excludes soil_spectrum.  band_mode: "interp" (the
         reference: np.interp at the band centre) or "srf" (SRF-weighted band means).
         precision="fp32" with float32 params: float32 in, float32 out (SPART_FLAG_F32_IO).
         compact=True: returns a CompactBands (R_TOC, R_TOA + etscale; two thirds of the bytes).
@@ -234,11 +255,11 @@ class Engine:
         lidf: a leaf inclination distribution [n, 13] (or one row for the whole batch) used instead of the one
         derived from LIDFa / LIDFb -- the reference's assigned `CanopyStructure.lidf`; FP64 only."""
         prec = _PRECISION[precision]
-        handle, st = self.sensor(sensor, soil_spectrum)
+        handle, st = self.sensor(sensor, soil_spectrum, soil_library)
         params, n, ld = self._prep(params, allow_f32=(prec == _lib.FP32))
         f32_io = params.dtype == torch.float32
         mask = self._geometry_mask(params, n, _lib.row_mask(broadcast_rows), uniform_geometry)
-        flags = self._flags(soil_spectrum, band_mode, f32_io, compact, reuse_record)
+        flags = self._flags(soil_spectrum, band_mode, f32_io, compact, reuse_record, soil_library)
         if lidf is not None:
             if prec != _lib.FP64 or reuse_record or n > MAX_SAMPLES_PER_CALL:
                 raise ValueError("lidf= needs precision='fp64', no reuse_record and at most "
@@ -267,7 +288,8 @@ class Engine:
         return CompactBands(out, n, nb, st.conv_ea, prec == _lib.FP32) if compact else out
 
     def forward_bands_multi(self, params, sensors, outs=None, precision="fp64", uniform_geometry=False,
-                            soil_spectrum=None, band_mode="interp", broadcast_rows=0, compact=False):
+                            soil_spectrum=None, band_mode="interp", broadcast_rows=0, compact=False,
+                            soil_library=None):
         """One batch evaluated for several sensors: the sensor-independent per-sample kernels run
         once and every further sensor only runs the band kernel (SPART_FLAG_REUSE_RECORD).
         Returns a list of results as forward_bands would."""
@@ -279,20 +301,23 @@ class Engine:
         res = []
         for i, s in enumerate(sensors):
             res.append(self.forward_bands(params, s, out=None if outs is None else outs[i], precision=precision,
-                                          soil_spectrum=soil_spectrum, band_mode=band_mode, broadcast_rows=mask,
+                                          soil_spectrum=soil_spectrum, soil_library=soil_library,
+                                          band_mode=band_mode, broadcast_rows=mask,
                                           compact=compact, reuse_record=i > 0, workspace=ws))
         return res
 
-    def forward_spectrum(self, params, out=None, soil_spectrum=None, rho_thermal=0.01, tau_thermal=0.01, lidf=None):
+    def forward_spectrum(self, params, out=None, soil_spectrum=None, rho_thermal=0.01, tau_thermal=0.01, lidf=None,
+                         soil_library=None):
         """params: CUDA float64 [27, n] -> CUDA float64 [n, 9, 2162]: leaf refl, leaf tran,
         kChlrel, soil refl, soil refl dry, rso, rdo, rsd, rdd.  rho_thermal / tau_thermal: leaf
-        reflectance / transmittance beyond 2400 nm (LeafBiology.rho_thermal / tau_thermal)."""
-        handle, _ = self.sensor("Sentinel2A-MSI", soil_spectrum)   # any context carries the wavelength tables
+        reflectance / transmittance beyond 2400 nm (LeafBiology.rho_thermal / tau_thermal).
+        soil_spectrum / soil_library as in forward_bands."""
+        handle, _ = self.sensor("Sentinel2A-MSI", soil_spectrum, soil_library)   # any context carries the wavelength tables
         params, n, ld = self._prep(params)
         if out is None:
             out = torch.empty((n, NSPEC, NWL_S), dtype=torch.float64, device=self.device)
         ws = self.workspace(n)
-        flags = _lib.FLAG_SOIL_SPECTRUM if soil_spectrum is not None else 0
+        flags = self._flags(soil_spectrum, "interp", soil_library=soil_library)
         with torch.cuda.device(self.device):
             stream = torch.cuda.current_stream(self.device).cuda_stream
             if lidf is not None:
@@ -354,13 +379,14 @@ class Engine:
 
     # ---- host path -----------------------------------------------------------------
     def forward_bands_host(self, params, sensor, out=None, precision="fp64", uniform_geometry=False,
-                           soil_spectrum=None, band_mode="interp", broadcast_rows=0, compact=False):
+                           soil_spectrum=None, band_mode="interp", broadcast_rows=0, compact=False,
+                           soil_library=None):
         """params: host float64 [27, n] (NumPy array or CPU tensor; float32 with precision="fp32") ->
         host array [n, nb, 3] of the same dtype (CompactBands when compact).  H2D, kernels and D2H are
         pipelined inside the C library; pinned memory is DMA'd directly, pageable memory is staged
         by the library's copy threads.  Other arguments as forward_bands."""
         prec = _PRECISION[precision]
-        handle, st = self.sensor(sensor, soil_spectrum)
+        handle, st = self.sensor(sensor, soil_spectrum, soil_library)
         p = params.numpy() if isinstance(params, torch.Tensor) else np.asarray(params)
         okdt = p.dtype == np.float64 or (p.dtype == np.float32 and prec == _lib.FP32)
         if not okdt or p.ndim != 2 or p.shape[0] != NPAR or (p.shape[1] > 1 and p.strides[1] != p.itemsize):
@@ -369,7 +395,7 @@ class Engine:
         n, nb = p.shape[1], st.n_bands
         ld = p.strides[0] // p.itemsize if n > 1 else max(n, 1)
         mask = self._geometry_mask(p, n, _lib.row_mask(broadcast_rows), uniform_geometry)
-        flags = self._flags(soil_spectrum, band_mode, p.dtype == np.float32, compact)
+        flags = self._flags(soil_spectrum, band_mode, p.dtype == np.float32, compact, soil_library=soil_library)
         elems = out_elems(n, nb, compact)
         if out is None:
             out = np.empty(elems if compact else (n, nb, NOUT), dtype=p.dtype)

@@ -12,20 +12,23 @@ from .engine import default_engine
 
 
 def generate(params, sensor, precision="fp64", chunk=1 << 20, out_dtype=torch.float32, column=None, path=None,
-             uniform_geometry=False):
+             uniform_geometry=False, soil_library=None):
     """params: [27, n] (NumPy or torch, host or device).  Evaluates the batch in chunks of `chunk`
     samples and returns a CUDA tensor [n, nb, 3] (or [n, nb] when `column` selects 0 = R_TOC,
     1 = R_TOA, 2 = L_TOA) in `out_dtype`.  With `path` the table is also written as a compressed
-    .npz holding `params` [n, 27] float32 and `lut`."""
+    .npz holding `params` [n, 27] float32 and `lut`.  soil_library: a SoilLibrary; row 9 of params then
+    holds each entry's index into it, so the stored params tell which soil the nearest entry of a
+    retrieval used."""
     eng = default_engine()
     p = params if isinstance(params, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(params))
     n = p.shape[1]
-    _, st = eng.sensor(sensor)
+    _, st = eng.sensor(sensor, soil_library=soil_library)
     shape = (n, st.n_bands) if column is not None else (n, st.n_bands, 3)
     lut = torch.empty(shape, dtype=out_dtype, device=eng.device)
     for s0 in range(0, n, chunk):
         blk = p[:, s0:s0 + chunk].to(eng.device, dtype=torch.float64).contiguous()
-        res = eng.forward_bands(blk, sensor, precision=precision, uniform_geometry=uniform_geometry)
+        res = eng.forward_bands(blk, sensor, precision=precision, uniform_geometry=uniform_geometry,
+                                soil_library=soil_library)
         lut[s0:s0 + chunk] = (res[..., column] if column is not None else res).to(out_dtype)
     if path is not None:
         np.savez_compressed(path, params=p.T.to(torch.float32).cpu().numpy(), lut=lut.cpu().numpy(),

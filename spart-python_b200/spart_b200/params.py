@@ -4,10 +4,12 @@ the reference's classes, so that user scripts written for wirrell/SPART-python r
   LeafBiology            reference src/SPART/prospect_5d.py:19-83
   SoilParameters         reference src/SPART/bsm.py:229-287
   SoilParametersFromFile reference src/SPART/bsm.py:155-226   (dry spectrum supplied by the user)
+  SoilLibrary            (new) many such spectra, one selected per sample of a batch
   CanopyStructure        reference src/SPART/sailh.py:304-348
   Angles                 reference src/SPART/sailh.py:275-301
   AtmosphericProperties  reference src/SPART/smac.py:275-330
 """
+import hashlib
 import math
 import warnings
 from dataclasses import dataclass
@@ -99,6 +101,52 @@ class SoilParametersFromFile:
 
     def as_row(self):
         return [0.0, 0.0, 0.0, self.SMp, self.SMC, self.film]      # B, lat, lon are not used
+
+
+class SoilLibrary:
+    """A library of k measured dry-soil spectra on the 400..2400 nm grid, for batches in which every sample
+    takes its own spectrum -- e.g. a look-up table whose entries each use one soil of the library, where the
+    reference builds one SoilParametersFromFile per SPART object.  Passed as `soil_library=` to the batched
+    entry points; row 9 (B) of the parameter block then holds each sample's 0-based index into the library
+    (rows 10, 11 are ignored).  An index that is not a whole number in [0, k) gives NaN soil outputs.
+
+    spectra: [k, 2001], or [k, 2001, 1] as stacked SoilParametersFromFile.rdry arrays; 1 <= k <= 2^24.
+    The library keeps a read-only float64 copy (`spectra`) and its content digest (`digest`)."""
+
+    MAX_SPECTRA = 1 << 24         # F32_IO carries the index as a float, which is exact for whole numbers up to 2^24
+
+    def __init__(self, spectra):
+        a = np.asarray(spectra, dtype=np.float64)
+        if a.ndim == 3 and a.shape[2] == 1:
+            a = a[:, :, 0]
+        if a.ndim != 2 or a.shape[1] != 2001:
+            raise ValueError(f"soil library spectra must be [k, 2001] (or [k, 2001, 1]), got {a.shape}")
+        if not 1 <= a.shape[0] <= self.MAX_SPECTRA:
+            raise ValueError(f"a soil library holds 1 to 2^24 spectra, got {a.shape[0]}")
+        a = np.array(a, dtype=np.float64, order="C")          # own copy
+        a.flags.writeable = False
+        self.spectra = a
+        self.digest = hashlib.sha1(a.tobytes()).hexdigest()
+
+    def __len__(self):
+        return self.spectra.shape[0]
+
+    @classmethod
+    def from_files(cls, paths):
+        """One spectrum per JPL spectral-library text file, read as SoilParametersFromFile does."""
+        return cls(np.stack([SoilParametersFromFile._load_jpl_soil_refl(p) for p in paths]))
+
+    @classmethod
+    def from_per_sample(cls, spectra):
+        """spectra [n, 2001] (one dry-soil spectrum per sample, e.g. the rdry of one SoilParametersFromFile per
+        sample) -> (library of the distinct spectra, index [n] float64) with library.spectra[index] == spectra."""
+        a = np.asarray(spectra, dtype=np.float64)
+        if a.ndim == 3 and a.shape[2] == 1:
+            a = a[:, :, 0]
+        if a.ndim != 2 or a.shape[1] != 2001:
+            raise ValueError(f"per-sample spectra must be [n, 2001], got {a.shape}")
+        uniq, index = np.unique(np.ascontiguousarray(a), axis=0, return_inverse=True)
+        return cls(uniq), index.reshape(-1).astype(np.float64)
 
 
 class CanopyStructure:
