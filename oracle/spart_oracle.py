@@ -433,9 +433,11 @@ def sailh(rs, rho, tau, canopy, angles, lidf=None, geo=None):
 
 
 # ------------------------------------------------------------------------------- SMAC
-def smac(angles, atm, coefs):
+def smac(angles, atm, coefs, terms=False):
     """SMAC (smac.py:14-213), batched: angles [n,3], atm [n,4] (aot550 uo3 uh2o Pa),
-    coefs = dict of [1, nb] arrays in their native dtype.  Returns dict of nine [n, nb]."""
+    coefs = dict of [1, nb] arrays in their native dtype.  Returns dict of nine [n, nb].
+    terms=True adds the summands the sums Ra_so, Ta_s and Ta_o are formed of (lists under "Ra_so_terms",
+    "Ta_s_terms", "Ta_o_terms"): what a test needs to judge how ill-conditioned those sums are."""
     angles = np.asarray(angles, dtype=np.float64)
     atm = np.asarray(atm, dtype=np.float64)
     tts, tto, psi = (angles[:, i:i + 1] for i in range(3))
@@ -516,8 +518,15 @@ def smac(angles, atm, coefs):
         tdir_ttv = np.exp(-tautot / uv)
         tdif_tts = ttetas - tdir_tts
         tdif_ttv = ttetav - tdir_ttv
-    return dict(Ta_s=ttetas, Ta_o=ttetav, Tg=tg, Ra_dd=s, Ra_so=atm_ref,
-                Ta_ss=tdir_tts, Ta_sd=tdif_tts, Ta_oo=tdir_ttv, Ta_do=tdif_ttv)
+    out = dict(Ta_s=ttetas, Ta_o=ttetav, Tg=tg, Ra_dd=s, Ra_so=atm_ref,
+               Ta_ss=tdir_tts, Ta_sd=tdif_tts, Ta_oo=tdir_ttv, Ta_do=tdif_ttv)
+    if terms:
+        with np.errstate(all="ignore"):
+            out["Ra_so_terms"] = [ray_ref, Res_ray, aer_ref1 / (us * uv), aer_ref2 / (us * uv), aer_ref3 / (us * uv),
+                                  Res_aer, Res_6s]
+            out["Ta_s_terms"] = [c["a0T"], c["a1T"] * taup550 / us, (c["a2T"] * Peq + c["a3T"]) / (1 + us)]
+            out["Ta_o_terms"] = [c["a0T"], c["a1T"] * taup550 / uv, (c["a2T"] * Peq + c["a3T"]) / (1 + uv)]
+    return out
 
 
 # ----------------------------------------------------- ET irradiance + SRF convolution

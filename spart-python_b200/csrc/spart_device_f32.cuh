@@ -64,9 +64,11 @@ __device__ __forceinline__ void load_tau_table_f(TauTableF* s) {
 }
 
 // tau(K) = (1-K) e^-K + K^2 E1(K), prospect_5d.py:182-196 (see plate_tau in spart_device.cuh).
-// Returns 1 - tau: for a weakly absorbing plate (K << 1) that is the quantity the leaf absorptance
-// hangs on, and it is formed without cancellation as (1 - e^-K) + K e^-K - K^2 E1(K).
-__device__ __forceinline__ float plate_one_minus_tau_f(float K, const TauTableF* tab) {
+// Returns tau and sets omt = 1 - tau, each formed where it has no cancellation.  For a weakly absorbing plate
+// (K < 1) 1 - tau is the quantity the leaf absorptance hangs on: (1 - e^-K) + K e^-K - K^2 E1(K).  For a strongly
+// absorbing one (K >= 1) tau = e^-K t H(t) is small (7e-11 at K = 21) and a float 1 - (1 - tau) would lose it, down
+// to 0 for K > ~14.5, where the N-layer solution then divides by zero.
+__device__ __forceinline__ float plate_tau_f(float K, const TauTableF* tab, float& omt) {
   const float emk = fexp(-K);
   int idx;
   float u, t = 0.0f;
@@ -86,9 +88,12 @@ __device__ __forceinline__ float plate_one_minus_tau_f(float K, const TauTableF*
   if (K < 1.0f) {
     const float e1 = fmaf(K, p, -0.57721566490153286061f - flog(K));
     const float ome = (K < 0.05f) ? K * (1.0f - K * (0.5f - K * (1.0f / 6.0f - K * (1.0f / 24.0f)))) : 1.0f - emk;
-    return fmaf(K, emk - K * e1, ome);
+    omt = fmaf(K, emk - K * e1, ome);
+    return 1.0f - omt;
   }
-  return 1.0f - emk * t * p;
+  const float tau = emk * t * p;
+  omt = 1.0f - tau;
+  return tau;
 }
 
 struct LeafParF {
@@ -123,9 +128,8 @@ __device__ __forceinline__ void prospect_point_f(const LeafParF& L, const float*
   const float Ksum = L.Cab * lc[LC_KAB] + L.Cca * lc[LC_KCA] + L.Cdm * lc[LC_KDM] + L.Cw * lc[LC_KW] +
                      L.Cs * lc[LC_KS] + L.Cant * lc[LC_KANT] + L.CBC * lc[LC_CBC] + L.PROT * lc[LC_PROT];
   const float Kall = Ksum * L.invN;
-  float omt = 0.0f;
-  if (Kall > 0.0f) omt = plate_one_minus_tau_f(Kall, tab);
-  const float tau = 1.0f - omt;
+  float omt = 0.0f, tau = 1.0f;
+  if (Kall > 0.0f) tau = plate_tau_f(Kall, tab, omt);
   const float t_alph = lc[LC_TALPH], t12 = lc[LC_T12], t21 = lc[LC_T21];
   const float r_alph = 1.0f - t_alph, r12 = 1.0f - t12, r21 = 1.0f - t21;
   const float tt21 = tau * t21;

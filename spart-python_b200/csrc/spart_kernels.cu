@@ -1095,7 +1095,7 @@ soillib_bands(const Params P, int64_t n, const double* __restrict__ rec, const d
 constexpr int kSrfChunk = 32;
 
 struct SrfPlan {               // device pointers, built by spart_create
-  int n_wl;                    // distinct wavelengths, ascending
+  int n_wl;                    // steps: distinct wavelengths, ascending, then one per band without SRF weight
   int n_slots;                 // accumulator slots (max. number of simultaneously open bands + 1 spare)
   const int32_t* wl_idx;       // [n_wl] index into 400..2400 nm
   const int32_t* pair_off;     // [n_wl + 1] offsets into pair_slot / pair_w
@@ -1821,8 +1821,9 @@ static int build_srf_plan(const SpartSensor& S, SpartCtx::SrfDev& dev) {
     }
     for (int b : ends[q]) free_slots.push_back(slot[b]);
   }
-  const int spare = n_slots++;          // never accumulated into: bands without any SRF sample read zeros from it
+  const int spare = n_slots++;          // only for bands without any SRF weight, see the end of the plan
   if (n_slots > kSrfMaxSlots) return fail(SPART_EINVAL, "spart_create: too many overlapping bands for the SRF band mode%s");
+  if (U == 0) return fail(SPART_EINVAL, "spart_create: SRF tables without a single sample%s");
   // per wavelength: pairs in ascending band order (each band's own sum keeps its ascending wavelength order)
   std::vector<std::vector<std::pair<int, double>>> pairs(U);
   for (int b = 0; b < nb; ++b)
@@ -1839,16 +1840,23 @@ static int build_srf_plan(const SpartSensor& S, SpartCtx::SrfDev& dev) {
       fin_band.push_back(b);
       fin_slot.push_back(slot[b]);
     }
-    if (q == U - 1)
-      for (int b = 0; b < nb; ++b)
-        if (last[b] < 0) {
-          fin_band.push_back(b);
-          fin_slot.push_back(spare);
-        }
     fin_off[q + 1] = (int32_t)fin_band.size();
   }
-  if (U == 0) return fail(SPART_EINVAL, "spart_create: SRF tables without a single sample%s");
-  dev.n_wl = U;
+  // A band without any SRF weight is 0 / 0 in calculate_spectral_convolution (SPART.py:389-396): its band
+  // reflectances, and with them R_TOC, R_TOA and L_TOA, are NaN.  Each such band gets one more step (a repeat
+  // of the last wavelength) that adds a NaN weight into the spare slot and finishes the band from there; the
+  // kernel needs no test of its own for it.
+  for (int b = 0; b < nb; ++b)
+    if (last[b] < 0) {
+      wl_idx.push_back(wl_idx[U - 1]);
+      pair_slot.push_back(spare);
+      pair_w.push_back(__builtin_nan(""));
+      pair_off.push_back((int32_t)pair_slot.size());
+      fin_band.push_back(b);
+      fin_slot.push_back(spare);
+      fin_off.push_back((int32_t)fin_band.size());
+    }
+  dev.n_wl = (int)wl_idx.size();
   dev.n_slots = n_slots;
   int rc;
   if ((rc = upload(wl_idx, &dev.wl_idx)) || (rc = upload(pair_off, &dev.pair_off)) ||
