@@ -185,6 +185,16 @@ int spart_forward_bands(const SpartCtx* ctx, int32_t sensor, const void* params_
                         int64_t n, int64_t ld, uint32_t broadcast_rows, int32_t precision,
                         int32_t flags, void* workspace_dev, void* out_dev, void* stream);
 
+/* spart_forward_bands with the broadcast rows read from a separate base: element 0 of broadcast row r
+ * is params_bc_dev[r * ld] (same element type and ld as params_dev), every other row is read from
+ * params_dev.  A caller that splits a batch of more than 65535 * 128 samples into calls passes
+ * params_dev = batch + first sample of the call and params_bc_dev = batch, so that every call reads the
+ * batch's own element 0 of each broadcast row; spart_forward_bands(..., p, ...) is
+ * spart_forward_bands_bc(..., p, p, ...).  params_bc_dev must not be NULL. */
+int spart_forward_bands_bc(const SpartCtx* ctx, int32_t sensor, const void* params_dev,
+                           const void* params_bc_dev, int64_t n, int64_t ld, uint32_t broadcast_rows,
+                           int32_t precision, int32_t flags, void* workspace_dev, void* out_dev, void* stream);
+
 /* Same computation with HOST buffers: params_host [SPART_NPAR][ld] and out_host (layout and
  * element type as above, SPART_OUT_ELEMS elements) are ordinary host memory.  The parameters travel
  * in spans of up to 128 Ki samples (one 2-D copy per run of per-sample rows) into three device
@@ -245,12 +255,16 @@ int spart_leafangles(const double* ab_dev, int64_t n, int64_t ld, double* out_de
  * one output column of spart_forward_bands cast to float) with the smallest weighted squared
  * distance sum_b (sqrt_w[b] (obs_b - lut_b))^2, ties to the lowest index.  weights_dev: sqrt of the
  * band weights [n_bands] or NULL (all 1).  workspace_dev: spart_lut_workspace_bytes(m) bytes.
- * Outputs best_index_dev int64 [m] (= index_offset + local index), best_cost_dev float [m].
+ * Outputs best_index_dev int64 [m] (= index_offset + local index), best_cost_dev float [m].  An entry whose
+ * cost is NaN (NaN in the entry or the observation) or not below 3e38 is never chosen; an observation without
+ * any other entry gets the "no entry" result: index 2^32 - 1 and cost NaN (packed word all ones).
  * Sharded tables: every GPU searches its own slice with index_offset = first global entry of the
  * slice and packed_dev != NULL; the call then leaves one word (cost bits << 32 | global index)
  * per observation in packed_dev [m] instead of unpacking it, the caller min-reduces the words
  * over the GPUs (ncclMin on 64-bit integers: costs are >= 0, so integer order = (cost, index)
- * order, ties to the lowest global index) and calls spart_lut_unpack.  The full table never has
+ * order, ties to the lowest global index) and calls spart_lut_unpack.  The all-ones "no entry" word is -1 as a
+ * signed integer: replace it by 2^63 - 1 (which unpacks to index 2^32 - 1, cost NaN) before a signed
+ * reduction.  The full table never has
  * to be gathered on one GPU.  index_offset + n < 2^32. */
 size_t spart_lut_workspace_bytes(int64_t m);
 int spart_lut_nearest(const float* lut_dev, int64_t n, int32_t n_bands, const float* obs_dev, int64_t m,

@@ -181,7 +181,7 @@ lut_nearest_tc_kernel(const float* __restrict__ lut, int64_t n, int nb, const fl
     const int cnt = (int)((e1 - t0 < kTcTile) ? (e1 - t0) : kTcTile);
     __syncthreads();
     // stage the tile: one thread per entry builds its padded, weighted row and |l|^2 (entries beyond cnt
-    // get a huge |l|^2 so that they never win)
+    // get |l|^2 = NaN: their comparisons are false, so they never win, not even against NaN-only entries)
     for (int e = threadIdx.x; e < kTcTile; e += blockDim.x) {
       float l2 = 0.0f;
       for (int k = 0; k < K; ++k) {
@@ -196,7 +196,7 @@ lut_nearest_tc_kernel(const float* __restrict__ lut, int64_t n, int nb, const fl
           s_lo[e][k] = tf32_hi(v - __uint_as_float(hi));
         }
       }
-      if (e >= cnt) l2 = 1.0e30f;
+      if (e >= cnt) l2 = __int_as_float(0x7fc00000);
       const unsigned h2 = tf32_hi(l2);
       s_hi[e][nb] = h2;                              // |l|^2 = h2 + rest, both meet the constant 1 of A
       s_lo[e][nb] = 0u;

@@ -2185,6 +2185,14 @@ int spart_forward_bands(const SpartCtx* ctx, int32_t sensor, const void* params_
                             workspace_dev, out_dev, stream);
 }
 
+int spart_forward_bands_bc(const SpartCtx* ctx, int32_t sensor, const void* params_dev, const void* params_bc_dev,
+                           int64_t n, int64_t ld, uint32_t broadcast_rows, int32_t precision, int32_t flags,
+                           void* workspace_dev, void* out_dev, void* stream) {
+  if (!params_bc_dev) return fail(SPART_EINVAL, "spart_forward_bands_bc: null broadcast base%s");
+  return forward_bands_impl(ctx, sensor, params_dev, params_bc_dev, n, ld, broadcast_rows, precision, flags,
+                            workspace_dev, out_dev, stream);
+}
+
 int spart_profile_enable(SpartCtx* ctx, int32_t on) {
   if (!ctx) return fail(SPART_EINVAL, "spart_profile_enable: null context%s");
   std::lock_guard<std::mutex> lock(ctx->prof_mu);

@@ -32,7 +32,7 @@ FP32 = 32
 EXPORTS = (
     "spart_abi_version", "spart_last_error", "spart_device_count", "spart_create", "spart_create_with_soils",
     "spart_destroy",
-    "spart_workspace_bytes", "spart_forward_bands", "spart_forward_bands_host", "spart_forward_spectrum",
+    "spart_workspace_bytes", "spart_forward_bands", "spart_forward_bands_bc", "spart_forward_bands_host", "spart_forward_spectrum",
     "spart_smac", "spart_sailh", "spart_lut_workspace_bytes", "spart_lut_nearest", "spart_lut_nearest_tc", "spart_lut_unpack",
     "spart_leafangles", "spart_set_lidf", "spart_profile_enable", "spart_profile_read", "spart_measure_peaks", "spart_measure_fp64_chain", "spart_launch_count",
 )
@@ -84,6 +84,8 @@ def load():
     lib.spart_workspace_bytes.restype = c_size_t
     lib.spart_forward_bands.argtypes = [c_void_p, c_int32, c_void_p, c_int64, c_int64, c_uint32, c_int32, c_int32,
                                         c_void_p, c_void_p, c_void_p]
+    lib.spart_forward_bands_bc.argtypes = [c_void_p, c_int32, c_void_p, c_void_p, c_int64, c_int64, c_uint32, c_int32,
+                                           c_int32, c_void_p, c_void_p, c_void_p]
     lib.spart_forward_bands_host.argtypes = [c_void_p, c_int32, c_void_p, c_int64, c_int64, c_uint32, c_int32,
                                              c_int32, c_void_p]
     lib.spart_forward_spectrum.argtypes = [c_void_p, c_void_p, c_int64, c_int64, c_int32, c_double, c_double,

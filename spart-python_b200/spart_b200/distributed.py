@@ -145,8 +145,9 @@ def run_batch_sharded_pipelined(params_local, sensor, precision="fp64", chunk=1 
         nb, conv_ea = st.n_bands, st.conv_ea
 
         def compute(p, view):
+            # p is a column slice of params_local: the broadcast rows' values sit in params_local's column 0
             eng.forward_bands(p, sensor, out=view if compact else view.view(p.shape[1], nb, NOUT), precision=precision,
-                              broadcast_rows=broadcast_rows, compact=compact)
+                              broadcast_rows=broadcast_rows, compact=compact, broadcast_base=params_local)
     else:
         nb, conv_ea = compute.n_bands, getattr(compute, "conv_ea", None)
     blocks = [out_elems(hi - lo, nb, compact) for lo, hi in bounds]

@@ -193,7 +193,8 @@ class Engine:
                              " (float32 is accepted with precision='fp32')")
         if params.device != self.device:
             raise ValueError(f"params on {params.device}, engine on {self.device}")
-        return params, params.shape[1], (params.stride(0) if params.shape[1] > 1 else max(params.shape[1], 1))
+        # a [27, 1] view of a wider batch keeps that batch's row stride, which is its ld
+        return params, params.shape[1], (params.stride(0) if params.shape[1] >= 1 else 1)
 
     def _geometry_mask(self, params, n, mask, uniform_geometry):
         """uniform_geometry=True is checked, not trusted: unless the three angle rows already are
@@ -236,7 +237,7 @@ class Engine:
 
     def forward_bands(self, params, sensor, out=None, precision="fp64", uniform_geometry=False,
                       soil_spectrum=None, band_mode="interp", broadcast_rows=0, compact=False,
-                      reuse_record=False, workspace=None, lidf=None, soil_library=None):
+                      reuse_record=False, workspace=None, lidf=None, soil_library=None, broadcast_base=None):
         """params: CUDA float64 [27, n] -> CUDA float64 [n, nb, 3] = (R_TOC, R_TOA, L_TOA).
         Asynchronous on the current torch stream.
 
@@ -253,7 +254,11 @@ class Engine:
         `out`: result buffer to fill ([n, nb, 3], or flat with out_elems(n, nb, True) elements when
         compact).
         lidf: a leaf inclination distribution [n, 13] (or one row for the whole batch) used instead of the one
-        derived from LIDFa / LIDFb -- the reference's assigned `CanopyStructure.lidf`; FP64 only."""
+        derived from LIDFa / LIDFb -- the reference's assigned `CanopyStructure.lidf`; FP64 only.
+        broadcast_base: the tensor whose column 0 holds the broadcast rows' values (default `params`): a
+        CUDA tensor [27, >= 1] of the params' dtype and row stride, typically the batch that `params` is a
+        column slice of.  A batch of more than MAX_SAMPLES_PER_CALL samples is split into calls, and every
+        call reads the broadcast rows from this column 0, never from its own first column."""
         prec = _PRECISION[precision]
         handle, st = self.sensor(sensor, soil_spectrum, soil_library)
         params, n, ld = self._prep(params, allow_f32=(prec == _lib.FP32))
@@ -275,6 +280,12 @@ class Engine:
                              " n*nb*2 + n elements when compact")
         if n > MAX_SAMPLES_PER_CALL and (compact or reuse_record):
             raise ValueError(f"compact / reuse_record runs handle at most {MAX_SAMPLES_PER_CALL} samples per call")
+        bc = params if broadcast_base is None else broadcast_base
+        if broadcast_base is not None and not (
+                isinstance(bc, torch.Tensor) and bc.device == params.device and bc.dtype == params.dtype
+                and bc.dim() == 2 and bc.shape[0] == NPAR and bc.shape[1] >= 1 and bc.stride(0) == ld):
+            raise ValueError("broadcast_base must be a tensor [27, >= 1] on the params' device with their dtype and row"
+                             " stride")
         esz = params.element_size()
         with torch.cuda.device(self.device):
             stream = torch.cuda.current_stream(self.device).cuda_stream
@@ -282,9 +293,11 @@ class Engine:
                 m = min(MAX_SAMPLES_PER_CALL, n - s0)
                 ws = workspace if (workspace is not None and s0 == 0 and m == n) else self.workspace(m)
                 keep = self._set_lidf(lidf, n, ws, stream) if lidf is not None else None      # noqa: F841
-                _lib.check(self.lib.spart_forward_bands(handle, 0, params.data_ptr() + esz * s0, m, ld, mask, prec, flags,
-                                                        ws.data_ptr(), out.data_ptr() + esz * s0 * nb * NOUT,
-                                                        stream), "spart_forward_bands")
+                # every call reads the broadcast rows from column 0 of the batch, not from its own first column
+                _lib.check(self.lib.spart_forward_bands_bc(handle, 0, params.data_ptr() + esz * s0, bc.data_ptr(), m, ld,
+                                                           mask, prec, flags, ws.data_ptr(),
+                                                           out.data_ptr() + esz * s0 * nb * NOUT, stream),
+                           "spart_forward_bands")
         return CompactBands(out, n, nb, st.conv_ea, prec == _lib.FP32) if compact else out
 
     def forward_bands_multi(self, params, sensors, outs=None, precision="fp64", uniform_geometry=False,
@@ -393,7 +406,7 @@ class Engine:
             raise ValueError("params must be a host float64 array [27, n] with contiguous rows"
                              " (float32 is accepted with precision='fp32')")
         n, nb = p.shape[1], st.n_bands
-        ld = p.strides[0] // p.itemsize if n > 1 else max(n, 1)
+        ld = p.strides[0] // p.itemsize if n >= 1 else 1
         mask = self._geometry_mask(p, n, _lib.row_mask(broadcast_rows), uniform_geometry)
         flags = self._flags(soil_spectrum, band_mode, p.dtype == np.float32, compact, soil_library=soil_library)
         elems = out_elems(n, nb, compact)

@@ -10,6 +10,8 @@ import torch
 from . import _lib
 from .engine import default_engine
 
+NO_ENTRY = 2 ** 32 - 1      # index `nearest` returns (with cost NaN) for an observation without a finite-cost entry
+
 
 def generate(params, sensor, precision="fp64", chunk=1 << 20, out_dtype=torch.float32, column=None, path=None,
              uniform_geometry=False, soil_library=None):
@@ -84,11 +86,21 @@ def unpack(words):
 
 def nearest(lut, obs, weights=None, method="exact"):
     """lut: CUDA float32 [n, nb]; obs: CUDA float32 [m, nb]; weights: optional per-band weights [nb].
-    Returns (index int64 [m], cost float32 [m]) of the entry minimising sum_b w_b (obs_b - lut_b)^2.
+    Returns (index int64 [m], cost float32 [m]) of the entry minimising sum_b w_b (obs_b - lut_b)^2, ties to the
+    lowest index.  Entries whose cost is NaN (a NaN value in the entry or in the observation) or not below 3e38 are
+    never chosen; an observation without any other entry gets the "no entry" result: index 2^32 - 1
+    (NO_ENTRY) and cost NaN.
     method="tensor": the comparison runs on the tensor cores in 3xTF32 (the entry is optimal up to ~1e-6 of
     |obs||entry|, its cost is exact)."""
     _check(lut, obs)
     return _search(lut, obs, weights, 0, packed=False, method=method)
+
+
+def for_min_reduction(words):
+    """Packed words of a search piece, ready for a signed 64-bit min-reduction with other pieces: the all-ones
+    "no entry" word is -1 as int64 and would win, so it becomes the reduction's identity 2^63 - 1 (which unpacks
+    to the same "no entry" result, index NO_ENTRY and cost NaN)."""
+    return words.masked_fill(words == -1, 2 ** 63 - 1)
 
 
 def nearest_sharded(lut_local, obs, weights=None, group=None, index_offset=None, search=None, unpack_words=None,
@@ -97,7 +109,8 @@ def nearest_sharded(lut_local, obs, weights=None, group=None, index_offset=None,
     `lut_local` [n_r, nb], rank order = table order; every rank passes the same `obs`).  Each GPU
     searches its own slice, the per-observation words (cost bits << 32 | global index) are
     min-reduced with one NCCL all-reduce of 8 bytes per observation, and every rank returns the
-    global (index, cost).  The table itself is never gathered.  `search` / `unpack_words` default to the
+    global (index, cost); an observation that finds no entry on any rank gets `nearest`'s "no entry"
+    result.  The table itself is never gathered.  `search` / `unpack_words` default to the
     CUDA kernels; CPU tests inject stand-ins to exercise the reduction logic with gloo."""
     import torch.distributed as dist
     if index_offset is None:
@@ -112,7 +125,7 @@ def nearest_sharded(lut_local, obs, weights=None, group=None, index_offset=None,
     if lut_local.shape[0] == 0:       # a rank without entries contributes the identity of the min-reduction
         words = torch.full((obs.shape[0],), 2 ** 63 - 1, dtype=torch.int64, device=obs.device)
     else:
-        words = search(lut_local, obs, weights, index_offset)
+        words = for_min_reduction(search(lut_local, obs, weights, index_offset))
     # costs are >= 0, so the signed 64-bit order of the words is the (cost, index) order
     dist.all_reduce(words, op=dist.ReduceOp.MIN, group=group)
     return (unpack_words or unpack)(words)
