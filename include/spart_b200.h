@@ -18,7 +18,8 @@
  *     allocator); the library never allocates per call on the device paths and all work is
  *     enqueued asynchronously on the caller's stream (a cudaStream_t passed as void*);
  *   - a context is immutable after spart_create and may be used concurrently from several
- *     host threads; create one context per GPU;
+ *     host threads until spart_destroy, which no other thread may overlap; create one context
+ *     per GPU;
  *   - there is NO CPU fallback: without a CUDA device every compute entry point fails.
  *
  * Batch parameter layout ("params"): struct-of-arrays, double, [SPART_NPAR][ld] with
@@ -169,6 +170,9 @@ int spart_create(const SpartTables* tables, const SpartSensor* sensors, int32_t 
  * serves runs without the flag exactly like one from spart_create. */
 int spart_create_with_soils(const SpartTables* tables, const SpartSensor* sensors, int32_t n_sensors,
                             const double* soils, int32_t n_soils, int32_t device, SpartCtx** out);
+/* Frees the context.  It first waits for all work on the context's device (cudaDeviceSynchronize), so
+ * device-path calls still queued on any stream finish before their tables are freed.  The caller must not
+ * destroy a context while another thread is inside a call on it, or call it afterwards. */
 int spart_destroy(SpartCtx* ctx);
 
 /* Device scratch the caller must provide to the *_dev entry points for a batch of n samples. */

@@ -1664,7 +1664,12 @@ struct NvtxRange {
 
 }  // namespace
 
-// __constant__ tables are per device: upload them once for every device that is used.
+constexpr int kSrfMaxSlots = 24;      // 24 x 4 x 128 doubles = 96 KB of accumulators at most
+
+// __constant__ tables are per device: upload them once for every device that is used.  The dynamic shared-memory
+// cap of the SRF kernels is set here too, once, to the largest plan spart_create accepts: the attribute belongs to
+// the kernel and device, not to a context, so setting it per call to that call's plan size would let a concurrent
+// call with a smaller plan lower it between another thread's set and launch.
 static int init_device_constants(int device) {
   static std::mutex mu;
   static bool done[64] = {false};
@@ -1701,6 +1706,9 @@ static int init_device_constants(int device) {
   }
   CUDA_TRY(cudaMemcpyToSymbol(c_sin_ttli, sl, sizeof(sl)));
   CUDA_TRY(cudaMemcpyToSymbol(c_cos_ttli, cl, sizeof(cl)));
+  const int srf_max_bytes = (int)(sizeof(double) * kSrfMaxSlots * 4 * kBandThreads);
+  CUDA_TRY(cudaFuncSetAttribute(band_kernel_srf, cudaFuncAttributeMaxDynamicSharedMemorySize, srf_max_bytes));
+  CUDA_TRY(cudaFuncSetAttribute(soillib_srf, cudaFuncAttributeMaxDynamicSharedMemorySize, srf_max_bytes));
 
   done[device] = true;
   return SPART_OK;
@@ -1724,7 +1732,9 @@ int spart_device_count(void) {
 int spart_destroy(SpartCtx* ctx) {
   if (!ctx) return SPART_OK;
   DeviceGuard guard(ctx->device);
-  if (ctx->compute_stream) cudaStreamSynchronize(ctx->compute_stream);
+  // work of device-path calls may still be queued on callers' streams and read the context's tables: wait for
+  // everything on the device, not only for the host path's own streams, before anything is freed
+  cudaDeviceSynchronize();
   for (int i = 0; i < SpartCtx::kSlots; ++i) {
     if (ctx->slot_rec[i]) cudaFree(ctx->slot_rec[i]);
     if (ctx->slot_out[i]) cudaFree(ctx->slot_out[i]);
@@ -1771,8 +1781,6 @@ static int upload(const std::vector<T>& v, T** d) {
   if (!v.empty()) CUDA_TRY(cudaMemcpy(*d, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice));
   return SPART_OK;
 }
-
-constexpr int kSrfMaxSlots = 24;      // 24 x 4 x 128 doubles = 96 KB of accumulators at most
 
 static int build_srf_plan(const SpartSensor& S, SpartCtx::SrfDev& dev) {
   const int nb = S.n_bands;
@@ -2134,14 +2142,11 @@ static int forward_bands_impl(const SpartCtx* ctx, int32_t sensor, const void* p
                          v.fin_slot};
       const size_t acc_bytes = sizeof(double) * v.n_slots * 4 * kBandThreads;
       const unsigned blocks = (unsigned)((n + kBandThreads - 1) / kBandThreads);
+      // the kernels' dynamic shared-memory cap was set to the kSrfMaxSlots bound once per device
       if (library) {
-        if (acc_bytes > 16 * 1024)
-          CUDA_TRY(cudaFuncSetAttribute(soillib_srf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)acc_bytes));
         soillib_srf<<<blocks, kBandThreads, acc_bytes, st>>>(P, n, rec, ctx->d_band[sensor], ctx->d_lc, plan, nb, out,
                                                              compact ? 1 : 0, lib);
       } else {
-        if (acc_bytes > 16 * 1024)
-          CUDA_TRY(cudaFuncSetAttribute(band_kernel_srf, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)acc_bytes));
         band_kernel_srf<<<blocks, kBandThreads, acc_bytes, st>>>(P, n, rec, ctx->d_band[sensor], ctx->d_lc, plan, nb,
                                                                  out, compact ? 1 : 0);
       }

@@ -7,6 +7,7 @@ lazily per sensor and cached (bounded, least recently used first out).
 import hashlib
 import threading
 from collections import OrderedDict
+from contextlib import contextmanager
 
 import numpy as np
 import torch
@@ -85,6 +86,15 @@ class CompactBands:
         return np.concatenate([self.R, self.L_TOA[..., None]], axis=2)
 
 
+class _Context:
+    """A cached C context: its handle and tables, the host arrays it was built from, the number of calls
+    using it (`Engine._use`) and whether it has left the cache (then the last user destroys it)."""
+    __slots__ = ("handle", "st", "keep", "uses", "retired")
+
+    def __init__(self, handle, st, keep):
+        self.handle, self.st, self.keep, self.uses, self.retired = handle, st, keep, 0, False
+
+
 def _sensor_digest(info):
     """Content hash of everything the hot path uses of a sensorinfo dict."""
     h = hashlib.sha1()
@@ -122,7 +132,33 @@ class Engine:
         must be run with SPART_FLAG_SOIL_SPECTRUM.  soil_library: optional SoilLibrary, uploaded once
         into the context (spart_create_with_soils) for runs with SPART_FLAG_SOIL_LIBRARY; keyed by its
         content digest.  At most MAX_CONTEXTS contexts are kept; the least recently used one is
-        destroyed (its device tables are freed) when a new one is needed."""
+        destroyed (its device tables are freed) when a new one is needed.  The returned handle is
+        therefore valid only until the cache evicts it: any later `sensor()` call that creates a context,
+        from this thread or another one, may destroy it.  The Engine's own methods hold their context
+        for the whole call (see `_use`)."""
+        e = self._entry(sensor, soil_spectrum, soil_library, pin=False)
+        return e.handle, e.st
+
+    @contextmanager
+    def _use(self, sensor, soil_spectrum=None, soil_library=None):
+        """(ctx, SensorTables) pinned for the duration of the `with` block: eviction (by any thread)
+        retires a pinned context instead of destroying it, and the last user's exit destroys it."""
+        e = self._entry(sensor, soil_spectrum, soil_library, pin=True)
+        try:
+            yield e.handle, e.st
+        finally:
+            with self._lock:
+                e.uses -= 1
+                if e.retired and e.uses == 0:
+                    self.lib.spart_destroy(e.handle)
+
+    def _retire(self, e):
+        """Called under _lock for an entry leaving the cache: destroy it now unless a call is using it."""
+        e.retired = True
+        if e.uses == 0:
+            self.lib.spart_destroy(e.handle)
+
+    def _entry(self, sensor, soil_spectrum, soil_library, pin):
         skey = sensor if isinstance(sensor, str) else ("custom", _sensor_digest(sensor))
         soil = None
         if soil_spectrum is not None and soil_library is not None:
@@ -138,10 +174,11 @@ class Engine:
         else:
             key = (skey, None if soil is None else hashlib.sha1(soil.tobytes()).hexdigest())
         with self._lock:
-            hit = self._ctx.get(key)
-            if hit is not None:
+            e = self._ctx.get(key)
+            if e is not None:
                 self._ctx.move_to_end(key)
-                return hit[0], hit[1]
+                e.uses += pin
+                return e
             info = T.load_sensor_info(sensor) if isinstance(sensor, str) else sensor
             st = T.build_sensor(sensor if isinstance(sensor, str) else "custom", info, self._opt)
             lc = self._lc
@@ -166,15 +203,16 @@ class Engine:
                                                             self.device.index, _lib.byref(handle)),
                            "spart_create_with_soils")
             while len(self._ctx) >= MAX_CONTEXTS:
-                _, (old, _, _) = self._ctx.popitem(last=False)
-                self.lib.spart_destroy(old)
-            self._ctx[key] = (handle, st, (smac, lc))
-            return handle, st
+                self._retire(self._ctx.popitem(last=False)[1])
+            e = self._ctx[key] = _Context(handle, st, (smac, lc))
+            e.uses += pin
+            return e
 
     def close(self):
+        """Destroy every cached context; one that a call is using is destroyed when that call ends."""
         with self._lock:
-            for handle, _, _ in self._ctx.values():
-                self.lib.spart_destroy(handle)
+            for e in self._ctx.values():
+                self._retire(e)
             self._ctx.clear()
 
     def __del__(self):
@@ -260,45 +298,46 @@ class Engine:
         column slice of.  A batch of more than MAX_SAMPLES_PER_CALL samples is split into calls, and every
         call reads the broadcast rows from this column 0, never from its own first column."""
         prec = _PRECISION[precision]
-        handle, st = self.sensor(sensor, soil_spectrum, soil_library)
-        params, n, ld = self._prep(params, allow_f32=(prec == _lib.FP32))
-        f32_io = params.dtype == torch.float32
-        mask = self._geometry_mask(params, n, _lib.row_mask(broadcast_rows), uniform_geometry)
-        flags = self._flags(soil_spectrum, band_mode, f32_io, compact, reuse_record, soil_library)
-        if lidf is not None:
-            if prec != _lib.FP64 or reuse_record or n > MAX_SAMPLES_PER_CALL:
-                raise ValueError("lidf= needs precision='fp64', no reuse_record and at most "
-                                 f"{MAX_SAMPLES_PER_CALL} samples per call")
-            flags |= _lib.FLAG_USER_LIDF
-        nb = st.n_bands
-        elems = out_elems(n, nb, compact)
-        if out is None:
-            out = torch.empty(elems if compact else (n, nb, NOUT), dtype=params.dtype, device=self.device)
-        elif not (out.is_cuda and out.dtype == params.dtype and out.is_contiguous() and out.numel() == elems
-                  and (compact or tuple(out.shape) == (n, nb, NOUT))):
-            raise ValueError("out must be a contiguous CUDA tensor of the params' dtype: [n, nb, 3], or flat with"
-                             " n*nb*2 + n elements when compact")
-        if n > MAX_SAMPLES_PER_CALL and (compact or reuse_record):
-            raise ValueError(f"compact / reuse_record runs handle at most {MAX_SAMPLES_PER_CALL} samples per call")
-        bc = params if broadcast_base is None else broadcast_base
-        if broadcast_base is not None and not (
-                isinstance(bc, torch.Tensor) and bc.device == params.device and bc.dtype == params.dtype
-                and bc.dim() == 2 and bc.shape[0] == NPAR and bc.shape[1] >= 1 and bc.stride(0) == ld):
-            raise ValueError("broadcast_base must be a tensor [27, >= 1] on the params' device with their dtype and row"
-                             " stride")
-        esz = params.element_size()
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-            for s0 in range(0, n, MAX_SAMPLES_PER_CALL):
-                m = min(MAX_SAMPLES_PER_CALL, n - s0)
-                ws = workspace if (workspace is not None and s0 == 0 and m == n) else self.workspace(m)
-                keep = self._set_lidf(lidf, n, ws, stream) if lidf is not None else None      # noqa: F841
-                # every call reads the broadcast rows from column 0 of the batch, not from its own first column
-                _lib.check(self.lib.spart_forward_bands_bc(handle, 0, params.data_ptr() + esz * s0, bc.data_ptr(), m, ld,
-                                                           mask, prec, flags, ws.data_ptr(),
-                                                           out.data_ptr() + esz * s0 * nb * NOUT, stream),
-                           "spart_forward_bands")
-        return CompactBands(out, n, nb, st.conv_ea, prec == _lib.FP32) if compact else out
+        with self._use(sensor, soil_spectrum, soil_library) as (handle, st):
+            params, n, ld = self._prep(params, allow_f32=(prec == _lib.FP32))
+            f32_io = params.dtype == torch.float32
+            mask = self._geometry_mask(params, n, _lib.row_mask(broadcast_rows), uniform_geometry)
+            flags = self._flags(soil_spectrum, band_mode, f32_io, compact, reuse_record, soil_library)
+            if lidf is not None:
+                if prec != _lib.FP64 or reuse_record or n > MAX_SAMPLES_PER_CALL:
+                    raise ValueError("lidf= needs precision='fp64', no reuse_record and at most "
+                                     f"{MAX_SAMPLES_PER_CALL} samples per call")
+                flags |= _lib.FLAG_USER_LIDF
+            nb = st.n_bands
+            elems = out_elems(n, nb, compact)
+            if out is None:
+                out = torch.empty(elems if compact else (n, nb, NOUT), dtype=params.dtype, device=self.device)
+            elif not (out.is_cuda and out.dtype == params.dtype and out.is_contiguous() and out.numel() == elems
+                      and (compact or tuple(out.shape) == (n, nb, NOUT))):
+                raise ValueError("out must be a contiguous CUDA tensor of the params' dtype: [n, nb, 3], or flat with"
+                                 " n*nb*2 + n elements when compact")
+            if n > MAX_SAMPLES_PER_CALL and (compact or reuse_record):
+                raise ValueError(f"compact / reuse_record runs handle at most {MAX_SAMPLES_PER_CALL} samples per"
+                                 " call")
+            bc = params if broadcast_base is None else broadcast_base
+            if broadcast_base is not None and not (
+                    isinstance(bc, torch.Tensor) and bc.device == params.device and bc.dtype == params.dtype
+                    and bc.dim() == 2 and bc.shape[0] == NPAR and bc.shape[1] >= 1 and bc.stride(0) == ld):
+                raise ValueError("broadcast_base must be a tensor [27, >= 1] on the params' device with their dtype and"
+                                 " row stride")
+            esz = params.element_size()
+            with torch.cuda.device(self.device):
+                stream = torch.cuda.current_stream(self.device).cuda_stream
+                for s0 in range(0, n, MAX_SAMPLES_PER_CALL):
+                    m = min(MAX_SAMPLES_PER_CALL, n - s0)
+                    ws = workspace if (workspace is not None and s0 == 0 and m == n) else self.workspace(m)
+                    keep = self._set_lidf(lidf, n, ws, stream) if lidf is not None else None      # noqa: F841
+                    # every call reads the broadcast rows from column 0 of the batch, not from its own first column
+                    _lib.check(self.lib.spart_forward_bands_bc(handle, 0, params.data_ptr() + esz * s0, bc.data_ptr(),
+                                                               m, ld, mask, prec, flags, ws.data_ptr(),
+                                                               out.data_ptr() + esz * s0 * nb * NOUT, stream),
+                               "spart_forward_bands")
+            return CompactBands(out, n, nb, st.conv_ea, prec == _lib.FP32) if compact else out
 
     def forward_bands_multi(self, params, sensors, outs=None, precision="fp64", uniform_geometry=False,
                             soil_spectrum=None, band_mode="interp", broadcast_rows=0, compact=False,
@@ -325,59 +364,60 @@ class Engine:
         kChlrel, soil refl, soil refl dry, rso, rdo, rsd, rdd.  rho_thermal / tau_thermal: leaf
         reflectance / transmittance beyond 2400 nm (LeafBiology.rho_thermal / tau_thermal).
         soil_spectrum / soil_library as in forward_bands."""
-        handle, _ = self.sensor("Sentinel2A-MSI", soil_spectrum, soil_library)   # any context carries the wavelength tables
-        params, n, ld = self._prep(params)
-        if out is None:
-            out = torch.empty((n, NSPEC, NWL_S), dtype=torch.float64, device=self.device)
-        ws = self.workspace(n)
-        flags = self._flags(soil_spectrum, "interp", soil_library=soil_library)
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-            if lidf is not None:
-                keep = self._set_lidf(lidf, n, ws, stream)      # noqa: F841
-                flags |= _lib.FLAG_USER_LIDF
-            _lib.check(self.lib.spart_forward_spectrum(handle, params.data_ptr(), n, ld, flags, float(rho_thermal),
-                                                       float(tau_thermal), ws.data_ptr(), out.data_ptr(), stream),
-                       "spart_forward_spectrum")
-        return out
+        # any context carries the wavelength tables
+        with self._use("Sentinel2A-MSI", soil_spectrum, soil_library) as (handle, _):
+            params, n, ld = self._prep(params)
+            if out is None:
+                out = torch.empty((n, NSPEC, NWL_S), dtype=torch.float64, device=self.device)
+            ws = self.workspace(n)
+            flags = self._flags(soil_spectrum, "interp", soil_library=soil_library)
+            with torch.cuda.device(self.device):
+                stream = torch.cuda.current_stream(self.device).cuda_stream
+                if lidf is not None:
+                    keep = self._set_lidf(lidf, n, ws, stream)      # noqa: F841
+                    flags |= _lib.FLAG_USER_LIDF
+                _lib.check(self.lib.spart_forward_spectrum(handle, params.data_ptr(), n, ld, flags,
+                                                           float(rho_thermal), float(tau_thermal), ws.data_ptr(),
+                                                           out.data_ptr(), stream), "spart_forward_spectrum")
+            return out
 
     def smac(self, params, sensor, out=None):
         """SMAC alone.  params: CUDA float64 [27, n] (angle and atmosphere rows used)
         -> CUDA float64 [n, 9, nb]: Ta_s, Ta_o, Tg, Ra_dd, Ra_so, Ta_ss, Ta_sd, Ta_oo, Ta_do."""
-        handle, st = self.sensor(sensor)
-        params, n, ld = self._prep(params)
-        if out is None:
-            out = torch.empty((n, 9, st.n_bands), dtype=torch.float64, device=self.device)
-        ws = self.workspace(n)
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-            _lib.check(self.lib.spart_smac(handle, 0, params.data_ptr(), n, ld, ws.data_ptr(), out.data_ptr(), stream),
-                       "spart_smac")
-        return out
+        with self._use(sensor) as (handle, st):
+            params, n, ld = self._prep(params)
+            if out is None:
+                out = torch.empty((n, 9, st.n_bands), dtype=torch.float64, device=self.device)
+            ws = self.workspace(n)
+            with torch.cuda.device(self.device):
+                stream = torch.cuda.current_stream(self.device).cuda_stream
+                _lib.check(self.lib.spart_smac(handle, 0, params.data_ptr(), n, ld, ws.data_ptr(), out.data_ptr(),
+                                               stream), "spart_smac")
+            return out
 
     def sailh(self, params, soil_refl, leaf_refl, leaf_tran, out=None):
         """SAILH on caller-supplied spectra.  params: CUDA float64 [27, n] (canopy and angle rows
         used); spectra: CUDA float64 [2162] (shared by all samples) or [n, 2162].
         -> CUDA float64 [n, 4, 2162] = rso, rdo, rsd, rdd."""
-        handle, _ = self.sensor("Sentinel2A-MSI")
-        params, n, ld = self._prep(params)
-        specs = [soil_refl, leaf_refl, leaf_tran]
-        shared = all(x.dim() == 1 for x in specs)
-        for x in specs:
-            ok = x.is_cuda and x.dtype == torch.float64 and x.is_contiguous() and (
-                tuple(x.shape) == (NWL_S,) if shared else tuple(x.shape) == (n, NWL_S))
-            if not ok:
-                raise RuntimeError("Parameter leafopt.refl must be of len 2162 i.e. include thermal specturm "
-                                   "(CUDA float64, all three spectra [2162] or all [n, 2162])")
-        if out is None:
-            out = torch.empty((n, 4, NWL_S), dtype=torch.float64, device=self.device)
-        ws = self.workspace(n)
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream(self.device).cuda_stream
-            _lib.check(self.lib.spart_sailh(handle, params.data_ptr(), n, ld, soil_refl.data_ptr(),
-                                            leaf_refl.data_ptr(), leaf_tran.data_ptr(), 0 if shared else NWL_S,
-                                            ws.data_ptr(), out.data_ptr(), stream), "spart_sailh")
-        return out
+        with self._use("Sentinel2A-MSI") as (handle, _):
+            params, n, ld = self._prep(params)
+            specs = [soil_refl, leaf_refl, leaf_tran]
+            shared = all(x.dim() == 1 for x in specs)
+            for x in specs:
+                ok = x.is_cuda and x.dtype == torch.float64 and x.is_contiguous() and (
+                    tuple(x.shape) == (NWL_S,) if shared else tuple(x.shape) == (n, NWL_S))
+                if not ok:
+                    raise RuntimeError("Parameter leafopt.refl must be of len 2162 i.e. include thermal specturm "
+                                       "(CUDA float64, all three spectra [2162] or all [n, 2162])")
+            if out is None:
+                out = torch.empty((n, 4, NWL_S), dtype=torch.float64, device=self.device)
+            ws = self.workspace(n)
+            with torch.cuda.device(self.device):
+                stream = torch.cuda.current_stream(self.device).cuda_stream
+                _lib.check(self.lib.spart_sailh(handle, params.data_ptr(), n, ld, soil_refl.data_ptr(),
+                                                leaf_refl.data_ptr(), leaf_tran.data_ptr(), 0 if shared else NWL_S,
+                                                ws.data_ptr(), out.data_ptr(), stream), "spart_sailh")
+            return out
 
     def leafangles(self, ab):
         """[n, 2] (LIDFa, LIDFb) host array -> [n, 13] lidf host array."""
@@ -399,40 +439,40 @@ class Engine:
         pipelined inside the C library; pinned memory is DMA'd directly, pageable memory is staged
         by the library's copy threads.  Other arguments as forward_bands."""
         prec = _PRECISION[precision]
-        handle, st = self.sensor(sensor, soil_spectrum, soil_library)
-        p = params.numpy() if isinstance(params, torch.Tensor) else np.asarray(params)
-        okdt = p.dtype == np.float64 or (p.dtype == np.float32 and prec == _lib.FP32)
-        if not okdt or p.ndim != 2 or p.shape[0] != NPAR or (p.shape[1] > 1 and p.strides[1] != p.itemsize):
-            raise ValueError("params must be a host float64 array [27, n] with contiguous rows"
-                             " (float32 is accepted with precision='fp32')")
-        n, nb = p.shape[1], st.n_bands
-        ld = p.strides[0] // p.itemsize if n >= 1 else 1
-        mask = self._geometry_mask(p, n, _lib.row_mask(broadcast_rows), uniform_geometry)
-        flags = self._flags(soil_spectrum, band_mode, p.dtype == np.float32, compact, soil_library=soil_library)
-        elems = out_elems(n, nb, compact)
-        if out is None:
-            out = np.empty(elems if compact else (n, nb, NOUT), dtype=p.dtype)
-        o = out.numpy() if isinstance(out, torch.Tensor) else out
-        if o.dtype != p.dtype or not o.flags.c_contiguous or o.size != elems or not (
-                compact or o.shape == (n, nb, NOUT)):
-            raise ValueError("out must be a C-contiguous host array of the params' dtype: [n, nb, 3], or flat with"
-                             " n*nb*2 + n elements when compact")
-        _lib.check(self.lib.spart_forward_bands_host(handle, 0, p.ctypes.data, n, ld, mask, prec, flags,
-                                                     o.ctypes.data), "spart_forward_bands_host")
-        return CompactBands(out, n, nb, st.conv_ea, prec == _lib.FP32) if compact else out
+        with self._use(sensor, soil_spectrum, soil_library) as (handle, st):
+            p = params.numpy() if isinstance(params, torch.Tensor) else np.asarray(params)
+            okdt = p.dtype == np.float64 or (p.dtype == np.float32 and prec == _lib.FP32)
+            if not okdt or p.ndim != 2 or p.shape[0] != NPAR or (p.shape[1] > 1 and p.strides[1] != p.itemsize):
+                raise ValueError("params must be a host float64 array [27, n] with contiguous rows"
+                                 " (float32 is accepted with precision='fp32')")
+            n, nb = p.shape[1], st.n_bands
+            ld = p.strides[0] // p.itemsize if n >= 1 else 1
+            mask = self._geometry_mask(p, n, _lib.row_mask(broadcast_rows), uniform_geometry)
+            flags = self._flags(soil_spectrum, band_mode, p.dtype == np.float32, compact, soil_library=soil_library)
+            elems = out_elems(n, nb, compact)
+            if out is None:
+                out = np.empty(elems if compact else (n, nb, NOUT), dtype=p.dtype)
+            o = out.numpy() if isinstance(out, torch.Tensor) else out
+            if o.dtype != p.dtype or not o.flags.c_contiguous or o.size != elems or not (
+                    compact or o.shape == (n, nb, NOUT)):
+                raise ValueError("out must be a C-contiguous host array of the params' dtype: [n, nb, 3], or flat with"
+                                 " n*nb*2 + n elements when compact")
+            _lib.check(self.lib.spart_forward_bands_host(handle, 0, p.ctypes.data, n, ld, mask, prec, flags,
+                                                         o.ctypes.data), "spart_forward_bands_host")
+            return CompactBands(out, n, nb, st.conv_ea, prec == _lib.FP32) if compact else out
 
     def profile_enable(self, sensor, on=True):
-        handle, _ = self.sensor(sensor)
-        _lib.check(self.lib.spart_profile_enable(handle, 1 if on else 0), "spart_profile_enable")
+        with self._use(sensor) as (handle, _):
+            _lib.check(self.lib.spart_profile_enable(handle, 1 if on else 0), "spart_profile_enable")
 
     def profile_read(self, sensor):
         """Summed CUDA-event durations of the three kernels since the last read:
         {'lidf_ms', 'geometry_ms', 'band_ms', 'calls'}."""
-        handle, _ = self.sensor(sensor)
-        ms = (_lib.c_double * _lib.NKERNELS)()
-        c = _lib.c_int64()
-        _lib.check(self.lib.spart_profile_read(handle, ms, _lib.byref(c)), "spart_profile_read")
-        return {"lidf_ms": ms[0], "geometry_ms": ms[1], "band_ms": ms[2], "calls": c.value}
+        with self._use(sensor) as (handle, _):
+            ms = (_lib.c_double * _lib.NKERNELS)()
+            c = _lib.c_int64()
+            _lib.check(self.lib.spart_profile_read(handle, ms, _lib.byref(c)), "spart_profile_read")
+            return {"lidf_ms": ms[0], "geometry_ms": ms[1], "band_ms": ms[2], "calls": c.value}
 
     def measure_peaks(self):
         a, b = _lib.c_double(), _lib.c_double()
