@@ -27,9 +27,12 @@
 #include <cstdlib>
 #include <cstring>
 #include <functional>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <thread>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "../../include/spart_b200.h"
@@ -81,6 +84,57 @@ static int fail(int code, const char* fmt, const char* detail = "") {
       return (int)_e;                                                                    \
     }                                                                                    \
   } while (0)
+
+// Every kernel launch of the library goes through here, so spart_launch_count() counts each one and a failed
+// launch is reported like any other failed CUDA call.
+template <typename... KArgs, typename... Args>
+static int launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+  kernel<<<grid, block, smem, st>>>(std::forward<Args>(args)...);
+  ++g_launches;
+  CUDA_TRY(cudaGetLastError());
+  return SPART_OK;
+}
+
+// --------------------------------------------------------------------------------------
+// owners of CUDA resources: each releases its resource when it is destroyed or reset, and never writes g_err
+// --------------------------------------------------------------------------------------
+struct DeviceFree { void operator()(void* p) const { cudaFree(p); } };
+struct PinnedFree { void operator()(void* p) const { cudaFreeHost(p); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+template <typename T = void> using DeviceBuf = std::unique_ptr<T, DeviceFree>;
+using PinnedBuf = std::unique_ptr<void, PinnedFree>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventDestroy>;
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamDestroy>;
+
+// (Re)allocate a buffer; the old one is released first, so that a grown buffer never coexists with its predecessor.
+template <typename T>
+static cudaError_t alloc(DeviceBuf<T>& buf, size_t bytes) {
+  buf.reset();
+  T* p = nullptr;
+  const cudaError_t e = cudaMalloc(&p, bytes);
+  buf.reset(e == cudaSuccess ? p : nullptr);
+  return e;
+}
+static cudaError_t alloc(PinnedBuf& buf, size_t bytes) {
+  buf.reset();
+  void* p = nullptr;
+  const cudaError_t e = cudaHostAlloc(&p, bytes, cudaHostAllocDefault);
+  buf.reset(e == cudaSuccess ? p : nullptr);
+  return e;
+}
+static cudaError_t create(Event& ev, unsigned flags = cudaEventDefault) {
+  cudaEvent_t e = nullptr;
+  const cudaError_t r = cudaEventCreateWithFlags(&e, flags);
+  ev.reset(r == cudaSuccess ? e : nullptr);
+  return r;
+}
+static cudaError_t create(Stream& stream) {
+  cudaStream_t s = nullptr;
+  const cudaError_t r = cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
+  stream.reset(r == cudaSuccess ? s : nullptr);
+  return r;
+}
 
 // --------------------------------------------------------------------------------------
 // device-side band table: one row of BT_COUNT doubles per band
@@ -176,51 +230,50 @@ struct SpartCtx {
   int device = 0;
   int n_sensors = 0;
   int sm_count = 0;
-  double* d_lc = nullptr;               // [LC_COUNT][SPART_NWL]
-  std::vector<double*> d_band;          // per sensor [nb][BT_COUNT]
-  std::vector<int32_t*> d_knot;         // per sensor [nb][2]: wl_lo, wl_hi (read by the soil-library kernels)
+  DeviceBuf<double> d_lc;               // [LC_COUNT][SPART_NWL]
+  std::vector<DeviceBuf<double>> d_band;     // per sensor [nb][BT_COUNT]
+  std::vector<DeviceBuf<int32_t>> d_knot;    // per sensor [nb][2]: wl_lo, wl_hi (read by the soil-library kernels)
   std::vector<int> n_bands;
   // optional soil library (spart_create_with_soils): [n_soils + 1][SPART_NWL], the extra last row all NaN
-  double* d_soils = nullptr;
+  DeviceBuf<double> d_soils;
   int n_soils = 0;
   // optional SRF tables per sensor (band_mode "srf"): per band the number of non-zero weights and
   // its offset into the concatenated (wavelength index, normalised weight) lists; nullptr when
   // the sensor was created without them
   struct SrfDev {                       // device arrays behind one SrfPlan (all nullptr: no SRF tables)
     int n_wl = 0, n_slots = 0;
-    int32_t *wl_idx = nullptr, *pair_off = nullptr, *pair_slot = nullptr, *fin_off = nullptr, *fin_band = nullptr,
-            *fin_slot = nullptr;
-    double* pair_w = nullptr;
+    DeviceBuf<int32_t> wl_idx, pair_off, pair_slot, fin_off, fin_band, fin_slot;
+    DeviceBuf<double> pair_w;
   };
   std::vector<SrfDev> srf;
   // host-buffer path: lazily created slots (device params / workspace / output, and pinned host
   // staging buffers that are only allocated when the caller's memory is pageable)
   std::mutex mu;
   static const int kSlots = 4;
-  cudaEvent_t slot_done[kSlots] = {};      // the slot's device->host copy has finished
-  cudaEvent_t slot_k[kSlots] = {};         // the slot's kernels have finished
-  cudaStream_t h2d_stream = nullptr, d2h_stream = nullptr;   // one stream per copy direction (see the host path)
-  cudaStream_t compute_stream = nullptr, join_stream = nullptr;
+  Event slot_done[kSlots];                 // the slot's device->host copy has finished
+  Event slot_k[kSlots];                    // the slot's kernels have finished
+  Stream h2d_stream, d2h_stream;           // one stream per copy direction (see the host path)
+  Stream compute_stream, join_stream;
   static const int kInSlots = 3;           // device buffers for the parameter spans of the host path
-  void* in_params[kInSlots] = {};
-  cudaEvent_t in_done[kInSlots] = {};      // the span's host->device copies have finished
-  cudaEvent_t in_free[kInSlots] = {};      // the kernels of all chunks of the span have finished
+  DeviceBuf<> in_params[kInSlots];
+  Event in_done[kInSlots];                 // the span's host->device copies have finished
+  Event in_free[kInSlots];                 // the kernels of all chunks of the span have finished
   int64_t in_cap = 0;                      // samples per span buffer
-  void* bc_stage = nullptr;                // pinned: element 0 of the broadcast rows of the current call
-  void* in_ets[kInSlots] = {};             // compact output: the span's etscale values, sent back once per span
-  cudaEvent_t ets_done[kInSlots] = {};
-  double* slot_rec[kSlots] = {};
-  void* slot_out[kSlots] = {};
-  void* stage_in[kSlots] = {};     // pinned host
-  void* stage_out[kSlots] = {};    // pinned host
+  PinnedBuf bc_stage;                      // element 0 of the broadcast rows of the current call
+  DeviceBuf<> in_ets[kInSlots];            // compact output: the span's etscale values, sent back once per span
+  Event ets_done[kInSlots];
+  DeviceBuf<double> slot_rec[kSlots];
+  DeviceBuf<> slot_out[kSlots];
+  PinnedBuf stage_in[kSlots];
+  PinnedBuf stage_out[kSlots];
   int64_t slot_cap = 0;        // samples per slot
   size_t slot_out_cap = 0;     // bytes of output per slot
   size_t stage_in_cap = 0, stage_out_cap = 0;   // bytes
-  HostPool* pool = nullptr;
+  std::unique_ptr<HostPool> pool;
   // optional per-kernel timing of spart_forward_bands (spart_profile_enable / _read)
   mutable std::mutex prof_mu;
   mutable bool profiling = false;
-  struct ProfEvents { cudaEvent_t e[4]; };
+  struct ProfEvents { Event e[4]; };
   mutable std::vector<ProfEvents> prof_pending;
   mutable std::vector<ProfEvents> prof_free;
 };
@@ -1573,61 +1626,38 @@ __global__ void __launch_bounds__(1024, 1) fp64_register_chain_kernel(double* ou
   if (u == -12345.678) out[0] = u;   // never true; keeps the chain alive
 }
 
-static int time_register_chain(int sm_count, double* tflops) {
-  double* d = nullptr;
-  CUDA_TRY(cudaMalloc(&d, sizeof(double)));
-  const int iters = 1 << 12, threads = 1024, blocks = sm_count;     // 8 warps per scheduler
-  cudaEvent_t e0, e1;
-  CUDA_TRY(cudaEventCreate(&e0));
-  CUDA_TRY(cudaEventCreate(&e1));
+// Best rate of four timed runs of `run(d)` on the default stream, the first run not counted (warm-up); `d` is a
+// device scratch double the kernels may write, `flops` the work of one run.
+template <typename Run>
+static int time_peak(double flops, double* tflops, Run run) {
+  DeviceBuf<double> d;
+  Event e0, e1;
+  CUDA_TRY(alloc(d, sizeof(double)));
+  CUDA_TRY(create(e0));
+  CUDA_TRY(create(e1));
   double best = 0.0;
   for (int rep = 0; rep < 4; ++rep) {
-    CUDA_TRY(cudaEventRecord(e0));
-    fp64_register_chain_kernel<<<blocks, threads>>>(d, iters);
-    ++g_launches;
-    CUDA_TRY(cudaEventRecord(e1));
-    CUDA_TRY(cudaEventSynchronize(e1));
+    CUDA_TRY(cudaEventRecord(e0.get()));
+    const int rc = run(d.get());
+    if (rc) return rc;
+    CUDA_TRY(cudaEventRecord(e1.get()));
+    CUDA_TRY(cudaEventSynchronize(e1.get()));
     float ms = 0.f;
-    CUDA_TRY(cudaEventElapsedTime(&ms, e0, e1));
-    const double flops = 2.0 * 6.0 * 4.0 * (double)iters * threads * (double)blocks;
+    CUDA_TRY(cudaEventElapsedTime(&ms, e0.get(), e1.get()));
     const double tf = flops / (ms * 1e-3) / 1e12;
     if (rep > 0 && tf > best) best = tf;
   }
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  cudaFree(d);
   *tflops = best;
   return SPART_OK;
 }
 
 template <typename T>
 static int time_fma(int sm_count, double* tflops) {
-  T* d = nullptr;
-  CUDA_TRY(cudaMalloc(&d, sizeof(T)));
   const int iters = 1 << 14, threads = 512, blocks = sm_count * 8;
-  cudaEvent_t e0, e1;
-  CUDA_TRY(cudaEventCreate(&e0));
-  CUDA_TRY(cudaEventCreate(&e1));
-  double best = 0.0;
-  for (int rep = 0; rep < 4; ++rep) {
-    CUDA_TRY(cudaEventRecord(e0));
-    fma_chain_kernel<T><<<blocks, threads>>>(d, iters, (T)1.0000001, (T)1e-7);
-    ++g_launches;
-    CUDA_TRY(cudaEventRecord(e1));
-    CUDA_TRY(cudaEventSynchronize(e1));
-    float ms = 0.f;
-    CUDA_TRY(cudaEventElapsedTime(&ms, e0, e1));
-    const double flops = 2.0 * 8.0 * (double)iters * threads * (double)blocks;
-    const double tf = flops / (ms * 1e-3) / 1e12;
-    if (rep > 0 && tf > best) best = tf;
-  }
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  cudaFree(d);
-  *tflops = best;
-  return SPART_OK;
+  return time_peak(2.0 * 8.0 * (double)iters * threads * (double)blocks, tflops, [&](double* d) {
+    return launch(fma_chain_kernel<T>, blocks, threads, 0, nullptr, (T*)d, iters, (T)1.0000001, (T)1e-7);
+  });
 }
-
 
 // --------------------------------------------------------------------------------------
 // C ABI
@@ -1735,53 +1765,22 @@ int spart_destroy(SpartCtx* ctx) {
   // work of device-path calls may still be queued on callers' streams and read the context's tables: wait for
   // everything on the device, not only for the host path's own streams, before anything is freed
   cudaDeviceSynchronize();
-  for (int i = 0; i < SpartCtx::kSlots; ++i) {
-    if (ctx->slot_rec[i]) cudaFree(ctx->slot_rec[i]);
-    if (ctx->slot_out[i]) cudaFree(ctx->slot_out[i]);
-    if (ctx->stage_in[i]) cudaFreeHost(ctx->stage_in[i]);
-    if (ctx->stage_out[i]) cudaFreeHost(ctx->stage_out[i]);
-    if (ctx->slot_done[i]) cudaEventDestroy(ctx->slot_done[i]);
-    if (ctx->slot_k[i]) cudaEventDestroy(ctx->slot_k[i]);
-  }
-  for (int i = 0; i < SpartCtx::kInSlots; ++i) {
-    if (ctx->in_params[i]) cudaFree(ctx->in_params[i]);
-    if (ctx->in_done[i]) cudaEventDestroy(ctx->in_done[i]);
-    if (ctx->in_free[i]) cudaEventDestroy(ctx->in_free[i]);
-    if (ctx->in_ets[i]) cudaFree(ctx->in_ets[i]);
-    if (ctx->ets_done[i]) cudaEventDestroy(ctx->ets_done[i]);
-  }
-  if (ctx->bc_stage) cudaFreeHost(ctx->bc_stage);
-  if (ctx->h2d_stream) cudaStreamDestroy(ctx->h2d_stream);
-  if (ctx->d2h_stream) cudaStreamDestroy(ctx->d2h_stream);
-  if (ctx->compute_stream) cudaStreamDestroy(ctx->compute_stream);
-  if (ctx->join_stream) cudaStreamDestroy(ctx->join_stream);
-  delete ctx->pool;
-  for (auto& pe : ctx->prof_pending) for (int i = 0; i < 4; ++i) cudaEventDestroy(pe.e[i]);
-  for (auto& pe : ctx->prof_free) for (int i = 0; i < 4; ++i) cudaEventDestroy(pe.e[i]);
-  for (double* d : ctx->d_band) cudaFree(d);
-  for (int32_t* d : ctx->d_knot) cudaFree(d);
-  if (ctx->d_soils) cudaFree(ctx->d_soils);
-  for (auto& v : ctx->srf) {
-    cudaFree(v.wl_idx); cudaFree(v.pair_off); cudaFree(v.pair_slot); cudaFree(v.fin_off); cudaFree(v.fin_band);
-    cudaFree(v.fin_slot); cudaFree(v.pair_w);
-  }
-  if (ctx->d_lc) cudaFree(ctx->d_lc);
   delete ctx;
   return SPART_OK;
 }
 
 }  // extern "C"
 
-// SRF band mode: turn the per-band (wavelength, weight) lists into the schedule band_kernel_srf walks --
-// distinct wavelengths in ascending order, per wavelength the (accumulator slot, weight) pairs to add and
-// the bands that are complete after it.  Slots are an interval colouring of the bands' supports.
 template <typename T>
-static int upload(const std::vector<T>& v, T** d) {
-  CUDA_TRY(cudaMalloc(d, sizeof(T) * (v.empty() ? 1 : v.size())));
-  if (!v.empty()) CUDA_TRY(cudaMemcpy(*d, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice));
+static int upload(const std::vector<T>& v, DeviceBuf<T>& d) {
+  CUDA_TRY(alloc(d, sizeof(T) * (v.empty() ? 1 : v.size())));
+  if (!v.empty()) CUDA_TRY(cudaMemcpy(d.get(), v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice));
   return SPART_OK;
 }
 
+// SRF band mode: turn the per-band (wavelength, weight) lists into the schedule band_kernel_srf walks --
+// distinct wavelengths in ascending order, per wavelength the (accumulator slot, weight) pairs to add and
+// the bands that are complete after it.  Slots are an interval colouring of the bands' supports.
 static int build_srf_plan(const SpartSensor& S, SpartCtx::SrfDev& dev) {
   const int nb = S.n_bands;
   std::vector<int64_t> off(nb + 1, 0);
@@ -1867,36 +1866,38 @@ static int build_srf_plan(const SpartSensor& S, SpartCtx::SrfDev& dev) {
   dev.n_wl = (int)wl_idx.size();
   dev.n_slots = n_slots;
   int rc;
-  if ((rc = upload(wl_idx, &dev.wl_idx)) || (rc = upload(pair_off, &dev.pair_off)) ||
-      (rc = upload(pair_slot, &dev.pair_slot)) || (rc = upload(pair_w, &dev.pair_w)) ||
-      (rc = upload(fin_off, &dev.fin_off)) || (rc = upload(fin_band, &dev.fin_band)) ||
-      (rc = upload(fin_slot, &dev.fin_slot)))
+  if ((rc = upload(wl_idx, dev.wl_idx)) || (rc = upload(pair_off, dev.pair_off)) ||
+      (rc = upload(pair_slot, dev.pair_slot)) || (rc = upload(pair_w, dev.pair_w)) ||
+      (rc = upload(fin_off, dev.fin_off)) || (rc = upload(fin_band, dev.fin_band)) ||
+      (rc = upload(fin_slot, dev.fin_slot)))
     return rc;
   return SPART_OK;
 }
 
-extern "C" {
-
-// body of spart_create; on any failure the caller releases the partially built context
+// body of spart_create; on any failure the caller deletes the partially built context, which releases it
 static int create_into(SpartCtx* ctx, const SpartTables* tables, const SpartSensor* sensors, int32_t n_sensors,
                        const double* soils, int32_t n_soils, int32_t device) {
   CUDA_TRY(cudaDeviceGetAttribute(&ctx->sm_count, cudaDevAttrMultiProcessorCount, device));
   int rc = init_device_constants(device);
   if (rc) return rc;
   const size_t lc_bytes = sizeof(double) * LC_COUNT * SPART_NWL;
-  CUDA_TRY(cudaMalloc(&ctx->d_lc, lc_bytes));
-  CUDA_TRY(cudaMemcpy(ctx->d_lc, tables->lc, lc_bytes, cudaMemcpyHostToDevice));
+  CUDA_TRY(alloc(ctx->d_lc, lc_bytes));
+  CUDA_TRY(cudaMemcpy(ctx->d_lc.get(), tables->lc, lc_bytes, cudaMemcpyHostToDevice));
   if (soils) {
     // the library plus one row of NaN that invalid sample indices are pointed at
     const size_t lib_bytes = sizeof(double) * (size_t)n_soils * SPART_NWL;
     const std::vector<double> nan_row(SPART_NWL, __builtin_nan(""));
-    CUDA_TRY(cudaMalloc(&ctx->d_soils, lib_bytes + sizeof(double) * SPART_NWL));
-    CUDA_TRY(cudaMemcpy(ctx->d_soils, soils, lib_bytes, cudaMemcpyHostToDevice));
-    CUDA_TRY(cudaMemcpy(ctx->d_soils + (size_t)n_soils * SPART_NWL, nan_row.data(), sizeof(double) * SPART_NWL,
+    CUDA_TRY(alloc(ctx->d_soils, lib_bytes + sizeof(double) * SPART_NWL));
+    CUDA_TRY(cudaMemcpy(ctx->d_soils.get(), soils, lib_bytes, cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(ctx->d_soils.get() + (size_t)n_soils * SPART_NWL, nan_row.data(), sizeof(double) * SPART_NWL,
                         cudaMemcpyHostToDevice));
     ctx->n_soils = n_soils;
   }
 
+  ctx->n_bands.resize(n_sensors);
+  ctx->d_band.resize(n_sensors);
+  ctx->d_knot.resize(n_sensors);
+  ctx->srf.resize(n_sensors);
   for (int i = 0; i < n_sensors; ++i) {
     const SpartSensor& S = sensors[i];
     std::vector<double> bt((size_t)S.n_bands * BT_COUNT, 0.0);
@@ -1911,20 +1912,13 @@ static int create_into(SpartCtx* ctx, const SpartTables* tables, const SpartSens
         row[BT_LC1 + r] = tables->lc[(size_t)r * SPART_NWL + S.wl_hi[b]];
       }
     }
-    // every vector gets its slot first, so that spart_destroy releases whatever was allocated
-    ctx->d_band.push_back(nullptr);
-    ctx->d_knot.push_back(nullptr);
-    ctx->n_bands.push_back(S.n_bands);
-    ctx->srf.emplace_back();
-    CUDA_TRY(cudaMalloc(&ctx->d_band[i], bt.size() * sizeof(double)));
-    CUDA_TRY(cudaMemcpy(ctx->d_band[i], bt.data(), bt.size() * sizeof(double), cudaMemcpyHostToDevice));
     std::vector<int32_t> knots((size_t)S.n_bands * 2);
     for (int b = 0; b < S.n_bands; ++b) {
       knots[(size_t)b * 2] = S.wl_lo[b];
       knots[(size_t)b * 2 + 1] = S.wl_hi[b];
     }
-    rc = upload(knots, &ctx->d_knot[i]);
-    if (rc) return rc;
+    ctx->n_bands[i] = S.n_bands;
+    if ((rc = upload(bt, ctx->d_band[i])) || (rc = upload(knots, ctx->d_knot[i]))) return rc;
     if (S.srf_idx && S.srf_len && S.srf_w) {
       rc = build_srf_plan(S, ctx->srf[i]);
       if (rc) return rc;
@@ -1950,21 +1944,17 @@ static int create_ctx(const SpartTables* tables, const SpartSensor* sensors, int
         return fail(SPART_EINVAL, "spart_create: band knot outside 400..2400 nm%s");
   }
   GUARD_DEVICE(device);
-  SpartCtx* ctx = new (std::nothrow) SpartCtx();
+  std::unique_ptr<SpartCtx> ctx(new (std::nothrow) SpartCtx());
   if (!ctx) return fail(SPART_ENOMEM, "spart_create: out of host memory%s");
   ctx->device = device;
   ctx->n_sensors = n_sensors;
-  const int rc = create_into(ctx, tables, sensors, n_sensors, soils, n_soils, device);
-  if (rc) {
-    char keep[sizeof(g_err)];
-    memcpy(keep, g_err, sizeof(keep));      // spart_destroy must not disturb the error text
-    spart_destroy(ctx);
-    memcpy(g_err, keep, sizeof(keep));
-    return rc;
-  }
-  *out = ctx;
+  const int rc = create_into(ctx.get(), tables, sensors, n_sensors, soils, n_soils, device);
+  if (rc) return rc;
+  *out = ctx.release();
   return SPART_OK;
 }
+
+extern "C" {
 
 int spart_create(const SpartTables* tables, const SpartSensor* sensors, int32_t n_sensors, int32_t device,
                  SpartCtx** out) {
@@ -1985,26 +1975,21 @@ size_t spart_workspace_bytes(const SpartCtx* ctx, int64_t n) {
   return sizeof(double) * (size_t)kWsRows * (size_t)n;
 }
 
+}  // extern "C"
+
 static int launch_lidf(const Params& P, int64_t n_batch, double* ws, cudaStream_t st) {
   // LIDFa and LIDFb both broadcast rows (a look-up table with one leaf-angle distribution): the twelve
   // iterations run once, geometry_kernel reads element 0 of the F rows (kFlagLidfBcast)
   const int64_t n = ((P.bc & kLidfRows) == kLidfRows) ? 1 : n_batch;
-  const unsigned blocks = (unsigned)((n + kL2Samples - 1) / kL2Samples);
-  lidf_kernel<<<blocks, kL2Threads, 0, st>>>(P.ptr(P_LIDFA, 0), P.ptr(P_LIDFB, 0),
-                                                ((P.bc >> P_LIDFA) & 1u) ? 0 : 1, ((P.bc >> P_LIDFB) & 1u) ? 0 : 1, n,
-                                                ws + (size_t)kRowF * n_batch, n_batch, 1);
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  return SPART_OK;
+  return launch(lidf_kernel, (unsigned)((n + kL2Samples - 1) / kL2Samples), kL2Threads, 0, st, P.ptr(P_LIDFA, 0),
+                P.ptr(P_LIDFB, 0), ((P.bc >> P_LIDFA) & 1u) ? 0 : 1, ((P.bc >> P_LIDFB) & 1u) ? 0 : 1, n,
+                ws + (size_t)kRowF * n_batch, n_batch, 1);
 }
 
 static int launch_geometry(const Params& P, int64_t n, double* ws, int kflags, cudaStream_t st) {
-  const unsigned blocks = (unsigned)((n + kSampleThreads - 1) / kSampleThreads);
   if ((P.bc & kLidfRows) == kLidfRows && !(kflags & kFlagLidfDirect)) kflags |= kFlagLidfBcast;
-  geometry_kernel<<<blocks, kSampleThreads, 0, st>>>(P, n, ws, kflags);
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  return SPART_OK;
+  return launch(geometry_kernel, (unsigned)((n + kSampleThreads - 1) / kSampleThreads), kSampleThreads, 0, st, P, n,
+                ws, kflags);
 }
 
 static int check_batch(const SpartCtx* ctx, const void* params, int64_t n, int64_t ld, uint32_t bc, const void* ws,
@@ -2054,32 +2039,27 @@ static int check_mode(const SpartCtx* ctx, int32_t sensor, int32_t precision, in
   return check_soil_library(ctx, flags, who);
 }
 
-}  // extern "C"
-
 template <typename TIO>
 static int launch_fp32(const SpartCtx* ctx, int sensor, const void* params_dev, const void* params_bc_dev, int64_t n,
                        int64_t ld, uint32_t bc, int kflags, bool reuse, bool compact, bool library, float* rec,
                        void* out_dev,
                        dim3 grid, cudaStream_t st, bool prof, const SpartCtx::ProfEvents& pe) {
   const ParamsT<TIO> P{(const TIO*)params_dev, ld, bc, (const TIO*)params_bc_dev};
-  if (prof) CUDA_TRY(cudaEventRecord(pe.e[1], st));
+  const double* band = ctx->d_band[sensor].get();
+  const int nb = ctx->n_bands[sensor];
+  if (prof) CUDA_TRY(cudaEventRecord(pe.e[1].get(), st));
   if (!reuse) {
     NvtxRange r("spart::geometry_f32");
-    const unsigned blocks = (unsigned)((n + kSampleThreads - 1) / kSampleThreads);
-    geometry_kernel_f32<TIO><<<blocks, kSampleThreads, 0, st>>>(P, n, rec, kflags);
-    ++g_launches;
-    CUDA_TRY(cudaGetLastError());
+    const int rc = launch(geometry_kernel_f32<TIO>, (unsigned)((n + kSampleThreads - 1) / kSampleThreads),
+                          kSampleThreads, 0, st, P, n, rec, kflags);
+    if (rc) return rc;
   }
-  if (prof) CUDA_TRY(cudaEventRecord(pe.e[2], st));
+  if (prof) CUDA_TRY(cudaEventRecord(pe.e[2].get(), st));
   NvtxRange r("spart::bands_f32");
   if (library)
-    soillib_bands_f32<TIO><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], ctx->n_bands[sensor],
-                                                          (TIO*)out_dev, compact ? 1 : 0,
-                                                          SoilLib{ctx->d_soils, ctx->n_soils}, ctx->d_knot[sensor]);
-  else
-    band_kernel_f32<TIO><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], ctx->n_bands[sensor],
-                                                        (TIO*)out_dev, compact ? 1 : 0);
-  return SPART_OK;
+    return launch(soillib_bands_f32<TIO>, grid, kBandThreads, 0, st, P, n, rec, band, nb, (TIO*)out_dev,
+                  compact ? 1 : 0, SoilLib{ctx->d_soils.get(), ctx->n_soils}, ctx->d_knot[sensor].get());
+  return launch(band_kernel_f32<TIO>, grid, kBandThreads, 0, st, P, n, rec, band, nb, (TIO*)out_dev, compact ? 1 : 0);
 }
 
 // spart_forward_bands with a separate base for the broadcast rows (see ParamsT); the host-buffer path calls it on
@@ -2095,6 +2075,7 @@ static int forward_bands_impl(const SpartCtx* ctx, int32_t sensor, const void* p
   GUARD_DEVICE(ctx->device);
   cudaStream_t st = (cudaStream_t)stream;
   double* rec = (double*)workspace_dev;
+  // the call's profiling events: released on any return before they are handed to prof_pending
   SpartCtx::ProfEvents pe;
   bool prof = false;
   {
@@ -2102,24 +2083,25 @@ static int forward_bands_impl(const SpartCtx* ctx, int32_t sensor, const void* p
     if (ctx->profiling) {
       prof = true;
       if (!ctx->prof_free.empty()) {
-        pe = ctx->prof_free.back();
+        pe = std::move(ctx->prof_free.back());
         ctx->prof_free.pop_back();
       } else {
-        for (int i = 0; i < 4; ++i) CUDA_TRY(cudaEventCreate(&pe.e[i]));
+        for (Event& e : pe.e) CUDA_TRY(create(e));
       }
     }
   }
   const int nb = ctx->n_bands[sensor];
+  const double* band = ctx->d_band[sensor].get();
   dim3 grid((unsigned)((nb + kBandChunk - 1) / kBandChunk), (unsigned)((n + kBandThreads - 1) / kBandThreads));
   const bool reuse = (flags & SPART_FLAG_REUSE_RECORD) != 0;   // workspace already holds this batch's record
-  const bool compact = (flags & SPART_FLAG_COMPACT_OUT) != 0;
+  const int compact = (flags & SPART_FLAG_COMPACT_OUT) ? 1 : 0;
   // one sun / observer geometry for the whole batch by construction: rows 19..21 are broadcast rows
   const bool uniform = (broadcast_rows & kGeometryRows) == kGeometryRows;
   const bool user_lidf = (flags & SPART_FLAG_USER_LIDF) != 0;   // the workspace holds the caller's distribution
   const bool library = (flags & SPART_FLAG_SOIL_LIBRARY) != 0;    // per-sample dry soil from the context's library
-  const SoilLib lib{ctx->d_soils, ctx->n_soils};
+  const SoilLib lib{ctx->d_soils.get(), ctx->n_soils};
   const int kflags = soil_kflags(flags) | (uniform ? kFlagUniform : 0) | (user_lidf ? kFlagLidfDirect : 0);
-  if (prof) CUDA_TRY(cudaEventRecord(pe.e[0], st));
+  if (prof) CUDA_TRY(cudaEventRecord(pe.e[0].get(), st));
   if (precision == SPART_FP64) {
     const Params P{(const double*)params_dev, ld, broadcast_rows, (const double*)params_bc_dev};
     double* out = (double*)out_dev;
@@ -2128,55 +2110,46 @@ static int forward_bands_impl(const SpartCtx* ctx, int32_t sensor, const void* p
       rc = launch_lidf(P, n, rec, st);
       if (rc) return rc;
     }
-    if (prof) CUDA_TRY(cudaEventRecord(pe.e[1], st));
+    if (prof) CUDA_TRY(cudaEventRecord(pe.e[1].get(), st));
     if (!reuse) {
       NvtxRange r("spart::geometry");
       rc = launch_geometry(P, n, rec, kflags, st);
       if (rc) return rc;
     }
-    if (prof) CUDA_TRY(cudaEventRecord(pe.e[2], st));
+    if (prof) CUDA_TRY(cudaEventRecord(pe.e[2].get(), st));
     NvtxRange r("spart::bands");
     if (flags & SPART_FLAG_SRF_BANDS) {
       const SpartCtx::SrfDev& v = ctx->srf[sensor];
-      const SrfPlan plan{v.n_wl, v.n_slots, v.wl_idx, v.pair_off, v.pair_slot, v.pair_w, v.fin_off, v.fin_band,
-                         v.fin_slot};
+      const SrfPlan plan{v.n_wl, v.n_slots, v.wl_idx.get(), v.pair_off.get(), v.pair_slot.get(), v.pair_w.get(),
+                         v.fin_off.get(), v.fin_band.get(), v.fin_slot.get()};
       const size_t acc_bytes = sizeof(double) * v.n_slots * 4 * kBandThreads;
       const unsigned blocks = (unsigned)((n + kBandThreads - 1) / kBandThreads);
       // the kernels' dynamic shared-memory cap was set to the kSrfMaxSlots bound once per device
-      if (library) {
-        soillib_srf<<<blocks, kBandThreads, acc_bytes, st>>>(P, n, rec, ctx->d_band[sensor], ctx->d_lc, plan, nb, out,
-                                                             compact ? 1 : 0, lib);
-      } else {
-        band_kernel_srf<<<blocks, kBandThreads, acc_bytes, st>>>(P, n, rec, ctx->d_band[sensor], ctx->d_lc, plan, nb,
-                                                                 out, compact ? 1 : 0);
-      }
-    } else if (library) {
-      if (uniform)
-        soillib_bands<true><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], nb, out, compact ? 1 : 0,
-                                                           lib, ctx->d_knot[sensor]);
+      if (library)
+        rc = launch(soillib_srf, blocks, kBandThreads, acc_bytes, st, P, n, rec, band, ctx->d_lc.get(), plan, nb, out,
+                    compact, lib);
       else
-        soillib_bands<false><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], nb, out, compact ? 1 : 0,
-                                                            lib, ctx->d_knot[sensor]);
-    } else if (uniform) {
-      band_kernel<true><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], nb, out, compact ? 1 : 0);
+        rc = launch(band_kernel_srf, blocks, kBandThreads, acc_bytes, st, P, n, rec, band, ctx->d_lc.get(), plan, nb,
+                    out, compact);
+    } else if (library) {
+      rc = launch(uniform ? soillib_bands<true> : soillib_bands<false>, grid, kBandThreads, 0, st, P, n, rec, band, nb,
+                  out, compact, lib, ctx->d_knot[sensor].get());
     } else {
-      band_kernel<false><<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], nb, out, compact ? 1 : 0);
+      rc = launch(uniform ? band_kernel<true> : band_kernel<false>, grid, kBandThreads, 0, st, P, n, rec, band, nb,
+                  out, compact);
     }
-  } else {   // SPART_FP32: the leaf angles are solved inside the geometry kernel
-    if (flags & SPART_FLAG_F32_IO)
-      rc = launch_fp32<float>(ctx, sensor, params_dev, params_bc_dev, n, ld, broadcast_rows, kflags, reuse, compact, library, (float*)rec,
-                              out_dev, grid, st, prof, pe);
-    else
-      rc = launch_fp32<double>(ctx, sensor, params_dev, params_bc_dev, n, ld, broadcast_rows, kflags, reuse, compact, library, (float*)rec,
-                               out_dev, grid, st, prof, pe);
-    if (rc) return rc;
+  } else if (flags & SPART_FLAG_F32_IO) {   // SPART_FP32: the leaf angles are solved inside the geometry kernel
+    rc = launch_fp32<float>(ctx, sensor, params_dev, params_bc_dev, n, ld, broadcast_rows, kflags, reuse, compact,
+                            library, (float*)rec, out_dev, grid, st, prof, pe);
+  } else {
+    rc = launch_fp32<double>(ctx, sensor, params_dev, params_bc_dev, n, ld, broadcast_rows, kflags, reuse, compact,
+                             library, (float*)rec, out_dev, grid, st, prof, pe);
   }
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
+  if (rc) return rc;
   if (prof) {
-    CUDA_TRY(cudaEventRecord(pe.e[3], st));
+    CUDA_TRY(cudaEventRecord(pe.e[3].get(), st));
     std::lock_guard<std::mutex> lock(ctx->prof_mu);
-    ctx->prof_pending.push_back(pe);
+    ctx->prof_pending.push_back(std::move(pe));
   }
   return SPART_OK;
 }
@@ -2202,7 +2175,7 @@ int spart_profile_enable(SpartCtx* ctx, int32_t on) {
   if (!ctx) return fail(SPART_EINVAL, "spart_profile_enable: null context%s");
   std::lock_guard<std::mutex> lock(ctx->prof_mu);
   ctx->profiling = on != 0;
-  for (auto& pe : ctx->prof_pending) ctx->prof_free.push_back(pe);
+  for (auto& pe : ctx->prof_pending) ctx->prof_free.push_back(std::move(pe));
   ctx->prof_pending.clear();
   return SPART_OK;
 }
@@ -2213,16 +2186,16 @@ int spart_profile_read(SpartCtx* ctx, double* kernel_ms, int64_t* calls) {
   std::lock_guard<std::mutex> lock(ctx->prof_mu);
   double acc[SPART_NKERNELS] = {0.0, 0.0, 0.0};
   for (auto& pe : ctx->prof_pending) {
-    CUDA_TRY(cudaEventSynchronize(pe.e[3]));
+    CUDA_TRY(cudaEventSynchronize(pe.e[3].get()));
     for (int k = 0; k < SPART_NKERNELS; ++k) {
       float ms = 0.f;
-      CUDA_TRY(cudaEventElapsedTime(&ms, pe.e[k], pe.e[k + 1]));
+      CUDA_TRY(cudaEventElapsedTime(&ms, pe.e[k].get(), pe.e[k + 1].get()));
       acc[k] += ms;
     }
-    ctx->prof_free.push_back(pe);
   }
   for (int k = 0; k < SPART_NKERNELS; ++k) kernel_ms[k] = acc[k];
   *calls = (int64_t)ctx->prof_pending.size();
+  for (auto& pe : ctx->prof_pending) ctx->prof_free.push_back(std::move(pe));
   ctx->prof_pending.clear();
   return SPART_OK;
 }
@@ -2253,12 +2226,12 @@ int spart_forward_spectrum(const SpartCtx* ctx, const double* params_dev, int64_
     const unsigned ny = (unsigned)((n - s0 < 65535) ? (n - s0) : 65535);
     dim3 grid((SPART_NWL_S + kSpecThreads - 1) / kSpecThreads, ny);
     if (flags & SPART_FLAG_SOIL_LIBRARY)
-      soillib_spectrum<<<grid, kSpecThreads, 0, st>>>(P, n, rec, ctx->d_lc, s0, rho_thermal, tau_thermal, out_dev,
-                                                      SoilLib{ctx->d_soils, ctx->n_soils});
+      rc = launch(soillib_spectrum, grid, kSpecThreads, 0, st, P, n, rec, ctx->d_lc.get(), s0, rho_thermal,
+                  tau_thermal, out_dev, SoilLib{ctx->d_soils.get(), ctx->n_soils});
     else
-      spectrum_kernel<<<grid, kSpecThreads, 0, st>>>(P, n, rec, ctx->d_lc, s0, rho_thermal, tau_thermal, out_dev);
-    ++g_launches;
-    CUDA_TRY(cudaGetLastError());
+      rc = launch(spectrum_kernel, grid, kSpecThreads, 0, st, P, n, rec, ctx->d_lc.get(), s0, rho_thermal,
+                  tau_thermal, out_dev);
+    if (rc) return rc;
   }
   return SPART_OK;
 }
@@ -2280,10 +2253,7 @@ int spart_smac(const SpartCtx* ctx, int32_t sensor, const double* params_dev, in
   if (rc) return rc;
   const int nb = ctx->n_bands[sensor];
   dim3 grid((unsigned)nb, (unsigned)((n + kBandThreads - 1) / kBandThreads));
-  smac_kernel<<<grid, kBandThreads, 0, st>>>(P, n, rec, ctx->d_band[sensor], nb, out_dev);
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  return SPART_OK;
+  return launch(smac_kernel, grid, kBandThreads, 0, st, P, n, rec, ctx->d_band[sensor].get(), nb, out_dev);
 }
 
 int spart_sailh(const SpartCtx* ctx, const double* params_dev, int64_t n, int64_t ld, const double* soil_refl_dev,
@@ -2307,121 +2277,107 @@ int spart_sailh(const SpartCtx* ctx, const double* params_dev, int64_t n, int64_
   for (int64_t s0 = 0; s0 < n; s0 += 65535) {
     const unsigned ny = (unsigned)((n - s0 < 65535) ? (n - s0) : 65535);
     dim3 grid((SPART_NWL_S + 255) / 256, ny);
-    sailh_spectra_kernel<<<grid, 256, 0, st>>>(P, n, rec, soil_refl_dev, leaf_refl_dev, leaf_tran_dev,
-                                               spectra_stride, s0, out_dev);
-    ++g_launches;
-    CUDA_TRY(cudaGetLastError());
+    rc = launch(sailh_spectra_kernel, grid, 256, 0, st, P, n, rec, soil_refl_dev, leaf_refl_dev, leaf_tran_dev,
+                spectra_stride, s0, out_dev);
+    if (rc) return rc;
   }
   return SPART_OK;
 }
 
 size_t spart_lut_workspace_bytes(int64_t m) { return m > 0 ? sizeof(unsigned long long) * (size_t)m : 0; }
 
-int spart_lut_nearest(const float* lut_dev, int64_t n, int32_t n_bands, const float* obs_dev, int64_t m,
-                      const float* weights_dev, int64_t index_offset, void* workspace_dev, int64_t* best_index_dev,
-                      float* best_cost_dev, unsigned long long* packed_dev, void* stream) {
-  if (!lut_dev || !obs_dev || (!workspace_dev && m > 0))
-    return fail(SPART_EINVAL, "spart_lut_nearest: null argument%s");
+}  // extern "C"
+
+// argument check of spart_lut_nearest (`who`, max_bands 32) and spart_lut_nearest_tc (max_bands 30)
+static int check_lut(const char* who, int max_bands, const float* lut_dev, int64_t n, int32_t n_bands,
+                     const float* obs_dev, int64_t m, int64_t index_offset, const void* workspace_dev,
+                     const int64_t* best_index_dev, const float* best_cost_dev, const unsigned long long* packed_dev) {
+  if (!lut_dev || !obs_dev || (!workspace_dev && m > 0)) return fail(SPART_EINVAL, "%s: null argument", who);
   if (!packed_dev && (!best_index_dev || !best_cost_dev))
-    return fail(SPART_EINVAL, "spart_lut_nearest: need best_index_dev + best_cost_dev or packed_dev%s");
-  if (n <= 0 || n > 0x7fffffffLL || m < 0 || n_bands < 1 || n_bands > 32 || index_offset < 0 ||
-      index_offset + n > 0xffffffffLL)
-    return fail(SPART_EINVAL,
-                "spart_lut_nearest: need 1 <= n < 2^31, m >= 0, 1 <= n_bands <= 32, index_offset + n < 2^32%s");
-  if (m == 0) return SPART_OK;
-  NvtxRange r("spart::lut_nearest");
-  cudaStream_t st = (cudaStream_t)stream;
+    return fail(SPART_EINVAL, "%s: need best_index_dev + best_cost_dev or packed_dev", who);
+  if (n <= 0 || n > 0x7fffffffLL || m < 0 || n_bands < 1 || n_bands > max_bands || index_offset < 0 ||
+      index_offset + n > 0xffffffffLL) {
+    snprintf(g_err, sizeof(g_err),
+             "%s: need 1 <= n < 2^31, m >= 0, 1 <= n_bands <= %d, index_offset + n < 2^32", who, max_bands);
+    return SPART_EINVAL;
+  }
+  return SPART_OK;
+}
+
+// Where a LUT search keeps its (cost, index) words, reset to "no entry", and its grid: `obs_per_block` observations
+// by LUT slices of whole `tile`-entry tiles, enough slices that the grid fills the GPU a few times over.
+struct LutPlan {
+  unsigned long long* best;
+  dim3 grid;
+  int64_t per_slice;
+};
+static int plan_lut(int64_t n, int64_t m, int64_t tile, int obs_per_block, void* workspace_dev,
+                    unsigned long long* packed_dev, cudaStream_t st, LutPlan& p) {
   // with packed_dev the (cost, index) words are the result (a sharded search min-reduces them across
   // GPUs before unpacking); otherwise they live in the workspace
-  unsigned long long* best = packed_dev ? packed_dev : (unsigned long long*)workspace_dev;
-  CUDA_TRY(cudaMemsetAsync(best, 0xff, sizeof(unsigned long long) * m, st));
+  p.best = packed_dev ? packed_dev : (unsigned long long*)workspace_dev;
+  CUDA_TRY(cudaMemsetAsync(p.best, 0xff, sizeof(unsigned long long) * m, st));
   int dev = 0, sms = 148;
   CUDA_TRY(cudaGetDevice(&dev));
   CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  const int64_t obs_blocks = (m + kLutObs - 1) / kLutObs;
-  // enough LUT slices that the grid fills the GPU a few times over, each slice a whole number of tiles
+  const int64_t obs_blocks = (m + obs_per_block - 1) / obs_per_block;
   int64_t slices = (8LL * sms + obs_blocks - 1) / obs_blocks;
-  const int64_t max_slices = (n + kLutTile - 1) / kLutTile;
+  const int64_t max_slices = (n + tile - 1) / tile;
   if (slices > max_slices) slices = max_slices;
   if (slices > 65535) slices = 65535;
   if (slices < 1) slices = 1;
-  int64_t per_slice = (n + slices - 1) / slices;
-  per_slice = ((per_slice + kLutTile - 1) / kLutTile) * kLutTile;
-  slices = (n + per_slice - 1) / per_slice;
-  dim3 grid((unsigned)obs_blocks, (unsigned)slices);
-  const int nb4 = (n_bands + 3) / 4;
-#define SPART_LUT_CASE(K)                                                                                          \
-  case K:                                                                                                          \
-    lut_nearest_kernel<K><<<grid, kLutObs, 0, st>>>(lut_dev, n, n_bands, obs_dev, m, weights_dev, per_slice,       \
-                                                    (unsigned)index_offset, best);                                 \
-    break;
-  switch (nb4) {
-    SPART_LUT_CASE(1) SPART_LUT_CASE(2) SPART_LUT_CASE(3) SPART_LUT_CASE(4)
-    SPART_LUT_CASE(5) SPART_LUT_CASE(6) SPART_LUT_CASE(7) SPART_LUT_CASE(8)
-  }
-#undef SPART_LUT_CASE
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  if (best_index_dev && best_cost_dev && !packed_dev) {
-    lut_unpack_kernel<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(best, m, best_index_dev, best_cost_dev);
-    ++g_launches;
-    CUDA_TRY(cudaGetLastError());
-  }
+  const int64_t per_slice = (n + slices - 1) / slices;
+  p.per_slice = ((per_slice + tile - 1) / tile) * tile;
+  p.grid = dim3((unsigned)obs_blocks, (unsigned)((n + p.per_slice - 1) / p.per_slice));
   return SPART_OK;
+}
+
+extern "C" {
+
+int spart_lut_nearest(const float* lut_dev, int64_t n, int32_t n_bands, const float* obs_dev, int64_t m,
+                      const float* weights_dev, int64_t index_offset, void* workspace_dev, int64_t* best_index_dev,
+                      float* best_cost_dev, unsigned long long* packed_dev, void* stream) {
+  int rc = check_lut("spart_lut_nearest", 32, lut_dev, n, n_bands, obs_dev, m, index_offset, workspace_dev,
+                     best_index_dev, best_cost_dev, packed_dev);
+  if (rc || m == 0) return rc;
+  NvtxRange r("spart::lut_nearest");
+  cudaStream_t st = (cudaStream_t)stream;
+  LutPlan p;
+  rc = plan_lut(n, m, kLutTile, kLutObs, workspace_dev, packed_dev, st, p);
+  if (rc) return rc;
+  // one instance per group of four bands
+  decltype(&lut_nearest_kernel<1>) const kernels[] = {lut_nearest_kernel<1>, lut_nearest_kernel<2>,
+                                                      lut_nearest_kernel<3>, lut_nearest_kernel<4>,
+                                                      lut_nearest_kernel<5>, lut_nearest_kernel<6>,
+                                                      lut_nearest_kernel<7>, lut_nearest_kernel<8>};
+  rc = launch(kernels[(n_bands + 3) / 4 - 1], p.grid, kLutObs, 0, st, lut_dev, n, n_bands, obs_dev, m, weights_dev,
+              p.per_slice, (unsigned)index_offset, p.best);
+  if (rc || packed_dev) return rc;
+  return launch(lut_unpack_kernel, (unsigned)((m + 255) / 256), 256, 0, st, p.best, m, best_index_dev, best_cost_dev);
 }
 
 int spart_lut_nearest_tc(const float* lut_dev, int64_t n, int32_t n_bands, const float* obs_dev, int64_t m,
                          const float* weights_dev, int64_t index_offset, void* workspace_dev, int64_t* best_index_dev,
                          float* best_cost_dev, unsigned long long* packed_dev, void* stream) {
-  if (!lut_dev || !obs_dev || (!workspace_dev && m > 0))
-    return fail(SPART_EINVAL, "spart_lut_nearest_tc: null argument%s");
-  if (!packed_dev && (!best_index_dev || !best_cost_dev))
-    return fail(SPART_EINVAL, "spart_lut_nearest_tc: need best_index_dev + best_cost_dev or packed_dev%s");
-  if (n <= 0 || n > 0x7fffffffLL || m < 0 || n_bands < 1 || n_bands > 30 || index_offset < 0 ||
-      index_offset + n > 0xffffffffLL)
-    return fail(SPART_EINVAL,
-                "spart_lut_nearest_tc: need 1 <= n < 2^31, m >= 0, 1 <= n_bands <= 30, index_offset + n < 2^32%s");
-  if (m == 0) return SPART_OK;
+  int rc = check_lut("spart_lut_nearest_tc", 30, lut_dev, n, n_bands, obs_dev, m, index_offset, workspace_dev,
+                     best_index_dev, best_cost_dev, packed_dev);
+  if (rc || m == 0) return rc;
   NvtxRange r("spart::lut_nearest_tc");
   cudaStream_t st = (cudaStream_t)stream;
-  unsigned long long* best = packed_dev ? packed_dev : (unsigned long long*)workspace_dev;
-  CUDA_TRY(cudaMemsetAsync(best, 0xff, sizeof(unsigned long long) * m, st));
-  int dev = 0, sms = 148;
-  CUDA_TRY(cudaGetDevice(&dev));
-  CUDA_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   const int ks = (n_bands + 2 + 7) / 8;                 // bands + the two |l|^2 slots, in k-steps of 8
-  const int obs_per_block = kTcWarps * 16 * (ks <= 2 ? 4 : 2);
-  const int64_t obs_blocks = (m + obs_per_block - 1) / obs_per_block;
-  int64_t slices = (8LL * sms + obs_blocks - 1) / obs_blocks;
-  const int64_t max_slices = (n + kTcTile - 1) / kTcTile;
-  if (slices > max_slices) slices = max_slices;
-  if (slices > 65535) slices = 65535;
-  if (slices < 1) slices = 1;
-  int64_t per_slice = (n + slices - 1) / slices;
-  per_slice = ((per_slice + kTcTile - 1) / kTcTile) * kTcTile;
-  slices = (n + per_slice - 1) / per_slice;
-  dim3 grid((unsigned)obs_blocks, (unsigned)slices);
+  LutPlan p;
+  rc = plan_lut(n, m, kTcTile, kTcWarps * 16 * (ks <= 2 ? 4 : 2), workspace_dev, packed_dev, st, p);
+  if (rc) return rc;
   const unsigned off = (unsigned)index_offset;
-  if (ks <= 2)
-    lut_nearest_tc_kernel<2, 4><<<grid, kTcWarps * 32, 0, st>>>(lut_dev, n, n_bands, obs_dev, m, weights_dev, per_slice,
-                                                               off, best);
-  else if (ks == 3)
-    lut_nearest_tc_kernel<3, 2><<<grid, kTcWarps * 32, 0, st>>>(lut_dev, n, n_bands, obs_dev, m, weights_dev, per_slice,
-                                                               off, best);
-  else
-    lut_nearest_tc_kernel<4, 2><<<grid, kTcWarps * 32, 0, st>>>(lut_dev, n, n_bands, obs_dev, m, weights_dev, per_slice,
-                                                               off, best);
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  lut_refine_kernel<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(lut_dev, n_bands, obs_dev, m, weights_dev, off, best);
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  if (!packed_dev) {
-    lut_unpack_kernel<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(best, m, best_index_dev, best_cost_dev);
-    ++g_launches;
-    CUDA_TRY(cudaGetLastError());
-  }
-  return SPART_OK;
+  const auto kernel = ks <= 2 ? lut_nearest_tc_kernel<2, 4> : ks == 3 ? lut_nearest_tc_kernel<3, 2>
+                                                                   : lut_nearest_tc_kernel<4, 2>;
+  rc = launch(kernel, p.grid, kTcWarps * 32, 0, st, lut_dev, n, n_bands, obs_dev, m, weights_dev, p.per_slice, off,
+              p.best);
+  if (rc) return rc;
+  rc = launch(lut_refine_kernel, (unsigned)((m + 255) / 256), 256, 0, st, lut_dev, n_bands, obs_dev, m, weights_dev,
+              off, p.best);
+  if (rc || packed_dev) return rc;
+  return launch(lut_unpack_kernel, (unsigned)((m + 255) / 256), 256, 0, st, p.best, m, best_index_dev, best_cost_dev);
 }
 
 int spart_lut_unpack(const unsigned long long* packed_dev, int64_t m, int64_t* best_index_dev, float* best_cost_dev,
@@ -2429,21 +2385,16 @@ int spart_lut_unpack(const unsigned long long* packed_dev, int64_t m, int64_t* b
   if (!packed_dev || !best_index_dev || !best_cost_dev || m < 0)
     return fail(SPART_EINVAL, "spart_lut_unpack: bad argument%s");
   if (m == 0) return SPART_OK;
-  lut_unpack_kernel<<<(unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream>>>(packed_dev, m, best_index_dev,
-                                                                                   best_cost_dev);
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  return SPART_OK;
+  return launch(lut_unpack_kernel, (unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream, packed_dev, m,
+                best_index_dev, best_cost_dev);
 }
 
 int spart_set_lidf(const double* lidf_dev, int64_t n, void* workspace_dev, void* stream) {
   if (!lidf_dev || (!workspace_dev && n > 0)) return fail(SPART_EINVAL, "spart_set_lidf: null argument%s");
   if (n < 0) return fail(SPART_EINVAL, "spart_set_lidf: n < 0%s");
   if (n == 0) return SPART_OK;
-  lidf_store_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(lidf_dev, n, (double*)workspace_dev);
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  return SPART_OK;
+  return launch(lidf_store_kernel, (unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream, lidf_dev, n,
+                (double*)workspace_dev);
 }
 
 int spart_leafangles(const double* ab_dev, int64_t n, int64_t ld, double* out_dev, void* stream) {
@@ -2457,15 +2408,14 @@ int spart_leafangles(const double* ab_dev, int64_t n, int64_t ld, double* out_de
     if (rc) return rc;
   }
   NvtxRange r("spart::leaf_angles");
-  lidf_kernel<<<(unsigned)((n + kL2Samples - 1) / kL2Samples), kL2Threads, 0, (cudaStream_t)stream>>>(
-      ab_dev, ab_dev + ld, 1, 1, n, out_dev, 1, 13);
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  lidf_diff_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(out_dev, n);
-  ++g_launches;
-  CUDA_TRY(cudaGetLastError());
-  return SPART_OK;
+  cudaStream_t st = (cudaStream_t)stream;
+  const int rc = launch(lidf_kernel, (unsigned)((n + kL2Samples - 1) / kL2Samples), kL2Threads, 0, st, ab_dev,
+                        ab_dev + ld, 1, 1, n, out_dev, 1, 13);
+  if (rc) return rc;
+  return launch(lidf_diff_kernel, (unsigned)((n + 255) / 256), 256, 0, st, out_dev, n);
 }
+
+}  // extern "C"
 
 // ---- host-buffer path ---------------------------------------------------------------------
 static bool is_pinned_host(const void* p) {
@@ -2481,48 +2431,28 @@ static bool is_pinned_host(const void* p) {
 // output slots of `chunk` samples, pinned staging buffers for pageable caller memory
 static int ensure_slots(SpartCtx* ctx, int64_t span, int64_t chunk, size_t out_bytes, bool stage_in, bool stage_out) {
   const size_t in_bytes = sizeof(double) * P_COUNT * (size_t)span;
-  cudaStream_t* streams[4] = {&ctx->h2d_stream, &ctx->d2h_stream, &ctx->compute_stream, &ctx->join_stream};
-  for (cudaStream_t* e : streams) {
-    if (!*e) CUDA_TRY(cudaStreamCreateWithFlags(e, cudaStreamNonBlocking));
-    CUDA_TRY(cudaStreamSynchronize(*e));
+  for (Stream* s : {&ctx->h2d_stream, &ctx->d2h_stream, &ctx->compute_stream, &ctx->join_stream}) {
+    if (!*s) CUDA_TRY(create(*s));
+    CUDA_TRY(cudaStreamSynchronize(s->get()));
   }
+  // a buffer below its capacity field is (re)allocated; the fields are raised once every buffer has grown
   for (int i = 0; i < SpartCtx::kSlots; ++i) {
-    if (!ctx->slot_done[i]) CUDA_TRY(cudaEventCreateWithFlags(&ctx->slot_done[i], cudaEventDisableTiming));
-    if (!ctx->slot_k[i]) CUDA_TRY(cudaEventCreateWithFlags(&ctx->slot_k[i], cudaEventDisableTiming));
-    if (ctx->slot_cap < chunk) {
-      if (ctx->slot_rec[i]) cudaFree(ctx->slot_rec[i]);
-      ctx->slot_rec[i] = nullptr;
-      CUDA_TRY(cudaMalloc(&ctx->slot_rec[i], sizeof(double) * kWsRows * chunk));
-    }
-    if (ctx->slot_out_cap < out_bytes) {
-      if (ctx->slot_out[i]) cudaFree(ctx->slot_out[i]);
-      ctx->slot_out[i] = nullptr;
-      CUDA_TRY(cudaMalloc(&ctx->slot_out[i], out_bytes));
-    }
-    if (stage_out && ctx->stage_out_cap < out_bytes) {
-      if (ctx->stage_out[i]) cudaFreeHost(ctx->stage_out[i]);
-      ctx->stage_out[i] = nullptr;
-      CUDA_TRY(cudaHostAlloc(&ctx->stage_out[i], out_bytes, cudaHostAllocDefault));
-    }
+    if (!ctx->slot_done[i]) CUDA_TRY(create(ctx->slot_done[i], cudaEventDisableTiming));
+    if (!ctx->slot_k[i]) CUDA_TRY(create(ctx->slot_k[i], cudaEventDisableTiming));
+    if (ctx->slot_cap < chunk) CUDA_TRY(alloc(ctx->slot_rec[i], sizeof(double) * kWsRows * chunk));
+    if (ctx->slot_out_cap < out_bytes) CUDA_TRY(alloc(ctx->slot_out[i], out_bytes));
+    if (stage_out && ctx->stage_out_cap < out_bytes) CUDA_TRY(alloc(ctx->stage_out[i], out_bytes));
   }
-  if (!ctx->bc_stage) CUDA_TRY(cudaHostAlloc(&ctx->bc_stage, sizeof(double) * P_COUNT, cudaHostAllocDefault));
+  if (!ctx->bc_stage) CUDA_TRY(alloc(ctx->bc_stage, sizeof(double) * P_COUNT));
   for (int i = 0; i < SpartCtx::kInSlots; ++i) {
-    if (!ctx->in_done[i]) CUDA_TRY(cudaEventCreateWithFlags(&ctx->in_done[i], cudaEventDisableTiming));
-    if (!ctx->in_free[i]) CUDA_TRY(cudaEventCreateWithFlags(&ctx->in_free[i], cudaEventDisableTiming));
-    if (!ctx->ets_done[i]) CUDA_TRY(cudaEventCreateWithFlags(&ctx->ets_done[i], cudaEventDisableTiming));
+    if (!ctx->in_done[i]) CUDA_TRY(create(ctx->in_done[i], cudaEventDisableTiming));
+    if (!ctx->in_free[i]) CUDA_TRY(create(ctx->in_free[i], cudaEventDisableTiming));
+    if (!ctx->ets_done[i]) CUDA_TRY(create(ctx->ets_done[i], cudaEventDisableTiming));
     if (ctx->in_cap < span) {
-      if (ctx->in_params[i]) cudaFree(ctx->in_params[i]);
-      if (ctx->in_ets[i]) cudaFree(ctx->in_ets[i]);
-      ctx->in_params[i] = nullptr;
-      ctx->in_ets[i] = nullptr;
-      CUDA_TRY(cudaMalloc(&ctx->in_params[i], in_bytes));
-      CUDA_TRY(cudaMalloc(&ctx->in_ets[i], sizeof(double) * (size_t)span));
+      CUDA_TRY(alloc(ctx->in_params[i], in_bytes));
+      CUDA_TRY(alloc(ctx->in_ets[i], sizeof(double) * (size_t)span));
     }
-    if (stage_in && ctx->stage_in_cap < in_bytes) {
-      if (ctx->stage_in[i]) cudaFreeHost(ctx->stage_in[i]);
-      ctx->stage_in[i] = nullptr;
-      CUDA_TRY(cudaHostAlloc(&ctx->stage_in[i], in_bytes, cudaHostAllocDefault));
-    }
+    if (stage_in && ctx->stage_in_cap < in_bytes) CUDA_TRY(alloc(ctx->stage_in[i], in_bytes));
   }
   if (ctx->slot_cap < chunk) ctx->slot_cap = chunk;
   if (ctx->in_cap < span) ctx->in_cap = span;
@@ -2535,7 +2465,7 @@ static int ensure_slots(SpartCtx* ctx, int64_t span, int64_t chunk, size_t out_b
     const int hw = (int)std::thread::hardware_concurrency();
     if (hw > 0 && want > hw) want = hw;
     if (want < 1) want = 1;
-    ctx->pool = new (std::nothrow) HostPool(want - 1);
+    ctx->pool.reset(new (std::nothrow) HostPool(want - 1));
     if (!ctx->pool) return fail(SPART_ENOMEM, "spart_forward_bands_host: out of host memory%s");
   }
   return SPART_OK;
@@ -2550,6 +2480,8 @@ static void pool_memcpy(HostPool* pool, void* dst, const void* src, size_t bytes
     memcpy((char*)dst + o, (const char*)src + o, (bytes - o < piece) ? bytes - o : piece);
   });
 }
+
+extern "C" {
 
 int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_host, int64_t n, int64_t ld,
                              uint32_t broadcast_rows, int32_t precision, int32_t flags, void* out_host) {
@@ -2631,24 +2563,24 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
   struct Pending { int64_t s0 = 0, m = 0; bool live = false; } pend[SpartCtx::kSlots];
   // SPART_HOST_TRACE=1 (tuning aid): CUDA events per span and per chunk, printed as a timeline when the call ends
   const bool trace = getenv("SPART_HOST_TRACE") != nullptr;
-  struct TraceEv { cudaEvent_t e[2]; int64_t m; int slot; bool span; };
+  struct TraceEv { Event e[2]; int64_t m; int slot; bool span; };
   std::vector<TraceEv> tev;
-  cudaEvent_t trace_t0 = nullptr;
+  Event trace_t0;
   if (trace) {
-    cudaEventCreate(&trace_t0);
-    cudaEventRecord(trace_t0, ctx->h2d_stream);
+    create(trace_t0);
+    cudaEventRecord(trace_t0.get(), ctx->h2d_stream.get());
   }
   auto trace_new = [&](int64_t m, int slot, bool span) {
     if (!trace) return;
     TraceEv t;
-    for (auto& e : t.e) cudaEventCreate(&e);
+    for (auto& e : t.e) create(e);
     t.m = m;
     t.slot = slot;
     t.span = span;
-    tev.push_back(t);
+    tev.push_back(std::move(t));
   };
   auto mark = [&](int which, cudaStream_t st) {
-    if (trace) cudaEventRecord(tev.back().e[which], st);
+    if (trace) cudaEventRecord(tev.back().e[which].get(), st);
   };
   // wait for a slot's chunk and, with a pageable output, copy it from the pinned staging buffer into the
   // caller's array (the staging buffer may then be reused)
@@ -2656,14 +2588,15 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
     Pending& q = pend[slot];
     if (!q.live) return SPART_OK;
     q.live = false;
-    CUDA_TRY(cudaEventSynchronize(ctx->slot_done[slot]));
+    CUDA_TRY(cudaEventSynchronize(ctx->slot_done[slot].get()));
     const size_t main_bytes = (size_t)q.m * nb * nout * elt;
-    pool_memcpy(ctx->pool, pout + (size_t)q.s0 * nb * nout * elt, ctx->stage_out[slot], main_bytes);
-    if (compact) memcpy(pets + (size_t)q.s0 * elt, (char*)ctx->stage_out[slot] + main_bytes, (size_t)q.m * elt);
+    pool_memcpy(ctx->pool.get(), pout + (size_t)q.s0 * nb * nout * elt, ctx->stage_out[slot].get(), main_bytes);
+    if (compact) memcpy(pets + (size_t)q.s0 * elt, (char*)ctx->stage_out[slot].get() + main_bytes, (size_t)q.m * elt);
     return SPART_OK;
   };
   auto run = [&]() -> int {
-    cudaStream_t sin = ctx->h2d_stream, sout = ctx->d2h_stream, st = ctx->compute_stream, sjoin = ctx->join_stream;
+    cudaStream_t sin = ctx->h2d_stream.get(), sout = ctx->d2h_stream.get();
+    cudaStream_t st = ctx->compute_stream.get(), sjoin = ctx->join_stream.get();
     bool in_used[SpartCtx::kInSlots] = {}, used[SpartCtx::kSlots] = {};
     int slot = 0;
     std::vector<int> fifo;       // pageable output: slots whose chunks are still to be copied out, oldest first
@@ -2673,7 +2606,8 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
     const int64_t dld = ctx->in_cap;
     if (broadcast_rows) {
       for (int r = 0; r < P_COUNT; ++r)
-        if ((broadcast_rows >> r) & 1u) memcpy((char*)ctx->bc_stage + (size_t)r * elt, pin + (size_t)r * ld * elt, elt);
+        if ((broadcast_rows >> r) & 1u)
+          memcpy((char*)ctx->bc_stage.get() + (size_t)r * elt, pin + (size_t)r * ld * elt, elt);
       for (int i = 0; i < SpartCtx::kInSlots && i < (int)spans.size(); ++i)
         for (int r0 = 0; r0 < P_COUNT;) {
           if (!((broadcast_rows >> r0) & 1u)) {
@@ -2682,8 +2616,8 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
           }
           int r1 = r0 + 1;
           while (r1 < P_COUNT && ((broadcast_rows >> r1) & 1u)) ++r1;
-          CUDA_TRY(cudaMemcpy2DAsync((char*)ctx->in_params[i] + (size_t)r0 * dld * elt, (size_t)dld * elt,
-                                     (char*)ctx->bc_stage + (size_t)r0 * elt, elt, elt, r1 - r0,
+          CUDA_TRY(cudaMemcpy2DAsync((char*)ctx->in_params[i].get() + (size_t)r0 * dld * elt, (size_t)dld * elt,
+                                     (char*)ctx->bc_stage.get() + (size_t)r0 * elt, elt, elt, r1 - r0,
                                      cudaMemcpyHostToDevice, sin));
           r0 = r1;
         }
@@ -2699,8 +2633,9 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
       size_t src_pitch = (size_t)ld * elt;
       size_t src_off = (size_t)sp0 * elt;
       if (stage_in) {
-        if (in_used[islot]) CUDA_TRY(cudaEventSynchronize(ctx->in_done[islot]));   // the staging buffer has been read
-        char* stg = (char*)ctx->stage_in[islot];
+        // the staging buffer has been read
+        if (in_used[islot]) CUDA_TRY(cudaEventSynchronize(ctx->in_done[islot].get()));
+        char* stg = (char*)ctx->stage_in[islot].get();
         ctx->pool->parallel_for(P_COUNT, [&](int r) {
           if (!((broadcast_rows >> r) & 1u))
             memcpy(stg + (size_t)r * sm * elt, pin + (size_t)r * ld * elt + (size_t)sp0 * elt, (size_t)sm * elt);
@@ -2709,7 +2644,7 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
         src_pitch = (size_t)sm * elt;
         src_off = 0;
       }
-      if (in_used[islot]) CUDA_TRY(cudaStreamWaitEvent(sin, ctx->in_free[islot], 0));
+      if (in_used[islot]) CUDA_TRY(cudaStreamWaitEvent(sin, ctx->in_free[islot].get(), 0));
       trace_new(sm, islot, true);
       mark(0, sin);
       for (int r0 = 0; r0 < P_COUNT;) {     // runs of per-sample rows become one 2-D copy each
@@ -2719,12 +2654,12 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
         }
         int r1 = r0 + 1;
         while (r1 < P_COUNT && !((broadcast_rows >> r1) & 1u)) ++r1;
-        CUDA_TRY(cudaMemcpy2DAsync((char*)ctx->in_params[islot] + (size_t)r0 * dld * elt, (size_t)dld * elt,
+        CUDA_TRY(cudaMemcpy2DAsync((char*)ctx->in_params[islot].get() + (size_t)r0 * dld * elt, (size_t)dld * elt,
                                    src + (size_t)r0 * src_pitch + src_off, src_pitch, (size_t)sm * elt, r1 - r0,
                                    cudaMemcpyHostToDevice, sin));
         r0 = r1;
       }
-      CUDA_TRY(cudaEventRecord(ctx->in_done[islot], sin));
+      CUDA_TRY(cudaEventRecord(ctx->in_done[islot].get(), sin));
       mark(1, sin);
       in_used[islot] = true;
       // ---- the span's chunks: kernels in place, device -> host
@@ -2741,30 +2676,31 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
         int rc2 = unstage(slot);      // pageable output: the slot's previous chunk leaves its staging buffer
         if (rc2) return rc2;
         trace_new(m, slot, false);
-        CUDA_TRY(cudaStreamWaitEvent(st, ctx->in_done[islot], 0));
-        if (used[slot]) CUDA_TRY(cudaStreamWaitEvent(st, ctx->slot_done[slot], 0));
+        CUDA_TRY(cudaStreamWaitEvent(st, ctx->in_done[islot].get(), 0));
+        if (used[slot]) CUDA_TRY(cudaStreamWaitEvent(st, ctx->slot_done[slot].get(), 0));
         if (ets_per_span && ci == 0 && j >= (size_t)SpartCtx::kInSlots)
-          CUDA_TRY(cudaStreamWaitEvent(st, ctx->ets_done[islot], 0));     // the span buffer's etscale array is free
-        rc2 = forward_bands_impl(ctx, sensor, (const char*)ctx->in_params[islot] + (size_t)off * elt,
-                                 ctx->in_params[islot], m, dld, broadcast_rows, precision, flags, ctx->slot_rec[slot],
-                                 ctx->slot_out[slot], st);
+          CUDA_TRY(cudaStreamWaitEvent(st, ctx->ets_done[islot].get(), 0));   // the span buffer's etscale array is free
+        rc2 = forward_bands_impl(ctx, sensor, (const char*)ctx->in_params[islot].get() + (size_t)off * elt,
+                                 ctx->in_params[islot].get(), m, dld, broadcast_rows, precision, flags,
+                                 ctx->slot_rec[slot].get(), ctx->slot_out[slot].get(), st);
         if (rc2) return rc2;
         const size_t main_bytes = (size_t)m * nb * nout * elt;
         if (ets_per_span)
-          CUDA_TRY(cudaMemcpyAsync((char*)ctx->in_ets[islot] + (size_t)off * elt, (char*)ctx->slot_out[slot] + main_bytes,
-                                   (size_t)m * elt, cudaMemcpyDeviceToDevice, st));
-        CUDA_TRY(cudaEventRecord(ctx->slot_k[slot], st));
+          CUDA_TRY(cudaMemcpyAsync((char*)ctx->in_ets[islot].get() + (size_t)off * elt,
+                                   (char*)ctx->slot_out[slot].get() + main_bytes, (size_t)m * elt,
+                                   cudaMemcpyDeviceToDevice, st));
+        CUDA_TRY(cudaEventRecord(ctx->slot_k[slot].get(), st));
         mark(0, st);
-        CUDA_TRY(cudaStreamWaitEvent(sjoin, ctx->slot_k[slot], 0));
-        CUDA_TRY(cudaStreamWaitEvent(sout, ctx->slot_k[slot], 0));
+        CUDA_TRY(cudaStreamWaitEvent(sjoin, ctx->slot_k[slot].get(), 0));
+        CUDA_TRY(cudaStreamWaitEvent(sout, ctx->slot_k[slot].get(), 0));
         if (stage_out) {
-          CUDA_TRY(cudaMemcpyAsync(ctx->stage_out[slot], ctx->slot_out[slot], main_bytes + (compact ? m * elt : 0),
-                                   cudaMemcpyDeviceToHost, sout));
+          CUDA_TRY(cudaMemcpyAsync(ctx->stage_out[slot].get(), ctx->slot_out[slot].get(),
+                                   main_bytes + (compact ? m * elt : 0), cudaMemcpyDeviceToHost, sout));
         } else {
-          CUDA_TRY(cudaMemcpyAsync(pout + (size_t)s0 * nb * nout * elt, ctx->slot_out[slot], main_bytes,
+          CUDA_TRY(cudaMemcpyAsync(pout + (size_t)s0 * nb * nout * elt, ctx->slot_out[slot].get(), main_bytes,
                                    cudaMemcpyDeviceToHost, sout));
         }
-        CUDA_TRY(cudaEventRecord(ctx->slot_done[slot], sout));
+        CUDA_TRY(cudaEventRecord(ctx->slot_done[slot].get(), sout));
         mark(1, sout);
         used[slot] = true;
         if (stage_out) {
@@ -2781,11 +2717,11 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
           }
         }
       }
-      CUDA_TRY(cudaEventRecord(ctx->in_free[islot], sjoin));    // every chunk of this span has been evaluated
+      CUDA_TRY(cudaEventRecord(ctx->in_free[islot].get(), sjoin));    // every chunk of this span has been evaluated
       if (ets_per_span) {          // (the d2h stream has already waited for the kernels of all chunks of the span)
-        CUDA_TRY(cudaMemcpyAsync(pets + (size_t)sp0 * elt, ctx->in_ets[islot], (size_t)sm * elt, cudaMemcpyDeviceToHost,
-                                 sout));
-        CUDA_TRY(cudaEventRecord(ctx->ets_done[islot], sout));
+        CUDA_TRY(cudaMemcpyAsync(pets + (size_t)sp0 * elt, ctx->in_ets[islot].get(), (size_t)sm * elt,
+                                 cudaMemcpyDeviceToHost, sout));
+        CUDA_TRY(cudaEventRecord(ctx->ets_done[islot].get(), sout));
       }
     }
     for (int i = 0; i < SpartCtx::kSlots; ++i) {
@@ -2797,29 +2733,24 @@ int spart_forward_bands_host(SpartCtx* ctx, int32_t sensor, const void* params_h
   rc = run();
   // on success and on failure alike: nothing of this call may still be in flight (the copy streams read and
   // write the caller's memory) when it returns
-  char keep[sizeof(g_err)];
-  memcpy(keep, g_err, sizeof(keep));
-  for (cudaStream_t sy : {ctx->compute_stream, ctx->h2d_stream, ctx->d2h_stream, ctx->join_stream}) {
-    const cudaError_t e = cudaStreamSynchronize(sy);
+  for (const Stream* sy : {&ctx->compute_stream, &ctx->h2d_stream, &ctx->d2h_stream, &ctx->join_stream}) {
+    const cudaError_t e = cudaStreamSynchronize(sy->get());
     if (e != cudaSuccess && rc == SPART_OK) {
-      snprintf(keep, sizeof(keep), "cudaStreamSynchronize failed: %s", cudaGetErrorString(e));
+      snprintf(g_err, sizeof(g_err), "cudaStreamSynchronize failed: %s", cudaGetErrorString(e));
       rc = (int)e;
     }
   }
-  if (rc) memcpy(g_err, keep, sizeof(keep));
   if (trace) {
     fprintf(stderr, "spart_forward_bands_host trace [ms from the first enqueue]\n"
                     "  span  <samples> <buffer> | H2D start .. end\n  chunk <samples> <slot>   | kernels end | D2H end\n");
     for (size_t i = 0; i < tev.size(); ++i) {
       float t[2] = {0, 0};
-      for (int k = 0; k < 2; ++k) cudaEventElapsedTime(&t[k], trace_t0, tev[i].e[k]);
+      for (int k = 0; k < 2; ++k) cudaEventElapsedTime(&t[k], trace_t0.get(), tev[i].e[k].get());
       if (tev[i].span)
         fprintf(stderr, "  span  %7lld %d | %7.3f .. %7.3f\n", (long long)tev[i].m, tev[i].slot, t[0], t[1]);
       else
         fprintf(stderr, "  chunk %7lld %d |            %7.3f | %7.3f\n", (long long)tev[i].m, tev[i].slot, t[0], t[1]);
-      for (auto& e : tev[i].e) cudaEventDestroy(e);
     }
-    cudaEventDestroy(trace_t0);
   }
   return rc;
 }
@@ -2845,7 +2776,10 @@ int spart_measure_fp64_chain(int32_t device, double* tflops) {
   GUARD_DEVICE(device);
   int sm = 0;
   CUDA_TRY(cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, device));
-  return time_register_chain(sm, tflops);
+  const int iters = 1 << 12, threads = 1024, blocks = sm;     // 8 warps per scheduler
+  return time_peak(2.0 * 6.0 * 4.0 * (double)iters * threads * (double)blocks, tflops, [&](double* d) {
+    return launch(fp64_register_chain_kernel, blocks, threads, 0, nullptr, d, iters);
+  });
 }
 
 }  // extern "C"

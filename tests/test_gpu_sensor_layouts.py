@@ -119,13 +119,21 @@ def test_srf_slot_limit(env, nb, slots):
 
 
 def test_srf_too_many_slots(env):
-    """25 slots: spart_create refuses the sensor."""
-    _, sb = env
+    """25 slots: spart_create refuses the sensor, and releases what it had already allocated (the refusal
+    comes from the SRF planner, after the wavelength, band and knot tables are on the device)."""
+    torch, sb = env
     centres, wl, p = gaussian_srfs(24)
     info = sensorinfo(centres, wl, p)
     assert srf_slots(sb, info) == 25
+    eng = sb.default_engine()
     with pytest.raises(sb.SpartError, match="too many overlapping bands"):
-        sb.default_engine().sensor(info)
+        eng.sensor(info)
+    free0 = torch.cuda.mem_get_info(eng.device)[0]
+    for _ in range(200):
+        with pytest.raises(sb.SpartError, match="too many overlapping bands"):
+            eng.sensor(info)
+    # a leak would keep at least the 272 KB wavelength table per refusal, about 54 MB in all
+    assert abs(torch.cuda.mem_get_info(eng.device)[0] - free0) <= 2 << 20
 
 
 def test_srf_single_wavelength_ends_and_zero_weight(env):
