@@ -285,6 +285,45 @@ int spart_lut_nearest_tc(const float* lut_dev, int64_t n, int32_t n_bands, const
 int spart_lut_unpack(const unsigned long long* packed_dev, int64_t m, int64_t* best_index_dev,
                      float* best_cost_dev, void* stream);
 
+/* The k nearest LUT entries of each observation (1 <= k <= 128, n_bands <= 32), with the cost of
+ * spart_lut_nearest bit for bit (so k = 1 returns its index and cost).  Per observation the k smallest words
+ * (cost bits << 32 | index_offset + local index) in unsigned order, i.e. ascending cost, ties to the lowest index
+ * (also at the k-th place), whatever the launch plan.  Entries whose cost is NaN or not below 3e38 are never chosen;
+ * slots beyond the qualifying entries hold the "no entry" word (all ones: index 2^32 - 1, cost NaN), which sorts
+ * last.  Outputs best_index_dev int64 [m][k] and best_cost_dev float [m][k]; with packed_dev != NULL the call
+ * instead leaves the sorted words in packed_dev [m][k], for spart_lut_topk_merge with the lists of other GPUs.
+ * workspace_dev: spart_lut_topk_workspace_bytes(n, m, k) bytes (depends on its arguments only).  Other arguments
+ * and limits as in spart_lut_nearest. */
+size_t spart_lut_topk_workspace_bytes(int64_t n, int64_t m, int32_t k);
+int spart_lut_topk(const float* lut_dev, int64_t n, int32_t n_bands, const float* obs_dev, int64_t m, int32_t k,
+                   const float* weights_dev, int64_t index_offset, void* workspace_dev, int64_t* best_index_dev,
+                   float* best_cost_dev, unsigned long long* packed_dev, void* stream);
+/* n_lists ascending lists of k words per observation, lists_dev [n_lists][m][k] (e.g. the packed_dev results of
+ * several GPUs, gathered), reduced to the k smallest words, ascending: best_index_dev [m][k] + best_cost_dev [m][k],
+ * or (packed_dev != NULL) the words in packed_dev [m][k].  1 <= n_lists <= 4096. */
+int spart_lut_topk_merge(const unsigned long long* lists_dev, int64_t n_lists, int64_t m, int32_t k,
+                         int64_t* best_index_dev, float* best_cost_dev, unsigned long long* packed_dev,
+                         void* stream);
+
+/* Moments of the parameters of the chosen entries, over a parameter table that may be sharded: a call sees the
+ * entries [index_offset, index_offset + n_local) (index_offset + n_local < 2^32).  Parameter p of local entry e is
+ * params_dev[p * stride_param + e * stride_entry] (elements; double, or float with SPART_FLAG_F32_IO), so both the
+ * [n_params][n] batch layout and an [n][n_params] table are read without a copy.  For each observation o and each
+ * of its k neighbours index_dev [m][k] (int64, e.g. spart_lut_topk's best_index_dev) that falls in the local range,
+ * in neighbour order, in FP64, added to acc_dev [m][n_params + 1] (zero it first):
+ *   centre_dev == NULL: acc[o][p] += x, and acc[o][n_params] += 1 (the count);
+ *   centre_dev [m][n_params]: acc[o][p] += (x - centre[o][p])^2, and the count as above.
+ * Pieces of a table accumulate into one acc_dev (on several GPUs: one sum all-reduce of acc_dev per pass).
+ * spart_lut_moments_finish: mean [m][n_params] = sum / count, count_dev int64 [m]; with sq_dev (the acc_dev of a
+ * second pass centred on that mean) also std_dev [m][n_params] = sqrt(sq / count), the population standard
+ * deviation.  count 0 gives NaN mean and std. */
+int spart_lut_moments_accumulate(const void* params_dev, int32_t n_params, int64_t stride_param,
+                                 int64_t stride_entry, int32_t flags, int64_t index_offset, int64_t n_local,
+                                 const int64_t* index_dev, int64_t m, int32_t k, const double* centre_dev,
+                                 double* acc_dev, void* stream);
+int spart_lut_moments_finish(const double* sum_dev, const double* sq_dev, int64_t m, int32_t n_params,
+                             double* mean_dev, double* std_dev, int64_t* count_dev, void* stream);
+
 /* Per-kernel timing of spart_forward_bands with CUDA events recorded on the caller's stream
  * (used by bench.py for the roofline).  After spart_profile_enable(ctx, 1) every
  * spart_forward_bands call records events around its SPART_NKERNELS kernels; spart_profile_read

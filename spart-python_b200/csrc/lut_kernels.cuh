@@ -82,6 +82,218 @@ __global__ void lut_unpack_kernel(const unsigned long long* __restrict__ best, i
   cost[i] = __uint_as_float((unsigned)(p >> 32));
 }
 
+// ---- k nearest entries ----------------------------------------------------------------------------------------
+// lut_topk_kernel: the search of lut_nearest_kernel (same FP32 cost: weighting, padding, c0 / c1 interleaving and
+// fmaf order, so k = 1 gives its index and cost bit for bit), keeping the k smallest words (cost bits << 32 | global
+// index) per observation instead of one.  Costs are >= 0, so unsigned word order is (cost, index) order.
+//   heap   = each thread's k words as a max-heap in a column of dynamic shared memory ([k][blockDim.x], conflict-free);
+//            the root is the k-th best so far and starts as the all-ones "no entry" word
+//   filter = an entry enters only if its cost is below the root's (below 3e38 while a "no entry" word is the root):
+//            a slice is walked in ascending index order, so an equal cost loses to the root's lower index and the
+//            compare is the word order.  After the first k entries the inner loop is the nearest kernel's loop;
+//            the heap is entered ~k ln(n_slice / k) times per observation and slice (replace root, sift down);
+//            4 entries per unrolled step keep enough independent cost chains in flight at the lower occupancy the
+//            heaps leave (measured +2..9 % at k = 16..50 over 2)
+//   result = each list heap-sorted ascending and written to lists [slice][m][k]; lut_topk_merge_kernel reduces them
+constexpr int kLutTopkMax = 128;
+
+// replace the root of the max-heap h[0..size) (element i at h[i * stride]) by w and restore the heap order
+__device__ __forceinline__ void topk_sift_down(unsigned long long* h, int stride, int size, unsigned long long w) {
+  int i = 0;
+  for (int c = 1; c < size; c = 2 * i + 1) {
+    unsigned long long cv = h[c * stride];
+    if (c + 1 < size) {
+      const unsigned long long r = h[(c + 1) * stride];
+      if (r > cv) {
+        cv = r;
+        ++c;
+      }
+    }
+    if (cv <= w) break;
+    h[i * stride] = cv;
+    i = c;
+  }
+  h[i * stride] = w;
+}
+
+template <int NB4>   // bands padded to 4 * NB4
+__global__ void __launch_bounds__(kLutObs)
+lut_topk_kernel(const float* __restrict__ lut, int64_t n, int nb, const float* __restrict__ obs, int64_t m,
+                const float* __restrict__ sqrt_w, int64_t per_slice, unsigned index_offset, int k,
+                unsigned long long* __restrict__ lists) {
+  constexpr int NBP = 4 * NB4;
+  __shared__ __align__(16) float s_l[kLutTile][NBP];
+  __shared__ float s_w[NBP];
+  extern __shared__ unsigned long long s_heap[];
+  const int nt = blockDim.x;
+  unsigned long long* h = s_heap + threadIdx.x;
+  for (int j = 0; j < k; ++j) h[j * nt] = ~0ull;
+  for (int b = threadIdx.x; b < NBP; b += blockDim.x) s_w[b] = (b < nb) ? (sqrt_w ? sqrt_w[b] : 1.0f) : 0.0f;
+  __syncthreads();
+  const int64_t oi = (int64_t)blockIdx.x * nt + threadIdx.x;
+  const int64_t oc = oi < m ? oi : m - 1;
+  float o[NBP];
+#pragma unroll
+  for (int b = 0; b < NBP; ++b) o[b] = (b < nb) ? obs[oc * nb + b] * s_w[b] : 0.0f;
+  const int64_t e0 = (int64_t)blockIdx.y * per_slice;
+  const int64_t e1 = (e0 + per_slice < n) ? e0 + per_slice : n;
+  float thr = 3.0e38f;
+  for (int64_t t0 = e0; t0 < e1; t0 += kLutTile) {
+    const int cnt = (int)((e1 - t0 < kLutTile) ? (e1 - t0) : kLutTile);
+    __syncthreads();
+    for (int i = threadIdx.x; i < cnt * NBP; i += blockDim.x) {
+      const int e = i / NBP, b = i % NBP;
+      s_l[e][b] = (b < nb) ? lut[(t0 + e) * nb + b] * s_w[b] : 0.0f;
+    }
+    __syncthreads();
+#pragma unroll 4
+    for (int e = 0; e < cnt; ++e) {
+      const float4* row = reinterpret_cast<const float4*>(s_l[e]);
+      float c0 = 0.0f, c1 = 0.0f;
+#pragma unroll
+      for (int q = 0; q < NB4; ++q) {
+        const float4 l = row[q];
+        const float d0 = o[4 * q] - l.x, d1 = o[4 * q + 1] - l.y, d2 = o[4 * q + 2] - l.z, d3 = o[4 * q + 3] - l.w;
+        c0 = fmaf(d0, d0, c0);
+        c1 = fmaf(d1, d1, c1);
+        c0 = fmaf(d2, d2, c0);
+        c1 = fmaf(d3, d3, c1);
+      }
+      const float c = c0 + c1;
+      if (c < thr) {
+        topk_sift_down(h, nt, k, ((unsigned long long)__float_as_uint(c) << 32) | ((unsigned)(t0 + e) + index_offset));
+        thr = fminf(__uint_as_float((unsigned)(h[0] >> 32)), 3.0e38f);   // a "no entry" root has cost bits NaN
+      }
+    }
+  }
+  for (int end = k - 1; end > 0; --end) {   // heap sort: ascending words
+    const unsigned long long top = h[0];
+    topk_sift_down(h, nt, end, h[end * nt]);
+    h[end * nt] = top;
+  }
+  if (oi < m) {
+    unsigned long long* out = lists + ((int64_t)blockIdx.y * m + oi) * k;
+    for (int j = 0; j < k; ++j) out[j] = h[j * nt];
+  }
+}
+
+// L ascending lists of k words per observation (lists [L][m][k]) -> the k smallest words, ascending.  One warp per
+// observation: each lane owns lists lane, lane + 32, ... and keeps the smallest of their heads; per output slot a
+// warp min picks the winner, whose owner (the lowest such lane) advances that list and re-scans its heads.  Heads
+// and cursors live in dynamic shared memory: [warps][L] words, then [warps][L] bytes.  Once the winner is the
+// "no entry" word every list is exhausted and the remaining slots are filled with it.  Writes each output that is
+// not NULL: idx / cost (unpacked as lut_unpack_kernel does) and packed.
+__global__ void lut_topk_merge_kernel(const unsigned long long* __restrict__ lists, int L, int64_t m, int k,
+                                      int64_t* __restrict__ idx, float* __restrict__ cost,
+                                      unsigned long long* __restrict__ packed) {
+  extern __shared__ unsigned long long s_merge[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = blockDim.x >> 5;
+  const int64_t o = (int64_t)blockIdx.x * warps + warp;
+  if (o >= m) return;                                  // whole warps leave together
+  unsigned long long* head = s_merge + (int64_t)warp * L;
+  unsigned char* cur = reinterpret_cast<unsigned char*>(s_merge + (int64_t)warps * L) + (int64_t)warp * L;
+  const unsigned long long* base = lists + o * k;
+  const int64_t lstride = m * k;
+  unsigned long long mine = ~0ull;
+  int mine_l = 0;
+  for (int l = lane; l < L; l += 32) {
+    const unsigned long long v = base[l * lstride];
+    head[l] = v;
+    cur[l] = 0;
+    if (v < mine) {
+      mine = v;
+      mine_l = l;
+    }
+  }
+  const int64_t out0 = o * k;
+  for (int r = 0; r < k; ++r) {
+    unsigned long long w = mine;
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) {
+      const unsigned long long x = __shfl_xor_sync(0xffffffffu, w, d);
+      w = x < w ? x : w;
+    }
+    if (w == ~0ull) {                                  // warp-uniform
+      for (int j = r + lane; j < k; j += 32) {
+        if (idx) idx[out0 + j] = 0xffffffffLL;
+        if (cost) cost[out0 + j] = __uint_as_float(0xffffffffu);
+        if (packed) packed[out0 + j] = ~0ull;
+      }
+      return;
+    }
+    if (lane == 0) {
+      if (idx) idx[out0 + r] = (int64_t)(w & 0xffffffffu);
+      if (cost) cost[out0 + r] = __uint_as_float((unsigned)(w >> 32));
+      if (packed) packed[out0 + r] = w;
+    }
+    const unsigned own = __ballot_sync(0xffffffffu, mine == w);
+    if (lane == __ffs(own) - 1) {
+      const int c = ++cur[mine_l];
+      head[mine_l] = c < k ? base[mine_l * lstride + c] : ~0ull;
+      mine = ~0ull;
+      for (int l = lane; l < L; l += 32) {
+        const unsigned long long v = head[l];
+        if (v < mine) {
+          mine = v;
+          mine_l = l;
+        }
+      }
+    }
+    __syncwarp();
+  }
+}
+
+// ---- moments of the parameters of the chosen entries ---------------------------------------------------------
+// Thread = (observation o, column p of acc [m][P + 1]).  Over the neighbours j of o in index order, those whose index
+// lies in this table piece [index_offset, index_offset + n_local) add x = params[p * stride_param + e * stride_entry]
+// (e = local index) -- or (x - centre[o][p])^2 with a centre -- in FP64; column P adds 1 per such neighbour (the
+// count).  The sum is added to acc, so pieces of a sharded table accumulate into one buffer.
+template <typename T>
+__global__ void lut_moments_kernel(const T* __restrict__ params, int P, int64_t stride_param, int64_t stride_entry,
+                                   int64_t index_offset, int64_t n_local, const int64_t* __restrict__ index,
+                                   int64_t m, int k, const double* __restrict__ centre, double* __restrict__ acc) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= m * (P + 1)) return;
+  const int64_t o = t / (P + 1);
+  const int p = (int)(t - o * (P + 1));
+  const double c = (centre && p < P) ? centre[o * P + p] : 0.0;
+  double s = 0.0;
+  for (int j = 0; j < k; ++j) {
+    const int64_t e = index[o * k + j] - index_offset;
+    if (e < 0 || e >= n_local) continue;
+    if (p == P) {
+      s += 1.0;
+    } else {
+      const double x = (double)params[p * stride_param + e * stride_entry];
+      if (centre) {
+        const double d = x - c;
+        s += d * d;
+      } else {
+        s += x;
+      }
+    }
+  }
+  acc[t] += s;
+}
+
+// mean = sum / count, std = sqrt(sum of squared deviations / count) (population); count 0 gives NaN for both.
+// Without sq only mean and count are written.
+__global__ void lut_moments_finish_kernel(const double* __restrict__ sum, const double* __restrict__ sq, int64_t m,
+                                          int P, double* __restrict__ mean, double* __restrict__ sd,
+                                          int64_t* __restrict__ count) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= m * (P + 1)) return;
+  const int64_t o = t / (P + 1);
+  const int p = (int)(t - o * (P + 1));
+  const double cnt = sum[o * (P + 1) + P];
+  if (p == P) {
+    count[o] = (int64_t)cnt;
+    return;
+  }
+  mean[o * P + p] = sum[t] / cnt;
+  if (sq) sd[o * P + p] = sqrt(sq[t] / cnt);
+}
+
 }  // namespace spart
 
 // ---- tensor-core variant ------------------------------------------------------------------------

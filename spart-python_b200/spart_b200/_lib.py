@@ -34,6 +34,8 @@ EXPORTS = (
     "spart_destroy",
     "spart_workspace_bytes", "spart_forward_bands", "spart_forward_bands_bc", "spart_forward_bands_host", "spart_forward_spectrum",
     "spart_smac", "spart_sailh", "spart_lut_workspace_bytes", "spart_lut_nearest", "spart_lut_nearest_tc", "spart_lut_unpack",
+    "spart_lut_topk_workspace_bytes", "spart_lut_topk", "spart_lut_topk_merge", "spart_lut_moments_accumulate",
+    "spart_lut_moments_finish",
     "spart_leafangles", "spart_set_lidf", "spart_profile_enable", "spart_profile_read", "spart_measure_peaks", "spart_measure_fp64_chain", "spart_launch_count",
 )
 
@@ -99,6 +101,15 @@ def load():
                                       c_void_p, c_void_p, c_void_p, c_void_p]
     lib.spart_lut_nearest_tc.argtypes = lib.spart_lut_nearest.argtypes
     lib.spart_lut_unpack.argtypes = [c_void_p, c_int64, c_void_p, c_void_p, c_void_p]
+    lib.spart_lut_topk_workspace_bytes.argtypes = [c_int64, c_int64, c_int32]
+    lib.spart_lut_topk_workspace_bytes.restype = c_size_t
+    lib.spart_lut_topk.argtypes = [c_void_p, c_int64, c_int32, c_void_p, c_int64, c_int32, c_void_p, c_int64, c_void_p,
+                                   c_void_p, c_void_p, c_void_p, c_void_p]
+    lib.spart_lut_topk_merge.argtypes = [c_void_p, c_int64, c_int64, c_int32, c_void_p, c_void_p, c_void_p, c_void_p]
+    lib.spart_lut_moments_accumulate.argtypes = [c_void_p, c_int32, c_int64, c_int64, c_int32, c_int64, c_int64,
+                                                 c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p]
+    lib.spart_lut_moments_finish.argtypes = [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p,
+                                             c_void_p]
     lib.spart_leafangles.argtypes = [c_void_p, c_int64, c_int64, c_void_p, c_void_p]
     lib.spart_set_lidf.argtypes = [c_void_p, c_int64, c_void_p, c_void_p]
     lib.spart_profile_enable.argtypes = [c_void_p, c_int32]
