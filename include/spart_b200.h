@@ -324,6 +324,55 @@ int spart_lut_moments_accumulate(const void* params_dev, int32_t n_params, int64
 int spart_lut_moments_finish(const double* sum_dev, const double* sq_dev, int64_t m, int32_t n_params,
                              double* mean_dev, double* std_dev, int64_t* count_dev, void* stream);
 
+/* Variance-based sensitivity analysis (new; the reference has none): a scrambled Sobol' design in the batch layout
+ * and the Saltelli (2010) estimators of the first-order and total Sobol' indices.  No context is needed; the
+ * calls run on the current device.
+ *
+ * spart_sobol_design writes rows rows[0..n_vary-1] (distinct, 0..26) of params_dev [SPART_NPAR][ld]; the other
+ * rows are the caller's.  rows, lo and hi are HOST arrays of n_vary entries; 1 <= n_vary <= 27.
+ *   Point i (0 <= first <= i < first + count <= 2^32) of dimension d is k_d(i) = XOR of v'[d][j] over the set
+ *   bits j of i ^ (i >> 1), XOR s_d, and u = k_d(i) 2^-32; v are the Joe-Kuo direction numbers that SciPy ships
+ *   (sobol_dirs.h).  Varied parameter p gets x = lo[p] + (hi[p] - lo[p]) u, rounded once per operation (no fused
+ *   multiply-add), and moved to the double below hi[p] if it rounds up to it, so x is in [lo[p], hi[p]).
+ *   scramble = 0: v' = v, s = 0, which is scipy.stats.qmc.Sobol(D, scramble=False, bits=32) bit for bit.
+ *   scramble = 1: v'[d][j] = L_d v[d][j] over GF(2) and a random digital shift s_d.  L_d is unit lower-triangular
+ *   (rows counted from the most significant bit); with the SplitMix64 stream of `seed`, dimension d draws the
+ *   words 32 d .. 32 d + 31: the strictly-lower part of row r = 1..31 is the low r bits of word 32 d + r - 1
+ *   (its bit r - 1 - c is column c), and s_d is the low 32 bits of word 32 d + 31.  Dimension d thus gets the
+ *   same scramble whatever the number of dimensions, and the net property of the points is kept.
+ *   saltelli = 0: `count` samples 0..count-1 of dimensions 0..n_vary-1 (ld >= count), e.g. a quasi-random LUT.
+ *   saltelli = 1: (n_vary + 2) count samples in blocks A, B, AB_1 .. AB_n_vary (sample block * count + j,
+ *   ld >= (n_vary + 2) count): A uses dimensions 0..n_vary-1, B dimensions n_vary..2 n_vary-1, and AB_i is A
+ *   with varied parameter i taken from B.  The A block equals the saltelli = 0 output.
+ *
+ * spart_sobol_accumulate adds the sums of one chunk of n base points to acc_dev (spart_sobol_acc_elems(n_out,
+ * n_vary) doubles; zero it before the first chunk).  f_dev [(n_vary + 2) n][n_out]: the outputs of the chunk's
+ * design blocks, f[(block n + j) n_out + o] -- spart_forward_bands' [samples][nb][3] over the blocks A, B, AB_i
+ * of the chunk, with n_out = 3 nb.  ref_dev [(n_vary + 2)][n_out]: the outputs of base point 0 of the whole
+ * design (A, B, AB_1 .. AB_n_vary), by which every summed quantity is shifted, so an output whose mean is far
+ * above its spread keeps its variance.  acc_dev [128][n_vary + 1][n_out][8]: per slice of the chunk's base
+ * points, for varied parameter i < n_vary, with D = f_ABi - f_A, p = (f_B - f_A0) D and u = D^2 (f_A0 = ref's
+ * f_A), the sums of (p - p_0), (p - p_0)^2, (D - D_0), (D - D_0)^2, (p - p_0)(D - D_0), (u - u_0), (u - u_0)^2
+ * and a zero (x_0: x at base point 0); slot n_vary: the sums of (f - f_A0) and (f - f_A0)^2 over f_A and f_B,
+ * then zeros.  All sums are FP64 in a fixed order, so a run is bit-reproducible; the accumulators of design
+ * pieces on several GPUs (each with the same ref) merge with one sum all-reduce.
+ *
+ * spart_sobol_finish, over n_total base points, with the estimators of scipy.stats.sobol_indices (method
+ * "saltelli_2010", outputs centred on their mean): mean_dev, var_dev [n_out]: mean and population variance V of
+ * f_A and f_B together; first_dev, total_dev [n_out][n_vary]: S_i = mean(t) / V with t = (f_B - mean) D, and
+ * ST_i = mean(u) / (2 V); first_se_dev, total_se_dev: std(t) / (sqrt(N) V) and std(u) / (2 sqrt(N) V),
+ * population standard deviations, which ignore the uncertainty of V (and of the mean).  V = 0 gives NaN
+ * indices. */
+int spart_sobol_design(const int32_t* rows, const double* lo, const double* hi, int32_t n_vary, uint64_t seed,
+                       int32_t scramble, int64_t first, int64_t count, int32_t saltelli, double* params_dev,
+                       int64_t ld, void* stream);
+size_t spart_sobol_acc_elems(int32_t n_out, int32_t n_vary);
+int spart_sobol_accumulate(const double* f_dev, int64_t n, int32_t n_out, int32_t n_vary, const double* ref_dev,
+                           double* acc_dev, void* stream);
+int spart_sobol_finish(const double* acc_dev, const double* ref_dev, int64_t n_total, int32_t n_out,
+                       int32_t n_vary, double* mean_dev, double* var_dev, double* first_dev, double* total_dev,
+                       double* first_se_dev, double* total_se_dev, void* stream);
+
 /* Per-kernel timing of spart_forward_bands with CUDA events recorded on the caller's stream
  * (used by bench.py for the roofline).  After spart_profile_enable(ctx, 1) every
  * spart_forward_bands call records events around its SPART_NKERNELS kernels; spart_profile_read

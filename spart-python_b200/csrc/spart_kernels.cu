@@ -22,6 +22,7 @@
 
 #include <nvtx3/nvToolsExt.h>
 
+#include <cmath>
 #include <condition_variable>
 #include <cstdio>
 #include <cstdlib>
@@ -39,6 +40,7 @@
 #include "spart_device.cuh"
 #include "spart_device_f32.cuh"
 #include "lut_kernels.cuh"
+#include "sobol_kernels.cuh"
 
 using namespace spart;
 
@@ -2532,6 +2534,97 @@ int spart_leafangles(const double* ab_dev, int64_t n, int64_t ld, double* out_de
                         ab_dev + ld, 1, 1, n, out_dev, 1, 13);
   if (rc) return rc;
   return launch(lidf_diff_kernel, (unsigned)((n + 255) / 256), 256, 0, st, out_dev, n);
+}
+
+}  // extern "C"
+
+// ---- sensitivity analysis -----------------------------------------------------------------
+static uint64_t splitmix64(uint64_t& state) {
+  uint64_t z = (state += 0x9e3779b97f4a7c15ull);
+  z = (z ^ (z >> 30)) * 0xbf58476d1ce4e5b9ull;
+  z = (z ^ (z >> 27)) * 0x94d049bb133111ebull;
+  return z ^ (z >> 31);
+}
+
+// Dimension `dim` draws words 32 dim .. 32 dim + 31 of the SplitMix64 stream of `seed`: 31 for the strictly-lower
+// rows of L, one for the shift, so its scramble does not depend on how many dimensions a call uses.
+static void sobol_scramble(uint64_t seed, int dim, unsigned (&v)[32], unsigned& shift) {
+  uint64_t state = seed + 32ull * (uint64_t)dim * 0x9e3779b97f4a7c15ull;
+  unsigned row[32];                   // row r of L (r = 0: most significant bit) as a mask over the input bits
+  row[0] = 1u << 31;
+  for (int r = 1; r < 32; ++r)
+    row[r] = ((unsigned)(splitmix64(state) & ((1ull << r) - 1)) << (32 - r)) | (1u << (31 - r));
+  shift = (unsigned)splitmix64(state);
+  for (int j = 0; j < 32; ++j) {
+    unsigned out = 0;
+    for (int r = 0; r < 32; ++r) out |= (unsigned)(__builtin_popcount(row[r] & v[j]) & 1) << (31 - r);
+    v[j] = out;
+  }
+}
+
+extern "C" {
+
+int spart_sobol_design(const int32_t* rows, const double* lo, const double* hi, int32_t n_vary, uint64_t seed,
+                       int32_t scramble, int64_t first, int64_t count, int32_t saltelli, double* params_dev,
+                       int64_t ld, void* stream) {
+  if (!rows || !lo || !hi || (!params_dev && count > 0))
+    return fail(SPART_EINVAL, "spart_sobol_design: null argument%s");
+  if (n_vary < 1 || n_vary > kSobolMaxVary || (scramble != 0 && scramble != 1) || (saltelli != 0 && saltelli != 1))
+    return fail(SPART_EINVAL, "spart_sobol_design: need 1 <= n_vary <= 27, scramble and saltelli 0 or 1%s");
+  if (first < 0 || count < 0 || first > (1ll << 32) || count > (1ll << 32) - first)
+    return fail(SPART_EINVAL, "spart_sobol_design: need first, count >= 0 and first + count <= 2^32%s");
+  if (ld < (saltelli ? (int64_t)(n_vary + 2) * count : count))
+    return fail(SPART_EINVAL, "spart_sobol_design: ld is below the number of samples written%s");
+  SobolDesignArgs a;
+  unsigned used = 0;
+  for (int p = 0; p < n_vary; ++p) {
+    if (rows[p] < 0 || rows[p] >= SPART_NPAR || (used >> rows[p] & 1u))
+      return fail(SPART_EINVAL, "spart_sobol_design: rows must be distinct values in 0..26%s");
+    used |= 1u << rows[p];
+    if (!(std::isfinite(lo[p]) && std::isfinite(hi[p]) && lo[p] < hi[p]))
+      return fail(SPART_EINVAL, "spart_sobol_design: need finite lo < hi%s");
+    a.row[p] = rows[p];
+    a.lo[p] = lo[p];
+    a.hi[p] = hi[p];
+  }
+  if (count == 0) return SPART_OK;
+  for (int d = 0; d < (saltelli ? 2 : 1) * n_vary; ++d) {
+    memcpy(a.v[d], SPART_SOBOL_V[d], sizeof(a.v[d]));
+    a.shift[d] = 0;
+    if (scramble) sobol_scramble(seed, d, a.v[d], a.shift[d]);
+  }
+  NvtxRange r("spart::sobol_design");
+  const dim3 grid((unsigned)((count + kSobolThreads - 1) / kSobolThreads), (unsigned)n_vary);
+  return launch(sobol_design_kernel, grid, kSobolThreads, 0, (cudaStream_t)stream, a, (int)n_vary, first, count,
+                (int)saltelli, params_dev, ld);
+}
+
+size_t spart_sobol_acc_elems(int32_t n_out, int32_t n_vary) {
+  if (n_out < 1 || n_vary < 1 || n_vary > kSobolMaxVary) return 0;
+  return (size_t)kSobolSlices * (size_t)(n_vary + 1) * (size_t)n_out * kSobolSums;
+}
+
+int spart_sobol_accumulate(const double* f_dev, int64_t n, int32_t n_out, int32_t n_vary, const double* ref_dev,
+                           double* acc_dev, void* stream) {
+  if ((!f_dev && n > 0) || !ref_dev || !acc_dev) return fail(SPART_EINVAL, "spart_sobol_accumulate: null argument%s");
+  if (n < 0 || n_out < 1 || n_vary < 1 || n_vary > kSobolMaxVary)
+    return fail(SPART_EINVAL, "spart_sobol_accumulate: need n >= 0, n_out >= 1, 1 <= n_vary <= 27%s");
+  if (n == 0) return SPART_OK;
+  NvtxRange r("spart::sobol_accumulate");
+  return launch(sobol_accumulate_kernel, dim3((unsigned)(n_vary + 1), kSobolSlices), kSobolThreads, 0,
+                (cudaStream_t)stream, f_dev, n, (int)n_out, (int)n_vary, ref_dev, acc_dev);
+}
+
+int spart_sobol_finish(const double* acc_dev, const double* ref_dev, int64_t n_total, int32_t n_out, int32_t n_vary,
+                       double* mean_dev, double* var_dev, double* first_dev, double* total_dev, double* first_se_dev,
+                       double* total_se_dev, void* stream) {
+  if (!acc_dev || !ref_dev || !mean_dev || !var_dev || !first_dev || !total_dev || !first_se_dev || !total_se_dev)
+    return fail(SPART_EINVAL, "spart_sobol_finish: null argument%s");
+  if (n_total < 1 || n_out < 1 || n_vary < 1 || n_vary > kSobolMaxVary)
+    return fail(SPART_EINVAL, "spart_sobol_finish: need n_total >= 1, n_out >= 1, 1 <= n_vary <= 27%s");
+  const int64_t threads = (int64_t)n_out * n_vary;
+  return launch(sobol_finish_kernel, (unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream, acc_dev, ref_dev,
+                n_total, (int)n_out, (int)n_vary, mean_dev, var_dev, first_dev, total_dev, first_se_dev, total_se_dev);
 }
 
 }  // extern "C"

@@ -5,7 +5,7 @@ CUDA device, every compute entry point raises.  Build with `python __graft_entry
 (or `python spart-python_b200/build.py`).
 """
 import ctypes
-from ctypes import POINTER, Structure, byref, c_char_p, c_double, c_int32, c_int64, c_size_t, c_uint32, c_void_p
+from ctypes import POINTER, Structure, byref, c_char_p, c_double, c_int32, c_int64, c_size_t, c_uint32, c_uint64, c_void_p
 from pathlib import Path
 
 import os
@@ -35,7 +35,8 @@ EXPORTS = (
     "spart_workspace_bytes", "spart_forward_bands", "spart_forward_bands_bc", "spart_forward_bands_host", "spart_forward_spectrum",
     "spart_smac", "spart_sailh", "spart_lut_workspace_bytes", "spart_lut_nearest", "spart_lut_nearest_tc", "spart_lut_unpack",
     "spart_lut_topk_workspace_bytes", "spart_lut_topk", "spart_lut_topk_merge", "spart_lut_moments_accumulate",
-    "spart_lut_moments_finish",
+    "spart_lut_moments_finish", "spart_sobol_design", "spart_sobol_acc_elems", "spart_sobol_accumulate",
+    "spart_sobol_finish",
     "spart_leafangles", "spart_set_lidf", "spart_profile_enable", "spart_profile_read", "spart_measure_peaks", "spart_measure_fp64_chain", "spart_launch_count",
 )
 
@@ -110,6 +111,12 @@ def load():
                                                  c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p]
     lib.spart_lut_moments_finish.argtypes = [c_void_p, c_void_p, c_int64, c_int32, c_void_p, c_void_p, c_void_p,
                                              c_void_p]
+    lib.spart_sobol_design.argtypes = [POINTER(c_int32), POINTER(c_double), POINTER(c_double), c_int32, c_uint64,
+                                       c_int32, c_int64, c_int64, c_int32, c_void_p, c_int64, c_void_p]
+    lib.spart_sobol_acc_elems.argtypes = [c_int32, c_int32]
+    lib.spart_sobol_acc_elems.restype = c_size_t
+    lib.spart_sobol_accumulate.argtypes = [c_void_p, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p]
+    lib.spart_sobol_finish.argtypes = [c_void_p, c_void_p, c_int64, c_int32, c_int32] + [c_void_p] * 7
     lib.spart_leafangles.argtypes = [c_void_p, c_int64, c_int64, c_void_p, c_void_p]
     lib.spart_set_lidf.argtypes = [c_void_p, c_int64, c_void_p, c_void_p]
     lib.spart_profile_enable.argtypes = [c_void_p, c_int32]
