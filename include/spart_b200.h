@@ -373,6 +373,72 @@ int spart_sobol_finish(const double* acc_dev, const double* ref_dev, int64_t n_t
                        int32_t n_vary, double* mean_dev, double* var_dev, double* first_dev, double* total_dev,
                        double* first_se_dev, double* total_se_dev, void* stream);
 
+/* Retrieval by bounded Levenberg-Marquardt (new; the reference has none): fit n_vary = P (1..16) varied rows of
+ * each observation's parameters to its band vector, from n_starts starts per observation.  A track is one start of
+ * one observation: track t (0 <= t < n_tracks) belongs to observation t / n_starts.  It is iterated in normalised
+ * coordinates u in [0, 1]^P, x_p = lo[p] + (hi[p] - lo[p]) u_p (each operation rounded once, no fused
+ * multiply-add).  lo and hi are HOST arrays of P finite values with lo < hi.  One iteration is
+ * spart_invert_design -> spart_forward_bands -> spart_invert_step over the active tracks, whose indices the caller
+ * lists in active_dev (int32 [n_active], distinct); a track is active while its status is SPART_INV_ACTIVE.  No
+ * context is needed; the calls run on the current device and on the caller's stream.
+ *
+ * State: double state_dev [spart_invert_state_rows(P)][n_tracks] (column t = track t); rows u [P], trial [P],
+ * J^T W J [P (P + 1) / 2] (lower triangle, (i, j <= i) at row i (i + 1) / 2 + j), J^T W r [P], C, lambda, status,
+ * forward calls.  The caller initialises it: trial = the start clipped to [0, 1] in u, C = NaN, lambda = 1e-3,
+ * status SPART_INV_ACTIVE (SPART_INV_INVALID for a start that is not finite), forward calls 0; u, J^T W J and
+ * J^T W r are written by the first step.  spart_invert_state_rows returns 0 for P outside 1..16.
+ *
+ * spart_invert_design writes the P + 1 samples of each active track, columns slot (P + 1) .. slot (P + 1) + P of
+ * params_dev [SPART_NPAR][ld] (ld >= n_active (P + 1)) for active_dev[slot]: sample 0 at the trial point and
+ * sample p + 1 with u_p moved by h = 2^-17, upwards when u_p + h <= 1, otherwise downwards.  Varied rows
+ * rows[0..P-1] get x; the n_obs_rows rows obs_rows[] (distinct, not varied) get the track's observation's value
+ * obs_values_dev[k ld_values + o]; every other row is a broadcast row: base[row] (HOST [27]) is written at element
+ * 0 only, so run the batch with those rows in broadcast_rows (fixed angles then select the folded geometry).
+ *
+ * spart_invert_step reads the forward outputs f_dev [n_active (P + 1)][n_bands][3] of that batch, column `column`
+ * (0 R_TOC, 1 R_TOA, 2 L_TOA), the observations obs_dev [n_tracks / n_starts][n_bands] and the weights
+ * weights_dev [n_bands] (NULL: all 1), and advances each active track by one step:
+ *   - C(trial) = sum_b w_b (f_b - y_b)^2 in band order.  On the first call the trial (the start) is accepted; a
+ *     non-finite observation value or C gives SPART_INV_INVALID.  Later, the trial is accepted if
+ *     C(trial) < C, strictly: then u = trial, C = C(trial), J^T W J and J^T W r are those of the trial (column p of
+ *     J = (f(sample p + 1) - f(sample 0)) / du_p, du_p the difference of the two x written over hi - lo), lambda =
+ *     max(lambda / 10, 1e-15), and SPART_INV_CONVERGED_COST if C_old - C <= ftol C_old.  On rejection lambda =
+ *     10 lambda.
+ *   - SPART_INV_STALLED if lambda > 1e16, else SPART_INV_MAX_ITER if the track has made max_iter forward calls.
+ *   - Otherwise (J^T W J + lambda D) delta = -J^T W r with D = diag(max(J^T W J_pp, 1e-30)) is solved by
+ *     Cholesky, with lambda = 10 lambda and a new factorisation while one fails (SPART_INV_STALLED past 1e16);
+ *     the next trial is clip(u + delta, 0, 1), and SPART_INV_CONVERGED_STEP if max_p |trial_p - u_p| <= xtol.
+ *   ftol, xtol >= 0 and finite; max_iter >= 1.  Each track's result depends on its own data only.
+ *
+ * spart_invert_finish, per observation o of n_obs (n_tracks = n_obs n_starts): the track with the lowest finite C
+ * (ties to the lowest start) gives x_dev [n_obs][P] (x of its u), cost_dev, status_dev, start_dev (the start's
+ * index, 0..n_starts-1) and iterations_dev (its forward calls); n_forward_dev is the forward runs of all the
+ * observation's tracks, sum of forward calls x (P + 1).  std_dev [n_obs][P] = (hi - lo) sqrt(s (A^-1)_pp) with
+ * A = J^T W J of that track, s = C / (n_bands - P) (absolute_sigma = 0, as scipy.optimize.curve_fit) or 1
+ * (absolute_sigma = 1: the weights are 1 / sigma_b^2); NaN when A is not positive definite, or when n_bands <= P
+ * with absolute_sigma = 0.  An observation without a finite-cost track gets NaN x, cost and std,
+ * SPART_INV_INVALID, start -1 and 0 iterations. */
+#define SPART_INV_ACTIVE 0
+#define SPART_INV_CONVERGED_COST 1
+#define SPART_INV_CONVERGED_STEP 2
+#define SPART_INV_MAX_ITER 3
+#define SPART_INV_STALLED 4
+#define SPART_INV_INVALID 5
+size_t spart_invert_state_rows(int32_t n_vary);
+int spart_invert_design(const int32_t* rows, const double* lo, const double* hi, int32_t n_vary,
+                        const int32_t* obs_rows, int32_t n_obs_rows, const double* obs_values_dev,
+                        int64_t ld_values, const double* base, int32_t n_starts, const double* state_dev,
+                        int64_t n_tracks, const int32_t* active_dev, int64_t n_active, double* params_dev,
+                        int64_t ld, void* stream);
+int spart_invert_step(const double* lo, const double* hi, int32_t n_vary, int32_t n_starts, const double* f_dev,
+                      int32_t n_bands, int32_t column, const double* obs_dev, const double* weights_dev, double ftol,
+                      double xtol, int32_t max_iter, double* state_dev, int64_t n_tracks, const int32_t* active_dev,
+                      int64_t n_active, void* stream);
+int spart_invert_finish(const double* lo, const double* hi, int32_t n_vary, int32_t n_starts, int32_t n_bands,
+                        int32_t absolute_sigma, const double* state_dev, int64_t n_obs, double* x_dev,
+                        double* cost_dev, double* std_dev, int32_t* status_dev, int32_t* start_dev,
+                        int32_t* iterations_dev, int64_t* n_forward_dev, void* stream);
+
 /* Per-kernel timing of spart_forward_bands with CUDA events recorded on the caller's stream
  * (used by bench.py for the roofline).  After spart_profile_enable(ctx, 1) every
  * spart_forward_bands call records events around its SPART_NKERNELS kernels; spart_profile_read

@@ -41,6 +41,7 @@
 #include "spart_device_f32.cuh"
 #include "lut_kernels.cuh"
 #include "sobol_kernels.cuh"
+#include "invert_kernels.cuh"
 
 using namespace spart;
 
@@ -2625,6 +2626,122 @@ int spart_sobol_finish(const double* acc_dev, const double* ref_dev, int64_t n_t
   const int64_t threads = (int64_t)n_out * n_vary;
   return launch(sobol_finish_kernel, (unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream, acc_dev, ref_dev,
                 n_total, (int)n_out, (int)n_vary, mean_dev, var_dev, first_dev, total_dev, first_se_dev, total_se_dev);
+}
+
+}  // extern "C"
+
+// ---- retrieval by bounded Levenberg-Marquardt ------------------------------------------------
+// Checks the box of the varied parameters (lo, hi may be NULL: then only n_vary is checked) and fills `a`.
+static int invert_args(const char* who, const int32_t* rows, const double* lo, const double* hi, int32_t n_vary,
+                       int32_t n_starts, InvertArgs& a) {
+  if (n_vary < 1 || n_vary > kInvMaxVary) return fail(SPART_EINVAL, "%s: need 1 <= n_vary <= 16", who);
+  if (n_starts < 1) return fail(SPART_EINVAL, "%s: need n_starts >= 1", who);
+  if (!lo || !hi) return fail(SPART_EINVAL, "%s: null argument", who);
+  a = InvertArgs{};
+  a.n_vary = n_vary;
+  a.n_starts = n_starts;
+  unsigned used = 0;
+  for (int p = 0; p < n_vary; ++p) {
+    if (rows) {
+      if (rows[p] < 0 || rows[p] >= SPART_NPAR || (used >> rows[p] & 1u))
+        return fail(SPART_EINVAL, "%s: rows must be distinct values in 0..26", who);
+      used |= 1u << rows[p];
+      a.row[p] = rows[p];
+    }
+    if (!(std::isfinite(lo[p]) && std::isfinite(hi[p]) && lo[p] < hi[p]))
+      return fail(SPART_EINVAL, "%s: need finite lo < hi", who);
+    a.lo[p] = lo[p];
+    a.hi[p] = hi[p];
+  }
+  return SPART_OK;
+}
+
+extern "C" {
+
+size_t spart_invert_state_rows(int32_t n_vary) {
+  return (n_vary < 1 || n_vary > kInvMaxVary) ? 0 : (size_t)inv_rows(n_vary);
+}
+
+int spart_invert_design(const int32_t* rows, const double* lo, const double* hi, int32_t n_vary,
+                        const int32_t* obs_rows, int32_t n_obs_rows, const double* obs_values_dev,
+                        int64_t ld_values, const double* base, int32_t n_starts, const double* state_dev,
+                        int64_t n_tracks, const int32_t* active_dev, int64_t n_active, double* params_dev,
+                        int64_t ld, void* stream) {
+  static const char* who = "spart_invert_design";
+  if (!rows || !base || (n_obs_rows > 0 && (!obs_rows || !obs_values_dev)) ||
+      (n_active > 0 && (!state_dev || !active_dev || !params_dev)))
+    return fail(SPART_EINVAL, "spart_invert_design: null argument%s");
+  InvertArgs a;
+  if (const int rc = invert_args(who, rows, lo, hi, n_vary, n_starts, a)) return rc;
+  if (n_tracks < 0 || n_active < 0 || n_active > n_tracks || n_tracks * (n_vary + 1) > INT32_MAX)
+    return fail(SPART_EINVAL, "spart_invert_design: need 0 <= n_active <= n_tracks and n_tracks (n_vary + 1) < 2^31%s");
+  if (ld < n_active * (n_vary + 1) || (n_active > 0 && ld < 1))
+    return fail(SPART_EINVAL, "spart_invert_design: ld is below the number of samples written%s");
+  if (n_obs_rows < 0 || n_obs_rows > SPART_NPAR - n_vary || (n_obs_rows > 0 && ld_values < n_tracks / n_starts))
+    return fail(SPART_EINVAL, "spart_invert_design: need 0 <= n_obs_rows <= 27 - n_vary and ld_values >= "
+                              "n_tracks / n_starts%s");
+  unsigned used = 0;
+  for (int p = 0; p < n_vary; ++p) used |= 1u << rows[p];
+  for (int k = 0; k < n_obs_rows; ++k) {
+    if (obs_rows[k] < 0 || obs_rows[k] >= SPART_NPAR || (used >> obs_rows[k] & 1u))
+      return fail(SPART_EINVAL, "spart_invert_design: obs_rows must be distinct rows in 0..26 that are not varied%s");
+    used |= 1u << obs_rows[k];
+    a.obs_row[k] = obs_rows[k];
+  }
+  a.n_obs_rows = n_obs_rows;
+  for (int r = 0; r < SPART_NPAR; ++r) {
+    a.base[r] = base[r];
+    if (!(used >> r & 1u)) a.bcast_row[a.n_bcast++] = r;
+  }
+  if (n_active == 0) return SPART_OK;
+  NvtxRange r("spart::invert_design");
+  const int64_t n = n_active * (n_vary + 1);
+  return launch(invert_design_kernel, (unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream, a, obs_values_dev,
+                ld_values, state_dev, n_tracks, active_dev, n_active, params_dev, ld);
+}
+
+int spart_invert_step(const double* lo, const double* hi, int32_t n_vary, int32_t n_starts, const double* f_dev,
+                      int32_t n_bands, int32_t column, const double* obs_dev, const double* weights_dev, double ftol,
+                      double xtol, int32_t max_iter, double* state_dev, int64_t n_tracks, const int32_t* active_dev,
+                      int64_t n_active, void* stream) {
+  static const char* who = "spart_invert_step";
+  if (n_active > 0 && (!f_dev || !obs_dev || !state_dev || !active_dev))
+    return fail(SPART_EINVAL, "spart_invert_step: null argument%s");
+  InvertArgs a;
+  if (const int rc = invert_args(who, nullptr, lo, hi, n_vary, n_starts, a)) return rc;
+  if (n_tracks < 0 || n_active < 0 || n_active > n_tracks || n_tracks > INT32_MAX)
+    return fail(SPART_EINVAL, "spart_invert_step: need 0 <= n_active <= n_tracks < 2^31%s");
+  if (n_bands < 1 || column < 0 || column >= SPART_NOUT || max_iter < 1)
+    return fail(SPART_EINVAL, "spart_invert_step: need n_bands >= 1, column 0..2 and max_iter >= 1%s");
+  if (!(ftol >= 0.0 && xtol >= 0.0 && std::isfinite(ftol) && std::isfinite(xtol)))
+    return fail(SPART_EINVAL, "spart_invert_step: need finite ftol, xtol >= 0%s");
+  if (n_active == 0) return SPART_OK;
+  NvtxRange r("spart::invert_step");
+  return launch(invert_step_kernel, (unsigned)((n_active + kInvThreads - 1) / kInvThreads), kInvThreads,
+                sizeof(double) * kInvThreads * inv_shared(n_vary), (cudaStream_t)stream, a, f_dev, (int)n_bands,
+                (int)column, obs_dev, weights_dev, ftol, xtol, (int)max_iter, state_dev, n_tracks, active_dev,
+                n_active);
+}
+
+int spart_invert_finish(const double* lo, const double* hi, int32_t n_vary, int32_t n_starts, int32_t n_bands,
+                        int32_t absolute_sigma, const double* state_dev, int64_t n_obs, double* x_dev,
+                        double* cost_dev, double* std_dev, int32_t* status_dev, int32_t* start_dev,
+                        int32_t* iterations_dev, int64_t* n_forward_dev, void* stream) {
+  static const char* who = "spart_invert_finish";
+  if (n_obs > 0 && (!state_dev || !x_dev || !cost_dev || !std_dev || !status_dev || !start_dev || !iterations_dev ||
+                    !n_forward_dev))
+    return fail(SPART_EINVAL, "spart_invert_finish: null argument%s");
+  InvertArgs a;
+  if (const int rc = invert_args(who, nullptr, lo, hi, n_vary, n_starts, a)) return rc;
+  if (n_obs < 0 || n_obs * n_starts > INT32_MAX || n_bands < 1 || (absolute_sigma != 0 && absolute_sigma != 1))
+    return fail(SPART_EINVAL, "spart_invert_finish: need 0 <= n_obs n_starts < 2^31, n_bands >= 1 and "
+                              "absolute_sigma 0 or 1%s");
+  if (n_obs == 0) return SPART_OK;
+  NvtxRange r("spart::invert_finish");
+  return launch(invert_finish_kernel, (unsigned)((n_obs + kInvThreads - 1) / kInvThreads), kInvThreads,
+                sizeof(double) * kInvThreads * inv_shared(n_vary), (cudaStream_t)stream, a, (int)n_bands,
+                (int)absolute_sigma, state_dev, n_obs, x_dev, cost_dev, std_dev, status_dev, start_dev,
+                iterations_dev, n_forward_dev);
 }
 
 }  // extern "C"

@@ -6,7 +6,7 @@ plus the batched entry points `run_batch` / `run_batch_params`.
 """
 from ._lib import SpartError
 from .batch import pack_batch, row_as_dataframe, run_batch, run_batch_params
-from . import lut, sensitivity
+from . import inversion, lut, sensitivity
 from .engine import CompactBands, Engine, default_engine
 from .model import SPART, SpectralBands, load_optical_parameters, load_sensor_info
 from .params import (Angles, AtmosphericProperties, CanopyStructure, LeafBiology, SoilParameters,
@@ -19,7 +19,7 @@ __all__ = [
     "SPART", "SpectralBands", "LeafBiology", "SoilParameters", "SoilParametersFromFile", "SoilLibrary",
     "CanopyStructure", "Angles",
     "AtmosphericProperties", "run_batch", "run_batch_params", "pack_batch", "pack_params",
-    "row_as_dataframe", "lut", "sensitivity", "Engine", "CompactBands", "default_engine", "SpartError", "SENSOR_NAMES",
+    "row_as_dataframe", "lut", "sensitivity", "inversion", "Engine", "CompactBands", "default_engine", "SpartError", "SENSOR_NAMES",
     "load_optical_parameters", "load_sensor_info", "synthetic_fullspectrum_sensorinfo",
     "PROSPECT_5D", "BSM", "SAILH", "SMAC", "prospect_batch", "bsm_batch", "sailh_batch", "smac_batch",
     "set_leaf_refl_trans_assumptions", "set_soil_refl_trans_assumptions",

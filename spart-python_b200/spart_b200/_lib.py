@@ -36,7 +36,7 @@ EXPORTS = (
     "spart_smac", "spart_sailh", "spart_lut_workspace_bytes", "spart_lut_nearest", "spart_lut_nearest_tc", "spart_lut_unpack",
     "spart_lut_topk_workspace_bytes", "spart_lut_topk", "spart_lut_topk_merge", "spart_lut_moments_accumulate",
     "spart_lut_moments_finish", "spart_sobol_design", "spart_sobol_acc_elems", "spart_sobol_accumulate",
-    "spart_sobol_finish",
+    "spart_sobol_finish", "spart_invert_state_rows", "spart_invert_design", "spart_invert_step", "spart_invert_finish",
     "spart_leafangles", "spart_set_lidf", "spart_profile_enable", "spart_profile_read", "spart_measure_peaks", "spart_measure_fp64_chain", "spart_launch_count",
 )
 
@@ -117,6 +117,16 @@ def load():
     lib.spart_sobol_acc_elems.restype = c_size_t
     lib.spart_sobol_accumulate.argtypes = [c_void_p, c_int64, c_int32, c_int32, c_void_p, c_void_p, c_void_p]
     lib.spart_sobol_finish.argtypes = [c_void_p, c_void_p, c_int64, c_int32, c_int32] + [c_void_p] * 7
+    lib.spart_invert_state_rows.argtypes = [c_int32]
+    lib.spart_invert_state_rows.restype = c_size_t
+    lib.spart_invert_design.argtypes = [POINTER(c_int32), POINTER(c_double), POINTER(c_double), c_int32,
+                                        POINTER(c_int32), c_int32, c_void_p, c_int64, POINTER(c_double), c_int32,
+                                        c_void_p, c_int64, c_void_p, c_int64, c_void_p, c_int64, c_void_p]
+    lib.spart_invert_step.argtypes = [POINTER(c_double), POINTER(c_double), c_int32, c_int32, c_void_p, c_int32,
+                                      c_int32, c_void_p, c_void_p, c_double, c_double, c_int32, c_void_p, c_int64,
+                                      c_void_p, c_int64, c_void_p]
+    lib.spart_invert_finish.argtypes = [POINTER(c_double), POINTER(c_double), c_int32, c_int32, c_int32, c_int32,
+                                        c_void_p, c_int64] + [c_void_p] * 8
     lib.spart_leafangles.argtypes = [c_void_p, c_int64, c_int64, c_void_p, c_void_p]
     lib.spart_set_lidf.argtypes = [c_void_p, c_int64, c_void_p, c_void_p]
     lib.spart_profile_enable.argtypes = [c_void_p, c_int32]
